@@ -361,6 +361,33 @@ def measured_peak():
     return 6650.0, "fallback (B200_PROFILING.md, 6.65 TB/s)"
 
 
+DUMP_FRAMES = 1 << 21  # frames kept per output: 16 MiB of CF32 + 32 MiB of I2S words as float64
+
+
+def dump_frames(frames: int):
+    """The frames --dump-outputs keeps of a block: all of them (None) up to DUMP_FRAMES, else the
+    same seeded, sorted sample on every run, so that two builds can be compared element for element."""
+    import numpy as np
+    if frames <= DUMP_FRAMES:
+        return None
+    return np.sort(np.random.default_rng(SEED).choice(frames, DUMP_FRAMES, replace=False))
+
+
+def dump_outputs(out_dir: Path, frames: int, cf, i2s_out):
+    """Write what the RX and TX conversions hand back to their caller, at the frames dump_frames()
+    picks: rx_cf32.npy (float32 I/Q samples) and tx_i2s.npy (the int32 I2S words as float64,
+    which holds every int32 exactly)."""
+    import numpy as np
+    import torch
+    pick = dump_frames(frames)
+    if pick is not None:
+        words = torch.from_numpy(np.stack([2 * pick, 2 * pick + 1], axis=1).ravel()).to(cf.device)
+        cf, i2s_out = cf.index_select(0, words), i2s_out.index_select(0, words)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "rx_cf32.npy", cf.cpu().numpy().astype(np.float32))
+    np.save(out_dir / "tx_i2s.npy", i2s_out.cpu().numpy().astype(np.float64))
+
+
 def run_gpu_arm(args, rank: int, local_rank: int, world: int):
     import torch
     import torch.distributed as dist
@@ -436,6 +463,8 @@ def run_gpu_arm(args, rank: int, local_rank: int, world: int):
     barrier()
     launches = ctx.counter("launches") - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), frames, cf, i2s_out)
 
     total_ms = ev[0].elapsed_time(ev[-1])
     rx_ms = [ev[2 * k].elapsed_time(ev[2 * k + 1]) for k in range(args.steps)]
@@ -1184,7 +1213,14 @@ def main():
                     help="--workload bank: capture frames come from sxgpu_bank_ingest instead of the synthetic generator")
     ap.add_argument("--fused", action="store_true",
                     help="--workload bank: the iteration as one sxgpu_bank_repeat launch instead of read + write")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="default workload: after the timed steps, write the last step's RX and TX outputs (rank 0's, "
+                         f"a fixed seeded sample of {DUMP_FRAMES} frames of larger blocks) as DIR/rx_cf32.npy and DIR/tx_i2s.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "blocks" or args.single_process):
+        ap.error("--dump-outputs is implemented for the default workload only (--impl b200 --workload blocks, one rank per GPU)")
 
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if args.single_process and args.impl != "reference":

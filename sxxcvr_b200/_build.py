@@ -71,7 +71,7 @@ def build_gpu_library(force: bool = False) -> Path:
 
 
 def build_soapy_module(force: bool = False) -> Path:
-    build_gpu_library(force)
+    build_gpu_library()
     deps = SOAPY_SOURCES + list((CSRC / "shim").rglob("*.h*")) + list((CSRC / "host").glob("*.hpp")) + [GPU_LIB]
     if force or _stale(SOAPY_LIB, deps):
         _run([
@@ -90,7 +90,7 @@ HOOK_EXAMPLE_LIB = LIB / "libsxhook_example.so"
 
 def build_examples(force: bool = False) -> Path:
     """examples/repeater.cpp: a C++ application on the SoapySDR API, linked against the module."""
-    build_soapy_module(force)
+    build_soapy_module()
     src = ROOT / "examples" / "repeater.cpp"
     if force or _stale(EXAMPLE_BIN, [src, SOAPY_LIB]):
         _run([os.environ.get("CXX", "g++"), "-std=c++17", "-O2", "-Wall", "-Wextra",
@@ -101,7 +101,7 @@ def build_examples(force: bool = False) -> Path:
 
 def build_hook_example(force: bool = False) -> Path:
     """examples/repeater_hook.cu: user DSP compiled into the fused bank iteration (include/sx_hook.cuh)."""
-    build_gpu_library(force)
+    build_gpu_library()
     src = ROOT / "examples" / "repeater_hook.cu"
     deps = [src, ROOT / "include" / "sx_hook.cuh", CSRC / "sx_bank.cuh", CSRC / "sx_kernels.cuh", GPU_LIB]
     if force or _stale(HOOK_EXAMPLE_LIB, deps):
@@ -111,6 +111,10 @@ def build_hook_example(force: bool = False) -> Path:
 
 
 def build_all(force: bool = False) -> None:
+    # `force` rebuilds each target once, in link order; the dependencies of each build_* call are
+    # only brought up to date.  Forcing them again would relink libsxgpu.so after the libraries
+    # linked against it, leaving those older than their dependency, so that the next load finds
+    # them stale and relinks them in the tree.
     build_gpu_library(force)
     build_soapy_module(force)
     build_examples(force)

@@ -56,3 +56,30 @@ def test_gpu_arm_prints_one_json_line_with_roofline_and_e2e():
     assert b["sustained"]["seconds"] >= 0.2
     assert b["cpu_baseline"]["kind"] in ("reference", "port")
     assert isinstance(b["clocks"]["reasons"], list)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("log2_frames", [16, 22], ids=["whole_block", "sampled_block"])
+def test_gpu_arm_dumps_what_the_last_timed_step_computed(oracle, tmp_path, log2_frames):
+    import numpy as np
+    import bench
+    import sxtest
+    frames = 1 << log2_frames
+    lines = run([sys.executable, "bench.py", "--steps", "2", "--warmup", "1", "--log2-frames", str(log2_frames),
+                 "--e2e-log2-frames", "16", "--min-seconds", "0", "--no-rows", "--no-cpu-baseline",
+                 "--dump-outputs", str(tmp_path)])
+    assert len(lines) == 1
+    b = json.loads(lines[0])
+    assert b["steps"] == 2 and b["gpu_launches"] == 2 * 2     # one RX and one TX launch per timed step
+    cf, words = np.load(tmp_path / "rx_cf32.npy"), np.load(tmp_path / "tx_i2s.npy")
+    assert cf.dtype == np.float32 and words.dtype == np.float64
+    want_cf = sxtest.oracle_rx(oracle, sxtest.synth_frames(oracle, 0, frames, bench.SEED))
+    want_words = sxtest.oracle_tx(oracle, want_cf, bench.THR2)
+    pick = bench.dump_frames(frames)
+    if pick is not None:
+        assert pick.size == bench.DUMP_FRAMES and np.array_equal(pick, bench.dump_frames(frames))
+        keep = np.stack([2 * pick, 2 * pick + 1], axis=1).ravel()
+        want_cf, want_words = want_cf[keep], want_words[keep]
+    assert cf.size == want_cf.size == 2 * min(frames, bench.DUMP_FRAMES)
+    assert np.array_equal(cf.view(np.uint32), want_cf.view(np.uint32))
+    assert np.array_equal(words.astype(np.int64), want_words.astype(np.int64))

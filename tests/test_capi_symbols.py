@@ -43,6 +43,35 @@ def test_library_is_sm100a_only_and_has_no_cpu_path():
     assert archs == {"sm_100a"}, archs
 
 
+def test_forced_build_links_each_target_once_and_leaves_none_stale(tmp_path, monkeypatch):
+    """build() forces every target.  Each must be linked once, after what it links against: a
+    target left older than a dependency is relinked in the tree by the next load, which fails
+    where the tree is read-only.  The compiler is replaced by a recorder that writes each output
+    with a strictly later time stamp."""
+    import os
+    import time
+    from sxxcvr_b200 import _build
+    for name in ("GPU_LIB", "SOAPY_LIB", "EXAMPLE_BIN", "HOOK_EXAMPLE_LIB"):
+        monkeypatch.setattr(_build, name, tmp_path / getattr(_build, name).name)
+    monkeypatch.setattr(_build, "LIB", tmp_path)
+    linked, clock = [], [time.time() + 10]
+
+    def record(cmd):
+        out = Path(cmd[cmd.index("-o") + 1])
+        out.write_bytes(b"")
+        clock[0] += 1
+        os.utime(out, (clock[0], clock[0]))
+        linked.append(out.name)
+
+    monkeypatch.setattr(_build, "_run", record)
+    monkeypatch.setattr(_build, "_find_nvcc", lambda: "nvcc")
+    _build.build_all(force=True)
+    assert sorted(linked) == sorted(p.name for p in (_build.GPU_LIB, _build.SOAPY_LIB, _build.EXAMPLE_BIN,
+                                                     _build.HOOK_EXAMPLE_LIB))
+    _build.build_all()
+    assert len(linked) == 4, linked[4:]
+
+
 def test_init_fails_loudly_without_a_gpu():
     import torch
     if torch.cuda.is_available():

@@ -204,18 +204,22 @@ def test_time_round_trip_over_arbitrary_rates(oracle, rate, ticks):
     assert t2n(ticks + 1, rate) > ns              # strictly monotonic: distinct ticks, distinct stamps
 
 
-def test_time_matches_shim_used_by_both_drivers(oracle, ref):
+def test_time_matches_shim_used_by_both_drivers(oracle):
+    """csrc/host/harness_capi.cpp is compiled into the product module and into the reference
+    build alike; the product's copy loads without a GPU."""
     import ctypes as C
-    ref.sxh_ticks_to_time_ns.argtypes = [C.c_longlong, C.c_double]
-    ref.sxh_ticks_to_time_ns.restype = C.c_longlong
-    ref.sxh_time_ns_to_ticks.argtypes = [C.c_longlong, C.c_double]
-    ref.sxh_time_ns_to_ticks.restype = C.c_longlong
+    from sxxcvr_b200 import _build
+    shim = C.CDLL(str(_build.build_soapy_module()))
+    shim.sxh_ticks_to_time_ns.argtypes = [C.c_longlong, C.c_double]
+    shim.sxh_ticks_to_time_ns.restype = C.c_longlong
+    shim.sxh_time_ns_to_ticks.argtypes = [C.c_longlong, C.c_double]
+    shim.sxh_time_ns_to_ticks.restype = C.c_longlong
     rng = np.random.default_rng(1)
     for rate in sxtest.RATES:
         for p in rng.integers(0, 2**45, size=200):
             p = int(p)
-            assert ref.sxh_ticks_to_time_ns(p, rate) == oracle.sxo_ticks_to_time_ns(p, rate)
-            assert ref.sxh_time_ns_to_ticks(p, rate) == oracle.sxo_time_ns_to_ticks(p, rate)
+            assert shim.sxh_ticks_to_time_ns(p, rate) == oracle.sxo_ticks_to_time_ns(p, rate)
+            assert shim.sxh_time_ns_to_ticks(p, rate) == oracle.sxo_time_ns_to_ticks(p, rate)
 
 
 # ---- extensions, stats, synthetic source -------------------------------------------------------------
