@@ -1,12 +1,13 @@
-// repeater_hook.cu -- the memoryless part of the reference repeater's DSP, compiled INTO the
-// fused bank iteration through include/sx_hook.cuh.
+// repeater_hook.cu -- the reference repeater's DSP, compiled INTO the fused bank iteration
+// through include/sx_hook.cuh.
 //
 // example/linear_repeater.py:100-106 (between its two channel filters):
 //         s *= 1000.0
 //         clip_signal(s)          # s /= np.maximum(np.abs(s), 1.0)        (:87-89)
 //         s *= 0.3
-// The scipy IIR filters around it carry state from sample to sample and are not part of this
-// example (sx_hook.cuh explains where such stages go).
+// is the functor below.  The scipy IIR channel filters around it carry state from block to block;
+// they are the library's sxgpu_iir cascades, which sx_example_repeat_filtered_clip_gain runs before
+// and after the functor in the same launch: the script's whole process().
 //
 // Arithmetic, chosen so that a CPU restatement can match it bit for bit (tests/test_gpu_hook.py):
 // every step is one correctly rounded IEEE operation, nothing is contracted; |s| is
@@ -55,6 +56,14 @@ int sx_example_repeat_clip_gain(sxgpu_bank *bank, void *d_cf32, long long rx_tim
 {
     return sx::bank_repeat_with(bank, d_cf32, rx_time_offset_ns, static_cast<cudaStream_t>(stream),
                                 ClipGain{pre_gain, post_gain});
+}
+
+// The script's whole process() inside the fused iteration: `pre` filter, the clipper, `post` filter.
+int sx_example_repeat_filtered_clip_gain(sxgpu_bank *bank, sxgpu_iir *pre, sxgpu_iir *post, void *d_cf32,
+                                         long long rx_time_offset_ns, float pre_gain, float post_gain, void *stream)
+{
+    return sx::bank_repeat_with(bank, d_cf32, rx_time_offset_ns, static_cast<cudaStream_t>(stream),
+                                ClipGain{pre_gain, post_gain}, pre, post);
 }
 
 // The same iteration as three launches around an ordinary kernel, the CF32 block kept in L2.

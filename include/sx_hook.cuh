@@ -18,12 +18,17 @@
 // may change them in place; what it leaves is what lands in the caller's CF32 block and what
 // the TX conversion packs.  Calls for one block are spread over the lanes of a warp in no
 // particular order, so the functor must be memoryless across samples (gain, clipper, mixer with
-// a per-frame phase, ...); filters with state along the stream (the IIRs of the reference's
-// example) need the two-launch form below.
+// a per-frame phase, ...).  Filters with state along the stream -- the channel filters of the
+// reference's example -- are the library's own: the seven-argument overload below runs a
+// sxgpu_iir cascade before the functor and another after it, in the same launch
 //
-// For DSP that cannot be expressed per sample pair: sxgpu_bank_repeat_begin() /
-// sxgpu_bank_repeat_end() (include/sxgpu.h) split the iteration around any kernel of the
-// caller's on the same stream and keep the CF32 block resident in L2 in between.
+//     sx::bank_repeat_with(bank, d_cf32, offset_ns, cuda_stream, Gain{0.5f}, pre, post);
+//
+// (examples/repeater_hook.cu does the script's whole process() so: filter, clip, filter).
+//
+// For DSP that is neither: sxgpu_bank_repeat_begin() / sxgpu_bank_repeat_end() (include/sxgpu.h)
+// split the iteration around any kernel of the caller's on the same stream and keep the CF32 block
+// resident in L2 in between.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -76,6 +81,37 @@ inline int bank_repeat_with(sxgpu_bank *bank, void *d_cf32, long long rx_time_of
     if (view.nstreams <= 16384)
         return launch(bank_repeat_reg_kernel<2, Hook>, 2);
     return launch(bank_repeat_reg_kernel<4, Hook>, 4);
+}
+
+// The same iteration with the reference's channel filters around the functor: read -> `pre`
+// cascade -> hook -> `post` cascade -> CF32 block and timed write, in one launch after the
+// decisions.  Same state, results, CF32 block and playback ring as sxgpu_bank_read, then
+// sxgpu_iir_apply(pre), the hook over the block, sxgpu_iir_apply(post), then sxgpu_bank_write
+// (HAS_TIME, rx time + offset).  Either filter may be NULL (both: the overload above).
+// With IdentityHook this is sxgpu_bank_repeat_filtered.  Needs an even period, a 16-byte aligned
+// CF32 buffer and two different filters of the bank's stream count.
+template <class Hook>
+inline int bank_repeat_with(sxgpu_bank *bank, void *d_cf32, long long rx_time_offset_ns, cudaStream_t stream,
+                            const Hook &hook, sxgpu_iir *pre, sxgpu_iir *post)
+{
+    BankState view;
+    int external = 0;
+    int rc = sxgpu_bank_device_view(bank, &view, sizeof view, &external);
+    if (rc != SXGPU_OK)
+        return rc;
+    IirView vpre = {}, vpost = {};
+    if (pre && (rc = sxgpu_iir_device_view(pre, &vpre, sizeof vpre)) != SXGPU_OK)
+        return rc;
+    if (post && (rc = sxgpu_iir_device_view(post, &vpost, sizeof vpost)) != SXGPU_OK)
+        return rc;
+    if ((pre && pre == post) || bank_repeat_iir_invalid(view, d_cf32, vpre, vpost))
+        return SXGPU_ERR_INVALID;
+    if (!pre && !post)
+        return bank_repeat_with(bank, d_cf32, rx_time_offset_ns, stream, hook);
+    return launch_bank_repeat_iir(view, static_cast<char *>(d_cf32), rx_time_offset_ns, external != 0, vpre, vpost, stream,
+                                  hook) == cudaSuccess
+               ? SXGPU_OK
+               : SXGPU_ERR_CUDA;
 }
 
 } // namespace sx

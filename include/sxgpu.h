@@ -168,18 +168,19 @@ int sxgpu_bank_read(sxgpu_bank *bank, void *d_cf32, sxgpu_stream stream);
  * when d_time_ns is NULL, at the timestamp its last read returned plus rx_time_offset_ns. */
 int sxgpu_bank_write(sxgpu_bank *bank, const void *d_cf32, int flags, const long long *d_time_ns,
                      long long rx_time_offset_ns, sxgpu_stream stream);
-/* The repeater iteration (example/linear_repeater.py:50-71 without its filters) in one launch:
- * sxgpu_bank_read(bank, d_cf32) followed by sxgpu_bank_write(bank, d_cf32, SOAPY_SDR_HAS_TIME,
- * NULL, rx_time_offset_ns).  Same state, results, CF32 block and playback ring as the two calls;
- * each stream's three stages run back to back on one warp, so the intermediate reads are served
- * from L2 and only the writes reach HBM. */
+/* The repeater iteration without its filters (example/linear_repeater.py:50-71 with an identity
+ * process()) in one launch: sxgpu_bank_read(bank, d_cf32) followed by sxgpu_bank_write(bank,
+ * d_cf32, SOAPY_SDR_HAS_TIME, NULL, rx_time_offset_ns).  Same state, results, CF32 block and
+ * playback ring as the two calls; each stream's three stages run back to back on one warp, so the
+ * intermediate reads are served from L2 and only the writes reach HBM.  With the script's channel
+ * filters: sxgpu_bank_repeat_filtered below. */
 int sxgpu_bank_repeat(sxgpu_bank *bank, void *d_cf32, long long rx_time_offset_ns, sxgpu_stream stream);
 /* The same iteration split around DSP of the caller's own (the process(buf) of
  * example/linear_repeater.py:62): begin = sxgpu_bank_read with the CF32 block marked persisting
  * in L2 for `stream`; the caller then launches its kernel(s) on that stream, in place on d_cf32;
  * end = sxgpu_bank_write(bank, d_cf32, SOAPY_SDR_HAS_TIME, NULL, rx_time_offset_ns) and the mark
  * is lifted.  DSP that is memoryless per sample can instead be compiled INTO the one-launch
- * iteration: include/sx_hook.cuh. */
+ * iteration, between the two filters of sxgpu_bank_repeat_filtered: include/sx_hook.cuh. */
 int sxgpu_bank_repeat_begin(sxgpu_bank *bank, void *d_cf32, sxgpu_stream stream);
 int sxgpu_bank_repeat_end(sxgpu_bank *bank, const void *d_cf32, long long rx_time_offset_ns, sxgpu_stream stream);
 /* Frames from outside instead of the synthetic capture: copy one period of I2S frames for each
@@ -214,6 +215,40 @@ int sxgpu_bank_positions(sxgpu_bank *bank, int64_t *h_clock, int64_t *h_rx_posit
 int sxgpu_bank_playback(sxgpu_bank *bank, uint32_t index, int64_t position, size_t nframes,
                         void *h_i2s, sxgpu_stream stream);
 int sxgpu_bank_ring_frames(sxgpu_bank *bank, uint64_t *ring_frames);
+
+/* ---- stateful IIR filters for a bank's streams ------------------------------------------- */
+
+/* The channel filters of the reference repeater (example/linear_repeater.py:78-109): a cascade of
+ * second-order sections with real coefficients, applied to I and Q independently, the state
+ * carried from block to block -- scipy.signal.sosfilt(sos, x, zi=state) with a real `sos` on
+ * complex x, one filter state per stream.  Float32 arithmetic in scipy's transposed direct form II,
+ * operation for operation (DESIGN.md, "Parity policy"): the same bits as sosfilt on complex64
+ * input with the float32-rounded coefficients. */
+#define SXGPU_IIR_MAX_SECTIONS 8
+typedef struct sxgpu_iir sxgpu_iir; /* per-stream cascade state in device memory, one per bank stream */
+/* sos: nsections rows of scipy's layout, b0 b1 b2 a0 a1 a2, as double; rounded to float32 once,
+ * here.  a0 must be exactly 1 and every coefficient finite; 1 <= nsections <= 8 (order 16).
+ * The state starts at zero.  sxgpu_destroy of the context refuses while a filter is alive. */
+int sxgpu_iir_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t nsections, const double *sos, sxgpu_iir **out);
+int sxgpu_iir_destroy(sxgpu_iir *f);
+/* zi / zf: scipy's layout for x of shape (nstreams, n) filtered along the last axis, that is
+ * [nsections][nstreams][2] complex64 on the host.  NULL zi = zeros.  Both synchronise with `stream`. */
+int sxgpu_iir_set_state(sxgpu_iir *f, const void *h_zi, sxgpu_stream stream);
+int sxgpu_iir_get_state(sxgpu_iir *f, void *h_zf, sxgpu_stream stream);
+/* Filter d_cf32[nstreams][period] in place, carrying the state: sosfilt(sos, x, zi=state) per
+ * stream.  1 <= period <= 65536; d_cf32 8-byte aligned device memory. */
+int sxgpu_iir_apply(sxgpu_iir *f, void *d_cf32, uint32_t period, sxgpu_stream stream);
+/* The repeater iteration with its filters: read -> pre -> post -> CF32 block and timed write.
+ * Same state, results, positions, CF32 block and playback ring, bit for bit, as sxgpu_bank_read,
+ * sxgpu_iir_apply(pre), sxgpu_iir_apply(post), sxgpu_bank_write(bank, d_cf32, SOAPY_SDR_HAS_TIME,
+ * NULL, rx_time_offset_ns); both filters advance on every iteration, also when the write is
+ * dropped as late.  Either filter may be NULL (both NULL: exactly sxgpu_bank_repeat).  Needs filters
+ * of the bank's stream count, two different filters, an even period and a 16-byte aligned d_cf32. */
+int sxgpu_bank_repeat_filtered(sxgpu_bank *bank, sxgpu_iir *pre, sxgpu_iir *post, void *d_cf32,
+                               long long rx_time_offset_ns, sxgpu_stream stream);
+/* For include/sx_hook.cuh, like sxgpu_bank_device_view: the filter's device-side view (struct
+ * sx::IirView).  out_bytes must be sizeof(sx::IirView). */
+int sxgpu_iir_device_view(sxgpu_iir *f, void *out, size_t out_bytes);
 
 /* ---- the hot path, host buffers ---------------------------------------------------------- */
 

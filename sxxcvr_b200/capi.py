@@ -79,6 +79,13 @@ SIGNATURES = {
     "sxgpu_bank_positions": (C.c_int, [_P, _P, _P, _P, _P]),
     "sxgpu_bank_playback": (C.c_int, [_P, C.c_uint32, C.c_int64, _S, _P, _P]),
     "sxgpu_bank_ring_frames": (C.c_int, [_P, C.POINTER(C.c_uint64)]),
+    "sxgpu_iir_create": (C.c_int, [_P, C.c_uint32, C.c_uint32, _P, C.POINTER(_P)]),
+    "sxgpu_iir_destroy": (C.c_int, [_P]),
+    "sxgpu_iir_set_state": (C.c_int, [_P, _P, _P]),
+    "sxgpu_iir_get_state": (C.c_int, [_P, _P, _P]),
+    "sxgpu_iir_apply": (C.c_int, [_P, _P, C.c_uint32, _P]),
+    "sxgpu_bank_repeat_filtered": (C.c_int, [_P, _P, _P, _P, C.c_longlong, _P]),
+    "sxgpu_iir_device_view": (C.c_int, [_P, _P, _S]),
     "sxgpu_convert_rx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S]),
     "sxgpu_convert_rx_buffer_host_gated": (C.c_int, [_P, _P, _S, _P, _S, _S, _P, _P]),
     "sxgpu_convert_tx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S, _F]),
@@ -327,6 +334,14 @@ class Bank:
         """read(d_cf32) then write(d_cf32, HAS_TIME, rx time + offset) in one launch."""
         self.ctx.check(self.lib.sxgpu_bank_repeat(self.handle, d_cf32, rx_time_offset_ns, stream), "sxgpu_bank_repeat")
 
+    def repeat_filtered(self, d_cf32, pre: "Iir | None" = None, post: "Iir | None" = None, rx_time_offset_ns=0,
+                        stream=None):
+        """repeat() with the channel filters: read, `pre` filter, `post` filter, timed write, in one
+        iteration that carries both filters' state (either may be None)."""
+        self.ctx.check(self.lib.sxgpu_bank_repeat_filtered(self.handle, pre.handle if pre else None,
+                                                           post.handle if post else None, d_cf32, rx_time_offset_ns,
+                                                           stream), "sxgpu_bank_repeat_filtered")
+
     def repeat_begin(self, d_cf32, stream=None):
         self.ctx.check(self.lib.sxgpu_bank_repeat_begin(self.handle, d_cf32, stream), "sxgpu_bank_repeat_begin")
 
@@ -367,6 +382,56 @@ class Bank:
         self.ctx.check(self.lib.sxgpu_bank_playback(self.handle, index, position, nframes, out.ctypes.data, stream),
                        "sxgpu_bank_playback")
         return out
+
+
+class Iir:
+    """A cascade of second-order sections with one state per stream (sxgpu_iir_* in include/sxgpu.h):
+    scipy.signal.sosfilt(sos, x, zi=state) along each stream's block, carried from call to call.
+    `sos` is what scipy's filter design functions return with output="sos": (nsections, 6)."""
+
+    def __init__(self, ctx: Context, nstreams: int, sos):
+        import numpy as np
+        self.np = np
+        self.ctx, self.lib = ctx, ctx.lib
+        self.handle = None
+        sos = np.ascontiguousarray(np.asarray(sos, dtype=np.float64))
+        if sos.ndim != 2 or sos.shape[1] != 6:
+            raise ValueError(f"sos must have shape (nsections, 6), got {sos.shape}")
+        h = _P()
+        ctx.check(self.lib.sxgpu_iir_create(ctx.handle, nstreams, sos.shape[0], sos.ctypes.data, C.byref(h)),
+                  "sxgpu_iir_create")
+        self.handle, self.nstreams, self.nsections = h, nstreams, sos.shape[0]
+
+    def close(self):
+        if self.handle:
+            self.lib.sxgpu_iir_destroy(self.handle)
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def apply(self, d_cf32, period, stream=None):
+        """Filter d_cf32[nstreams][period] (complex64 on the device) in place."""
+        self.ctx.check(self.lib.sxgpu_iir_apply(self.handle, d_cf32, period, stream), "sxgpu_iir_apply")
+
+    def state(self, stream=None):
+        """The state as scipy's zf: (nsections, nstreams, 2) complex64."""
+        zf = self.np.empty((self.nsections, self.nstreams, 2), self.np.complex64)
+        self.ctx.check(self.lib.sxgpu_iir_get_state(self.handle, zf.ctypes.data, stream), "sxgpu_iir_get_state")
+        return zf
+
+    def set_state(self, zi=None, stream=None):
+        """Set the state from scipy's zi layout, (nsections, nstreams, 2); None = zeros."""
+        ptr = None
+        if zi is not None:
+            zi = self.np.ascontiguousarray(zi, dtype=self.np.complex64)
+            if zi.shape != (self.nsections, self.nstreams, 2):
+                raise ValueError(f"zi must have shape {(self.nsections, self.nstreams, 2)}, got {zi.shape}")
+            ptr = zi.ctypes.data
+        self.ctx.check(self.lib.sxgpu_iir_set_state(self.handle, ptr, stream), "sxgpu_iir_set_state")
 
 
 class Multi:

@@ -35,6 +35,7 @@
 #pragma once
 
 #include "host/stream_plan.hpp"
+#include "sx_iir.cuh"
 #include "sx_kernels.cuh"
 #include "sx_time.h"
 
@@ -885,6 +886,137 @@ inline cudaError_t launch_bank_half_planned(const BankState &b, char *cf32, bool
     cfg.attrs = attr;
     cfg.numAttrs = programmatic ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, bank_repeat_data_kernel<U, IdentityHook, MODE>, b, cf32, capture_in_slot, IdentityHook());
+}
+
+// ---------------------------------------------------------------------------------------
+// The repeater iteration with its filters (sxgpu_bank_repeat_filtered, sx_hook.cuh): read, pre
+// cascade, the hook, post cascade, then the CF32 block and the timed write.  Same state, results,
+// CF32 block and playback ring as sxgpu_bank_read, sxgpu_iir_apply(pre), sxgpu_iir_apply(post) and
+// sxgpu_bank_write(HAS_TIME, rx time + offset) -- the filter state advances on every iteration,
+// also when the write is dropped as late, since the block is filtered before it is written.
+//
+// The decisions are bank_plan_repeat_kernel's, unchanged; this is the data kernel after it.  A
+// recurrence needs whole streams per CTA, so unlike bank_repeat_data_kernel (flat vectors) a CTA
+// takes kIirStreamsPerCta streams through the period in tiles of kIirTile frames (sx_iir.cuh):
+//   1. coalesced: the capture (synthesised and stored to the slot, or read from an ingested
+//      slot), RxCf32, into the tile's rows (a warp takes 16 vectors of two streams);
+//   2. the sequential pass: lane (stream, component) runs pre cascade, hook, post cascade;
+//   3. coalesced: the CF32 block stored, TxCf32, the ring stored -- by the same rules as the data
+//      kernel: a block that starts on a period boundary of the ring in vectors, one that straddles
+//      two slices frame by frame, nothing for a write dropped as late.
+// Needs an even period and a 16-byte aligned CF32 block.  Every bank size takes this schedule.
+// ---------------------------------------------------------------------------------------
+template <class Hook>
+__global__ void __launch_bounds__(kIirThreads) bank_repeat_iir_kernel(BankState b, char *cf32, bool capture_in_slot,
+                                                                      const __grid_constant__ IirView pre,
+                                                                      const __grid_constant__ IirView post, Hook hook)
+{
+    __shared__ __align__(16) float tile[kIirStreamsPerCta * kIirRow];
+    __shared__ long long s_first[kIirStreamsPerCta], s_off[kIirStreamsPerCta], s_at[kIirStreamsPerCta];
+    const uint32_t j = threadIdx.x >> 1, c = threadIdx.x & 1;
+    const uint64_t s0 = uint64_t(blockIdx.x) * kIirStreamsPerCta, s = s0 + j;
+    const uint32_t count = uint32_t(b.nstreams - s0 < kIirStreamsPerCta ? b.nstreams - s0 : kIirStreamsPerCta);
+    const bool active = j < count;
+    constexpr uint32_t kVecs = kIirTile / 2; // 16-byte vectors per row of a tile
+    pdl_wait(); // the decisions, and everything before them on the stream, are in memory
+    if (threadIdx.x < count) {
+        s_first[threadIdx.x] = b.rx_first_frame[s0 + threadIdx.x];
+        s_off[threadIdx.x] = b.tx_ring_offset[s0 + threadIdx.x];
+        s_at[threadIdx.x] = b.tx_write_position[s0 + threadIdx.x];
+    }
+    float zp[kIirMaxSections][2], zq[kIirMaxSections][2];
+    iir_load_state(pre, s, c, active, zp);
+    iir_load_state(post, s, c, active, zq);
+    __syncthreads();
+
+    for (uint32_t t0 = 0; t0 < b.period; t0 += kIirTile) {
+        const uint32_t n = b.period - t0 < kIirTile ? b.period - t0 : kIirTile; // even
+        for (uint32_t q = threadIdx.x; q < count * kVecs; q += kIirThreads) {
+            const uint32_t r = q / kVecs, m = q % kVecs;
+            if (2 * m >= n)
+                continue;
+            char *slot = b.capture_stage + ((s0 + r) * b.period + t0 + 2 * m) * 8;
+            Pack<4> cap, mid;
+            if (capture_in_slot) {
+                cap = ld_stream<16>(slot);
+            } else {
+                const uint64_t first = uint64_t(s_first[r]) + t0 + 2 * m;
+                const uint64_t z0 = sx_synth_frame(b.seed + s0 + r, first), z1 = sx_synth_frame(b.seed + s0 + r, first + 1);
+                cap.w[0] = uint32_t(z0), cap.w[1] = uint32_t(z0 >> 32);
+                cap.w[2] = uint32_t(z1), cap.w[3] = uint32_t(z1 >> 32);
+                st_stream<16>(slot, cap);
+            }
+            RxCf32::apply<2>(cap, mid, 0.0f);
+            *reinterpret_cast<Pack<4> *>(&tile[r * kIirRow + 4 * m]) = mid;
+        }
+        __syncthreads();
+        if constexpr (std::is_same<Hook, IdentityHook>::value)
+            iir_tile_pass<2>(&tile[j * kIirRow], c, n, pre.k, zp, post.k, zq, NoIirHook(), s, active, t0);
+        else
+            iir_tile_pass<2>(&tile[j * kIirRow], c, n, pre.k, zp, post.k, zq, hook, s, active, t0);
+        __syncthreads();
+        for (uint32_t q = threadIdx.x; q < count * kVecs; q += kIirThreads) {
+            const uint32_t r = q / kVecs, m = q % kVecs;
+            if (2 * m >= n)
+                continue;
+            const Pack<4> mid = *reinterpret_cast<const Pack<4> *>(&tile[r * kIirRow + 4 * m]);
+            const uint64_t v = t0 / 2 + m; // vector index within the block
+            st_stream<16>(cf32 + ((s0 + r) * b.period) * 8 + v * 16, mid);
+            const long long off = s_off[r];
+            if (off < 0)
+                continue; // discarded as late
+            Pack<4> out;
+            TxCf32::apply<2>(mid, out, b.thr2);
+            if ((off & 1) == 0) {
+                st_stream<16>(b.playback_ring + off + v * 16, out);
+            } else { // straddles two slices of the time-major ring: frame by frame
+                const uint64_t at = uint64_t(s_at[r]);
+                Pack<2> f0, f1;
+                f0.w[0] = out.w[0], f0.w[1] = out.w[1], f1.w[0] = out.w[2], f1.w[1] = out.w[3];
+                st_stream<8>(ring_frame(b, s0 + r, at + 2 * v), f0);
+                st_stream<8>(ring_frame(b, s0 + r, at + 2 * v + 1), f1);
+            }
+        }
+        __syncthreads(); // the next tile overwrites the rows
+    }
+    iir_store_state(pre, s, c, active, zp);
+    iir_store_state(post, s, c, active, zq);
+}
+
+// Why a filtered iteration's arguments are refused (nullptr: they are not).  A stage left out has
+// nsections == 0.
+inline const char *bank_repeat_iir_invalid(const BankState &b, const void *cf32, const IirView &pre, const IirView &post)
+{
+    if (!cf32 || reinterpret_cast<uintptr_t>(cf32) % 16)
+        return "the filtered iteration needs a 16-byte aligned CF32 buffer";
+    if (b.period % 2)
+        return "the filtered iteration needs an even period";
+    if ((pre.k.nsections && pre.nstreams != b.nstreams) || (post.k.nsections && post.nstreams != b.nstreams))
+        return "a filter must have as many streams as the bank";
+    if (pre.k.nsections && post.k.nsections && pre.state == post.state)
+        return "the two stages cannot share one filter (and its state)";
+    return nullptr;
+}
+
+// bank_plan_repeat_kernel, then bank_repeat_iir_kernel as its programmatic dependent.
+template <class Hook>
+inline cudaError_t launch_bank_repeat_iir(const BankState &b, char *cf32, long long rx_time_offset_ns, bool capture_in_slot,
+                                          const IirView &pre, const IirView &post, cudaStream_t st, const Hook &hook)
+{
+    bank_plan_repeat_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, cf32, rx_time_offset_ns);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess)
+        return e;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(unsigned((uint64_t(b.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta));
+    cfg.blockDim = dim3(kIirThreads);
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, bank_repeat_iir_kernel<Hook>, b, cf32, capture_in_slot, pre, post, hook);
 }
 
 __global__ void bank_advance_kernel(BankState b, long long frames)

@@ -8,6 +8,7 @@
 
 #include "sx_kernels.cuh"
 #include "sx_bank.cuh"
+#include "sx_iir.cuh"
 #include "sx_resident.cuh"
 #include "host/par_copy.hpp"
 #include "host/worker_pool.hpp"
@@ -15,6 +16,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -123,6 +125,7 @@ struct sxgpu_ctx {
 
     std::atomic<uint64_t> resident_launches{0}, resident_calls{0}, flagged_calls{0};
     std::atomic<int> live_banks{0}; // banks keep a pointer to their context
+    std::atomic<int> live_iirs{0};  // so do filters
     bool l2_carveout_set = false;   // sxgpu_bank_repeat_begin sets the persisting-L2 limit once
 
     // host pipeline: lane 0 serves the RX conversions, lane 1 the TX conversions
@@ -1460,6 +1463,8 @@ int sxgpu_destroy(sxgpu_ctx *ctx)
         return SXGPU_ERR_INVALID;
     if (ctx->live_banks.load() != 0)
         return ctx->invalid("destroy the context's stream banks first");
+    if (ctx->live_iirs.load() != 0)
+        return ctx->invalid("destroy the context's filters first");
     cudaSetDevice(ctx->device);
     for (HostLane &lane : ctx->lanes) {
         std::lock_guard<std::mutex> lock(lane.mutex);
@@ -2142,6 +2147,182 @@ int sxgpu_bank_playback(sxgpu_bank *bank, uint32_t index, int64_t position, size
         return ctx->fail(e, "sxgpu_bank_playback");
     ctx->launches++;
     SX_CUDA(ctx, cudaStreamSynchronize(st));
+    return SXGPU_OK;
+}
+
+// ---- stateful IIR filters (sx_iir.cuh) --------------------------------------------------------
+} // extern "C"
+
+struct sxgpu_iir {
+    sxgpu_ctx *ctx = nullptr;
+    IirView view = {}; // the state in device memory and the float32 coefficients
+};
+
+namespace {
+
+size_t iir_state_bytes(const IirView &v)
+{
+    return size_t(v.k.nsections) * v.nstreams * 16; // two complex64 values per section and stream
+}
+
+cudaStream_t iir_stream(sxgpu_iir *f, sxgpu_stream stream)
+{
+    return stream ? static_cast<cudaStream_t>(stream) : f->ctx->stream;
+}
+
+// A stage of the filtered iteration: the filter's view, or no sections for a stage left out.
+IirView iir_stage(const sxgpu_iir *f)
+{
+    IirView v = {};
+    if (f)
+        v = f->view;
+    return v;
+}
+
+} // namespace
+
+extern "C" {
+
+int sxgpu_iir_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t nsections, const double *sos, sxgpu_iir **out)
+{
+    if (!ctx || !out)
+        return SXGPU_ERR_INVALID;
+    *out = nullptr;
+    if (nstreams == 0)
+        return ctx->invalid("a filter needs at least one stream");
+    if (nsections < 1 || nsections > SXGPU_IIR_MAX_SECTIONS || !sos)
+        return ctx->invalid("a filter has 1 to SXGPU_IIR_MAX_SECTIONS second-order sections");
+    IirView v = {};
+    v.nstreams = nstreams;
+    v.k.nsections = nsections;
+    for (uint32_t q = 0; q < nsections; q++) {
+        const double *row = sos + size_t(q) * 6;
+        for (int i = 0; i < 6; i++)
+            if (!std::isfinite(row[i]))
+                return ctx->invalid("every filter coefficient must be finite");
+        if (row[3] != 1.0)
+            return ctx->invalid("a0 of every section must be 1 (scipy's sos layout: b0 b1 b2 a0 a1 a2)");
+        v.k.b0[q] = float(row[0]);
+        v.k.b1[q] = float(row[1]);
+        v.k.b2[q] = float(row[2]);
+        v.k.a1[q] = float(row[4]);
+        v.k.a2[q] = float(row[5]);
+    }
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t bytes = iir_state_bytes(v);
+    void *state = nullptr;
+    cudaError_t e = cudaMalloc(&state, bytes);
+    if (e != cudaSuccess)
+        return ctx->fail(e, "cudaMalloc(filter state)");
+    e = cudaMemsetAsync(state, 0, bytes, ctx->stream);
+    if (e == cudaSuccess)
+        e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) {
+        cudaFree(state);
+        return ctx->fail(e, "cudaMemset(filter state)");
+    }
+    v.state = static_cast<float *>(state);
+    sxgpu_iir *f = new sxgpu_iir();
+    f->ctx = ctx;
+    f->view = v;
+    ctx->live_iirs++;
+    *out = f;
+    return SXGPU_OK;
+}
+
+int sxgpu_iir_destroy(sxgpu_iir *f)
+{
+    if (!f)
+        return SXGPU_ERR_INVALID;
+    cudaSetDevice(f->ctx->device);
+    for (HostLane &lane : f->ctx->lanes) { // a resident converter would hold the device-wide sync up
+        std::lock_guard<std::mutex> lock(lane.mutex);
+        resident_stop(f->ctx, lane);
+    }
+    cudaDeviceSynchronize();
+    cudaFree(f->view.state);
+    f->ctx->live_iirs--;
+    delete f;
+    return SXGPU_OK;
+}
+
+int sxgpu_iir_set_state(sxgpu_iir *f, const void *h_zi, sxgpu_stream stream)
+{
+    if (!f)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = f->ctx;
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = iir_stream(f, stream);
+    const size_t bytes = iir_state_bytes(f->view);
+    if (h_zi)
+        SX_CUDA(ctx, cudaMemcpyAsync(f->view.state, h_zi, bytes, cudaMemcpyHostToDevice, st));
+    else
+        SX_CUDA(ctx, cudaMemsetAsync(f->view.state, 0, bytes, st));
+    SX_CUDA(ctx, cudaStreamSynchronize(st));
+    return SXGPU_OK;
+}
+
+int sxgpu_iir_get_state(sxgpu_iir *f, void *h_zf, sxgpu_stream stream)
+{
+    if (!f || !h_zf)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = f->ctx;
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = iir_stream(f, stream);
+    SX_CUDA(ctx, cudaMemcpyAsync(h_zf, f->view.state, iir_state_bytes(f->view), cudaMemcpyDeviceToHost, st));
+    SX_CUDA(ctx, cudaStreamSynchronize(st));
+    return SXGPU_OK;
+}
+
+int sxgpu_iir_apply(sxgpu_iir *f, void *d_cf32, uint32_t period, sxgpu_stream stream)
+{
+    if (!f)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = f->ctx;
+    if (!d_cf32 || reinterpret_cast<uintptr_t>(d_cf32) % 8)
+        return ctx->invalid("CF32 buffer must be 8-byte aligned device memory");
+    if (period < 1 || period > 65536)
+        return ctx->invalid("the period is 1 to 65536 frames");
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const unsigned grid = unsigned((uint64_t(f->view.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta);
+    iir_apply_kernel<<<grid, kIirThreads, 0, iir_stream(f, stream)>>>(f->view, static_cast<char *>(d_cf32), period);
+    SX_CUDA(ctx, cudaGetLastError());
+    ctx->launches++;
+    return SXGPU_OK;
+}
+
+int sxgpu_bank_repeat_filtered(sxgpu_bank *bank, sxgpu_iir *pre, sxgpu_iir *post, void *d_cf32,
+                               long long rx_time_offset_ns, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = bank->ctx;
+    if ((pre && pre->ctx != ctx) || (post && post->ctx != ctx))
+        return ctx->invalid("a filter belongs to another context");
+    if (pre && pre == post)
+        return ctx->invalid("the two stages cannot share one filter (and its state)");
+    const IirView vpre = iir_stage(pre), vpost = iir_stage(post);
+    if (const char *why = bank_repeat_iir_invalid(bank->st, d_cf32, vpre, vpost))
+        return ctx->invalid(why);
+    if (!pre && !post)
+        return sxgpu_bank_repeat(bank, d_cf32, rx_time_offset_ns, stream);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const BankState &b = bank->st;
+    SX_CUDA(ctx, launch_bank_repeat_iir(b, static_cast<char *>(d_cf32), rx_time_offset_ns, bank->external_capture, vpre,
+                                        vpost, bank_stream(bank, stream), IdentityHook()));
+    ctx->launches += 2;
+    ctx->frames_rx += uint64_t(b.nstreams) * b.period;
+    ctx->frames_tx += uint64_t(b.nstreams) * b.period;
+    return SXGPU_OK;
+}
+
+int sxgpu_iir_device_view(sxgpu_iir *f, void *out, size_t out_bytes)
+{
+    if (!f || !out)
+        return SXGPU_ERR_INVALID;
+    if (out_bytes != sizeof(IirView))
+        return f->ctx->invalid("sxgpu_iir_device_view: size mismatch (header and library disagree)");
+    std::memcpy(out, &f->view, sizeof(IirView));
     return SXGPU_OK;
 }
 
