@@ -246,6 +246,21 @@ int sxgpu_iir_apply(sxgpu_iir *f, void *d_cf32, uint32_t period, sxgpu_stream st
  * of the bank's stream count, two different filters, an even period and a 16-byte aligned d_cf32. */
 int sxgpu_bank_repeat_filtered(sxgpu_bank *bank, sxgpu_iir *pre, sxgpu_iir *post, void *d_cf32,
                                long long rx_time_offset_ns, sxgpu_stream stream);
+/* The two halves with a filter fused in, for a bank used only as receivers or only as transmitters,
+ * and for the repeater split around DSP of the caller's own: read_filtered(pre), the caller's
+ * kernels on d_cf32, then write_filtered(post, SOAPY_SDR_HAS_TIME, NULL, rx_time_offset_ns) is the
+ * filtered repeater iteration with that DSP between its filters.  Each is one pass over the CF32
+ * block instead of two.  Same requirements as sxgpu_bank_repeat_filtered: a filter of this context
+ * with the bank's stream count, an even period and a 16-byte aligned d_cf32 (checked also when f is
+ * NULL).
+ * sxgpu_bank_read, then sxgpu_iir_apply(f, d_cf32, period): the same state, results, positions,
+ * capture and CF32 block, bit for bit, in one pass.  f NULL: exactly sxgpu_bank_read. */
+int sxgpu_bank_read_filtered(sxgpu_bank *bank, sxgpu_iir *f, void *d_cf32, sxgpu_stream stream);
+/* The caller's block filtered by f and then written as sxgpu_bank_write(bank, ., flags, d_time_ns,
+ * rx_time_offset_ns) would write it.  d_cf32 is not modified.  f's state advances also when a
+ * stream's write is dropped as late.  f NULL: exactly sxgpu_bank_write. */
+int sxgpu_bank_write_filtered(sxgpu_bank *bank, sxgpu_iir *f, const void *d_cf32, int flags,
+                              const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream);
 /* For include/sx_hook.cuh, like sxgpu_bank_device_view: the filter's device-side view (struct
  * sx::IirView).  out_bytes must be sizeof(sx::IirView). */
 int sxgpu_iir_device_view(sxgpu_iir *f, void *out, size_t out_bytes);

@@ -85,6 +85,8 @@ SIGNATURES = {
     "sxgpu_iir_get_state": (C.c_int, [_P, _P, _P]),
     "sxgpu_iir_apply": (C.c_int, [_P, _P, C.c_uint32, _P]),
     "sxgpu_bank_repeat_filtered": (C.c_int, [_P, _P, _P, _P, C.c_longlong, _P]),
+    "sxgpu_bank_read_filtered": (C.c_int, [_P, _P, _P, _P]),
+    "sxgpu_bank_write_filtered": (C.c_int, [_P, _P, _P, C.c_int, _P, C.c_longlong, _P]),
     "sxgpu_iir_device_view": (C.c_int, [_P, _P, _S]),
     "sxgpu_convert_rx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S]),
     "sxgpu_convert_rx_buffer_host_gated": (C.c_int, [_P, _P, _S, _P, _S, _S, _P, _P]),
@@ -341,6 +343,16 @@ class Bank:
         self.ctx.check(self.lib.sxgpu_bank_repeat_filtered(self.handle, pre.handle if pre else None,
                                                            post.handle if post else None, d_cf32, rx_time_offset_ns,
                                                            stream), "sxgpu_bank_repeat_filtered")
+
+    def read_filtered(self, d_cf32, f: "Iir | None", stream=None):
+        """read(d_cf32) then f.apply(d_cf32, period) in one pass (f None: read)."""
+        self.ctx.check(self.lib.sxgpu_bank_read_filtered(self.handle, f.handle if f else None, d_cf32, stream),
+                       "sxgpu_bank_read_filtered")
+
+    def write_filtered(self, d_cf32, f: "Iir | None", flags=4, d_time_ns=None, rx_time_offset_ns=0, stream=None):
+        """write() of d_cf32 filtered by f, in one pass that leaves d_cf32 as it was (f None: write)."""
+        self.ctx.check(self.lib.sxgpu_bank_write_filtered(self.handle, f.handle if f else None, d_cf32, flags, d_time_ns,
+                                                          rx_time_offset_ns, stream), "sxgpu_bank_write_filtered")
 
     def repeat_begin(self, d_cf32, stream=None):
         self.ctx.check(self.lib.sxgpu_bank_repeat_begin(self.handle, d_cf32, stream), "sxgpu_bank_repeat_begin")

@@ -905,8 +905,14 @@ inline cudaError_t launch_bank_half_planned(const BankState &b, char *cf32, bool
 //      kernel: a block that starts on a period boundary of the ring in vectors, one that straddles
 //      two slices frame by frame, nothing for a write dropped as late.
 // Needs an even period and a 16-byte aligned CF32 block.  Every bank size takes this schedule.
+//
+// MODE: the whole iteration, or one half of it with one filter (`pre`; `post` is not used) for the
+// separate calls -- sxgpu_bank_read_filtered after bank_plan_read_kernel: pass 1 as above, the
+// cascade, the CF32 block stored; sxgpu_bank_write_filtered after bank_plan_write_kernel(...,
+// for_data_kernel = true): the caller's CF32 block loaded, the cascade, TxCf32 and the ring by the
+// rules above, and the block itself left as it was.
 // ---------------------------------------------------------------------------------------
-template <class Hook>
+template <class Hook, int MODE = kBankModeRepeat>
 __global__ void __launch_bounds__(kIirThreads) bank_repeat_iir_kernel(BankState b, char *cf32, bool capture_in_slot,
                                                                       const __grid_constant__ IirView pre,
                                                                       const __grid_constant__ IirView post, Hook hook)
@@ -920,13 +926,17 @@ __global__ void __launch_bounds__(kIirThreads) bank_repeat_iir_kernel(BankState 
     constexpr uint32_t kVecs = kIirTile / 2; // 16-byte vectors per row of a tile
     pdl_wait(); // the decisions, and everything before them on the stream, are in memory
     if (threadIdx.x < count) {
-        s_first[threadIdx.x] = b.rx_first_frame[s0 + threadIdx.x];
-        s_off[threadIdx.x] = b.tx_ring_offset[s0 + threadIdx.x];
-        s_at[threadIdx.x] = b.tx_write_position[s0 + threadIdx.x];
+        if (MODE != kBankModeWrite)
+            s_first[threadIdx.x] = b.rx_first_frame[s0 + threadIdx.x];
+        if (MODE != kBankModeRead) {
+            s_off[threadIdx.x] = b.tx_ring_offset[s0 + threadIdx.x];
+            s_at[threadIdx.x] = b.tx_write_position[s0 + threadIdx.x];
+        }
     }
     float zp[kIirMaxSections][2], zq[kIirMaxSections][2];
     iir_load_state(pre, s, c, active, zp);
-    iir_load_state(post, s, c, active, zq);
+    if (MODE == kBankModeRepeat)
+        iir_load_state(post, s, c, active, zq);
     __syncthreads();
 
     for (uint32_t t0 = 0; t0 < b.period; t0 += kIirTile) {
@@ -935,25 +945,35 @@ __global__ void __launch_bounds__(kIirThreads) bank_repeat_iir_kernel(BankState 
             const uint32_t r = q / kVecs, m = q % kVecs;
             if (2 * m >= n)
                 continue;
-            char *slot = b.capture_stage + ((s0 + r) * b.period + t0 + 2 * m) * 8;
-            Pack<4> cap, mid;
-            if (capture_in_slot) {
-                cap = ld_stream<16>(slot);
+            Pack<4> mid;
+            if (MODE == kBankModeWrite) {
+                mid = ld_stream<16>(cf32 + ((s0 + r) * b.period + t0 + 2 * m) * 8);
             } else {
-                const uint64_t first = uint64_t(s_first[r]) + t0 + 2 * m;
-                const uint64_t z0 = sx_synth_frame(b.seed + s0 + r, first), z1 = sx_synth_frame(b.seed + s0 + r, first + 1);
-                cap.w[0] = uint32_t(z0), cap.w[1] = uint32_t(z0 >> 32);
-                cap.w[2] = uint32_t(z1), cap.w[3] = uint32_t(z1 >> 32);
-                st_stream<16>(slot, cap);
+                char *slot = b.capture_stage + ((s0 + r) * b.period + t0 + 2 * m) * 8;
+                Pack<4> cap;
+                if (capture_in_slot) {
+                    cap = ld_stream<16>(slot);
+                } else {
+                    const uint64_t first = uint64_t(s_first[r]) + t0 + 2 * m;
+                    const uint64_t z0 = sx_synth_frame(b.seed + s0 + r, first), z1 = sx_synth_frame(b.seed + s0 + r, first + 1);
+                    cap.w[0] = uint32_t(z0), cap.w[1] = uint32_t(z0 >> 32);
+                    cap.w[2] = uint32_t(z1), cap.w[3] = uint32_t(z1 >> 32);
+                    st_stream<16>(slot, cap);
+                }
+                RxCf32::apply<2>(cap, mid, 0.0f);
             }
-            RxCf32::apply<2>(cap, mid, 0.0f);
             *reinterpret_cast<Pack<4> *>(&tile[r * kIirRow + 4 * m]) = mid;
         }
         __syncthreads();
-        if constexpr (std::is_same<Hook, IdentityHook>::value)
+        if constexpr (MODE != kBankModeRepeat) {
+            IirCoeffs none; // a half runs one cascade
+            none.nsections = 0;
+            iir_tile_pass<2>(&tile[j * kIirRow], c, n, pre.k, zp, none, zq, NoIirHook(), s, active, t0);
+        } else if constexpr (std::is_same<Hook, IdentityHook>::value) {
             iir_tile_pass<2>(&tile[j * kIirRow], c, n, pre.k, zp, post.k, zq, NoIirHook(), s, active, t0);
-        else
+        } else {
             iir_tile_pass<2>(&tile[j * kIirRow], c, n, pre.k, zp, post.k, zq, hook, s, active, t0);
+        }
         __syncthreads();
         for (uint32_t q = threadIdx.x; q < count * kVecs; q += kIirThreads) {
             const uint32_t r = q / kVecs, m = q % kVecs;
@@ -961,7 +981,10 @@ __global__ void __launch_bounds__(kIirThreads) bank_repeat_iir_kernel(BankState 
                 continue;
             const Pack<4> mid = *reinterpret_cast<const Pack<4> *>(&tile[r * kIirRow + 4 * m]);
             const uint64_t v = t0 / 2 + m; // vector index within the block
-            st_stream<16>(cf32 + ((s0 + r) * b.period) * 8 + v * 16, mid);
+            if (MODE != kBankModeWrite)
+                st_stream<16>(cf32 + ((s0 + r) * b.period) * 8 + v * 16, mid);
+            if (MODE == kBankModeRead)
+                continue;
             const long long off = s_off[r];
             if (off < 0)
                 continue; // discarded as late
@@ -980,7 +1003,8 @@ __global__ void __launch_bounds__(kIirThreads) bank_repeat_iir_kernel(BankState 
         __syncthreads(); // the next tile overwrites the rows
     }
     iir_store_state(pre, s, c, active, zp);
-    iir_store_state(post, s, c, active, zq);
+    if (MODE == kBankModeRepeat)
+        iir_store_state(post, s, c, active, zq);
 }
 
 // Why a filtered iteration's arguments are refused (nullptr: they are not).  A stage left out has
@@ -1017,6 +1041,33 @@ inline cudaError_t launch_bank_repeat_iir(const BankState &b, char *cf32, long l
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, bank_repeat_iir_kernel<Hook>, b, cf32, capture_in_slot, pre, post, hook);
+}
+
+// One half with its filter (sxgpu_bank_read_filtered / sxgpu_bank_write_filtered): the matching
+// plan kernel, then bank_repeat_iir_kernel in that mode as its programmatic dependent.  One
+// schedule for every bank size, as for the whole iteration.
+template <int MODE>
+inline cudaError_t launch_bank_half_iir(const BankState &b, char *cf32, bool capture_in_slot, int flags, const long long *time_ns,
+                                        long long rx_time_offset_ns, const IirView &f, cudaStream_t st)
+{
+    if (MODE == kBankModeRead)
+        bank_plan_read_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, cf32);
+    else
+        bank_plan_write_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, flags, time_ns, rx_time_offset_ns, true);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess)
+        return e;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(unsigned((uint64_t(b.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta));
+    cfg.blockDim = dim3(kIirThreads);
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, bank_repeat_iir_kernel<IdentityHook, MODE>, b, cf32, capture_in_slot, f, IirView{},
+                              IdentityHook());
 }
 
 __global__ void bank_advance_kernel(BankState b, long long frames)

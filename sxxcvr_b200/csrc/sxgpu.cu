@@ -2316,6 +2316,50 @@ int sxgpu_bank_repeat_filtered(sxgpu_bank *bank, sxgpu_iir *pre, sxgpu_iir *post
     return SXGPU_OK;
 }
 
+int sxgpu_bank_read_filtered(sxgpu_bank *bank, sxgpu_iir *f, void *d_cf32, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = bank->ctx;
+    if (f && f->ctx != ctx)
+        return ctx->invalid("a filter belongs to another context");
+    const IirView v = iir_stage(f);
+    if (const char *why = bank_repeat_iir_invalid(bank->st, d_cf32, v, IirView{}))
+        return ctx->invalid(why);
+    if (!f)
+        return sxgpu_bank_read(bank, d_cf32, stream);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const BankState &b = bank->st;
+    SX_CUDA(ctx, launch_bank_half_iir<kBankModeRead>(b, static_cast<char *>(d_cf32), bank->external_capture, 0, nullptr, 0, v,
+                                                     bank_stream(bank, stream)));
+    ctx->launches += 2;
+    ctx->frames_rx += uint64_t(b.nstreams) * b.period;
+    return SXGPU_OK;
+}
+
+int sxgpu_bank_write_filtered(sxgpu_bank *bank, sxgpu_iir *f, const void *d_cf32, int flags, const long long *d_time_ns,
+                              long long rx_time_offset_ns, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = bank->ctx;
+    if (f && f->ctx != ctx)
+        return ctx->invalid("a filter belongs to another context");
+    const IirView v = iir_stage(f);
+    if (const char *why = bank_repeat_iir_invalid(bank->st, d_cf32, v, IirView{}))
+        return ctx->invalid(why);
+    if (!f)
+        return sxgpu_bank_write(bank, d_cf32, flags, d_time_ns, rx_time_offset_ns, stream);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const BankState &b = bank->st;
+    // the kernel only loads from the block in this mode
+    SX_CUDA(ctx, launch_bank_half_iir<kBankModeWrite>(b, const_cast<char *>(static_cast<const char *>(d_cf32)), false, flags,
+                                                      d_time_ns, rx_time_offset_ns, v, bank_stream(bank, stream)));
+    ctx->launches += 2;
+    ctx->frames_tx += uint64_t(b.nstreams) * b.period;
+    return SXGPU_OK;
+}
+
 int sxgpu_iir_device_view(sxgpu_iir *f, void *out, size_t out_bytes)
 {
     if (!f || !out)
