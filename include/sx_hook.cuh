@@ -59,7 +59,10 @@ inline int bank_repeat_with(sxgpu_bank *bank, void *d_cf32, long long rx_time_of
     if (cudaGetDevice(&device) != cudaSuccess ||
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess)
         return SXGPU_ERR_CUDA;
-    // Same schedule choice as the library's own fused iteration: K streams per warp round.
+    // Below the large-bank size: K streams per warp round (K = 1 up to 2048 streams, 2 up to 16384,
+    // 4 above), always with the intermediates in registers, because only that form has a hook
+    // point.  This is not the library's own choice from 2 049 streams up: sxgpu_bank_repeat takes
+    // the memory-staged form there (K = 2 up to 8192, 4 up to 32768, then 32 streams per CTA).
     auto launch = [&](auto kernel, uint64_t k) -> int {
         int per_sm = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, 0) != cudaSuccess || per_sm < 1)
@@ -72,15 +75,15 @@ inline int bank_repeat_with(sxgpu_bank *bank, void *d_cf32, long long rx_time_of
         return cudaGetLastError() == cudaSuccess ? SXGPU_OK : SXGPU_ERR_CUDA;
     };
     if (bank_is_large(view)) // the library's own choice for large banks: decisions first, then the samples
-        return launch_bank_repeat_planned<2>(view, static_cast<char *>(d_cf32), rx_time_offset_ns, external != 0, stream, hook) ==
-                       cudaSuccess
+        return launch_bank_planned<kBankModeRepeat, 2>(view, static_cast<char *>(d_cf32), external != 0, SX_HAS_TIME, nullptr,
+                                                       rx_time_offset_ns, stream, hook) == cudaSuccess
                    ? SXGPU_OK
                    : SXGPU_ERR_CUDA;
     if (view.nstreams <= 2048)
-        return launch(bank_repeat_reg_kernel<1, Hook>, 1);
+        return launch(bank_repeat_warp_kernel<1, true, Hook>, 1);
     if (view.nstreams <= 16384)
-        return launch(bank_repeat_reg_kernel<2, Hook>, 2);
-    return launch(bank_repeat_reg_kernel<4, Hook>, 4);
+        return launch(bank_repeat_warp_kernel<2, true, Hook>, 2);
+    return launch(bank_repeat_warp_kernel<4, true, Hook>, 4);
 }
 
 // The same iteration with the reference's channel filters around the functor: read -> `pre`
@@ -108,8 +111,8 @@ inline int bank_repeat_with(sxgpu_bank *bank, void *d_cf32, long long rx_time_of
         return SXGPU_ERR_INVALID;
     if (!pre && !post)
         return bank_repeat_with(bank, d_cf32, rx_time_offset_ns, stream, hook);
-    return launch_bank_repeat_iir(view, static_cast<char *>(d_cf32), rx_time_offset_ns, external != 0, vpre, vpost, stream,
-                                  hook) == cudaSuccess
+    return launch_bank_iir<kBankModeRepeat>(view, static_cast<char *>(d_cf32), external != 0, SX_HAS_TIME, nullptr,
+                                            rx_time_offset_ns, vpre, vpost, stream, hook) == cudaSuccess
                ? SXGPU_OK
                : SXGPU_ERR_CUDA;
 }

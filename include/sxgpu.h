@@ -385,15 +385,13 @@ int sxgpu_multi_sync(sxgpu_multi *m);
  *                               leaves after 2 ms without work, after 20 ms in any case, and at
  *                               once when the library is about to synchronise the device
  *   "bank_repeat_variant"       schedule of sxgpu_bank_repeat: 0 = auto (by stream count),
- *                               K in {1, 2, 4, 8} = a warp takes K streams per round, stage by
+ *                               K in {1, 2, 4} = a warp takes K streams per round, stage by
  *                               stage through memory; 100 = a CTA takes 32 streams per round;
  *                               200 + K, K in {1, 2, 4} = a warp takes K streams per round and
- *                               keeps every intermediate in registers (stores only); 300, 302,
- *                               303 = the same with a CTA's first warp deciding for 32 streams;
+ *                               keeps every intermediate in registers (stores only);
  *                               600, 604 = decisions by a thread-per-stream kernel, then
  *                               the samples by CTAs that take one chunk each (2 or 4 vectors per
  *                               thread), the second kernel a programmatic dependent of the first
- *                               ("bank_pdl" = 0 turns that off)
  *   "batch_variant"             blocks above 4096 frames in sxgpu_convert_*_batch: 0 = auto
  *                               (2 when the blocks are of similar length, else 3), 1 = slices of
  *                               CTAs on vector accesses, 2 = one chunk per CTA in block-then-chunk

@@ -20,16 +20,23 @@
 //                             forwarded-over gaps + the conversion into the playback ring
 // and, for the repeater pattern (read, then a timed write of the block just read), all of the
 // above in one launch:
-//     bank_repeat_warp_kernel<K> / bank_repeat_kernel   K lanes decide for K streams from
+//     bank_repeat_warp_kernel<K, IN_REGISTERS, Hook>   K lanes decide for K streams from
 //                             registers, then the warp takes each stream through the three
-//                             stages back to back, each stage reading from L2 what the previous
-//                             one has just written
+//                             stages back to back: stage by stage through memory (each stage
+//                             reading from L2 what the previous one has just written), or with
+//                             every intermediate in registers and only the stores (the form
+//                             with a hook point, sx_hook.cuh)
+//     bank_repeat_kernel      the memory-staged form with a CTA's first warp deciding for 32 streams
 // Large banks (bank_is_large: bound by HBM, not by launch latency) run every call -- the fused
 // iteration and the separate read and write -- as two kernels instead:
 //     bank_plan_{repeat,read,write}_kernel   the decisions, one thread per stream
 //     bank_repeat_data_kernel<U, Hook, MODE> the samples: one chunk of vectors per CTA, CTAs handed
 //                             out in order by the hardware, every intermediate in registers,
 //                             launched as a programmatic dependent of the plan kernel
+// and the iteration or a half of it with IIR filters (every bank size) as:
+//     bank_plan_{repeat,read,write}_kernel, then bank_repeat_iir_kernel<Hook, MODE>: whole
+//                             streams per CTA through shared-memory tiles, as a programmatic
+//                             dependent of the plan kernel
 // The virtual clock follows the same rule as the host-side ALSA stand-in: it moves when a
 // blocking transfer must wait (by exactly the deficit) or when the owner advances it.
 #pragma once
@@ -77,10 +84,8 @@ struct BankState {
     long long *tx_write_position;
     long long *tx_gap_start; // forwarded-over region to be silenced
     long long *tx_gap_length;
-    long long *tx_ring_offset; // byte offset in playback_ring of the block's first frame (a multiple of 8),
-                               // + 1 when the block does not start on a period boundary of the ring (it then
-                               // spans two slices); -1: discarded as late.  Written by
-                               // bank_plan_repeat_kernel for the data kernels.
+    long long *tx_ring_offset; // the block's place in playback_ring, see bank_ring_offset(); written by the
+                               // plan kernels for the data kernels
 
     char *capture_stage; // [nstreams][period] I2S frames
     char *playback_ring; // [ring / period][nstreams][period] I2S frames, see ring_frame()
@@ -103,6 +108,72 @@ __device__ __forceinline__ char *ring_frame(const BankState &b, uint64_t s, uint
     }
     const uint64_t slice = (pos / b.period) % (b.ring / b.period);
     return b.playback_ring + ((slice * b.nstreams + s) * b.period + pos % b.period) * 8;
+}
+
+// What the data kernels find in tx_ring_offset[s] for a block written at counter `at`: the byte
+// offset in playback_ring of its first frame (a multiple of 8), + 1 when the block does not start
+// on a period boundary of the ring (it then spans two slices); -1 when it was discarded as late.
+__device__ __forceinline__ long long bank_ring_offset(const BankState &b, uint64_t s, long long at)
+{
+    return at >= 0 ? (long long)(ring_frame(b, s, uint64_t(at)) - b.playback_ring) + (uint64_t(at) % b.period != 0 ? 1 : 0)
+                   : -1;
+}
+
+// Two converted frames, at and at + 1, into stream s's ring one by one: the store of a block that
+// straddles two slices of the time-major ring (rare: a stream out of step).
+__device__ __forceinline__ void ring_store_pair(const BankState &b, uint64_t s, uint64_t at, const Pack<4> &out)
+{
+    Pack<2> f0, f1;
+    f0.w[0] = out.w[0], f0.w[1] = out.w[1], f1.w[0] = out.w[2], f1.w[1] = out.w[3];
+    st_stream<8>(ring_frame(b, s, at), f0);
+    st_stream<8>(ring_frame(b, s, at + 1), f1);
+}
+
+// The stand-in I2S DMA: capture frame k of the stream whose generator is seeded with `seed`
+// (the bank's seed + the stream's index) as one I2S frame, and frames k, k + 1 as one vector.
+__device__ __forceinline__ Pack<2> capture_frame(uint64_t seed, uint64_t k)
+{
+    const uint64_t z = sx_synth_frame(seed, k);
+    Pack<2> p;
+    p.w[0] = uint32_t(z);
+    p.w[1] = uint32_t(z >> 32);
+    return p;
+}
+__device__ __forceinline__ Pack<4> capture_pair(uint64_t seed, uint64_t k)
+{
+    const uint64_t z0 = sx_synth_frame(seed, k), z1 = sx_synth_frame(seed, k + 1);
+    Pack<4> p;
+    p.w[0] = uint32_t(z0), p.w[1] = uint32_t(z0 >> 32);
+    p.w[2] = uint32_t(z1), p.w[3] = uint32_t(z1 >> 32);
+    return p;
+}
+
+// Silence for frames [start, start + n) of stream s's ring, written by the lanes of a warp side by side.
+__device__ __forceinline__ void ring_zero(const BankState &b, uint64_t s, long long start, long long n, uint32_t lane)
+{
+    Pack<2> zero;
+    zero.w[0] = zero.w[1] = 0;
+    for (long long i = lane; i < n; i += 32)
+        st_stream<8>(ring_frame(b, s, uint64_t(start + i)), zero);
+}
+
+// A forwarded-over region [start, start + gap) older than one lap: only its last lap is still in the ring.
+__device__ __forceinline__ void clamp_gap_to_ring(const BankState &b, long long &start, long long &gap)
+{
+    if (gap > (long long)b.ring) {
+        start += gap - (long long)b.ring;
+        gap = (long long)b.ring;
+    }
+}
+
+// ALSA plays zeros for regions the application skipped (silence_size = boundary, :493-496): the
+// warp silences stream s's forwarded-over region [start, start + gap) before the block is written.
+// A gap of a whole lap or more silences the slots the block is about to take, hence the barrier.
+__device__ __forceinline__ void bank_silence_gap(const BankState &b, uint64_t s, long long start, long long gap, uint32_t lane)
+{
+    clamp_gap_to_ring(b, start, gap);
+    ring_zero(b, s, start, gap, lane);
+    __syncwarp();
 }
 
 constexpr int SX_HAS_TIME = 1 << 2; // SOAPY_SDR_HAS_TIME
@@ -196,10 +267,7 @@ __global__ void bank_capture_kernel(BankState b, char *cf32_out, bool fused, boo
             continue;
         char *out = b.capture_stage + s * b.period * 8;
         for (uint32_t i = lane; i < b.period; i += 32) {
-            uint64_t z = sx_synth_frame(b.seed + s, first + i);
-            Pack<2> p;
-            p.w[0] = uint32_t(z);
-            p.w[1] = uint32_t(z >> 32);
+            const Pack<2> p = capture_frame(b.seed + s, first + i);
             st_stream<8>(out + size_t(i) * 8, p);
         }
     }
@@ -288,20 +356,8 @@ __device__ __forceinline__ void bank_play_block(const BankState &b, uint64_t s, 
 {
     if (at < 0)
         return;
-
-    // ALSA plays zeros for regions the application skipped (silence_size = boundary, :493-496).
-    if (gap > 0) {
-        if (gap > (long long)b.ring) { // older than one lap: only the last lap is still in the ring
-            start += gap - (long long)b.ring;
-            gap = (long long)b.ring;
-        }
-        Pack<2> zero;
-        zero.w[0] = zero.w[1] = 0;
-        for (long long i = lane; i < gap; i += 32)
-            st_stream<8>(ring_frame(b, s, uint64_t(start + i)), zero);
-        // A gap of a whole lap or more silences the slots the block is about to take.
-        __syncwarp();
-    }
+    if (gap > 0)
+        bank_silence_gap(b, s, start, gap, lane);
 
     // The block may straddle a period boundary of the ring: at most two contiguous spans.
     const uint64_t into = uint64_t(at) % b.period;
@@ -328,20 +384,14 @@ __device__ __forceinline__ void bank_play_block(const BankState &b, uint64_t s, 
 __device__ __forceinline__ void bank_silence_by_warp(const BankState &b, uint64_t s, long long start, long long gap)
 {
     const uint32_t lane = threadIdx.x & 31;
-    if (gap > (long long)b.ring) { // older than one lap: only the last lap is still in the ring
-        start += gap - (long long)b.ring;
-        gap = (long long)b.ring;
-    }
+    clamp_gap_to_ring(b, start, gap);
     unsigned pending = __ballot_sync(0xffffffffu, gap > 0);
     while (pending) {
         const int j = __ffs(pending) - 1;
         pending &= pending - 1;
         const uint64_t sj = __shfl_sync(0xffffffffu, s, j);
         const long long start_j = __shfl_sync(0xffffffffu, start, j), gap_j = __shfl_sync(0xffffffffu, gap, j);
-        Pack<2> zero;
-        zero.w[0] = zero.w[1] = 0;
-        for (long long i = lane; i < gap_j; i += 32)
-            st_stream<8>(ring_frame(b, sj, uint64_t(start_j + i)), zero);
+        ring_zero(b, sj, start_j, gap_j, lane);
     }
 }
 
@@ -357,9 +407,7 @@ __global__ void bank_plan_write_kernel(BankState b, int flags, const long long *
     if (s < b.nstreams) {
         w = bank_plan_write(b, s, flags, time_ns, rx_time_offset_ns);
         if (for_data_kernel)
-            b.tx_ring_offset[s] = w.at >= 0 ? (long long)(ring_frame(b, s, uint64_t(w.at)) - b.playback_ring) +
-                                                  (uint64_t(w.at) % b.period != 0 ? 1 : 0)
-                                            : -1;
+            b.tx_ring_offset[s] = bank_ring_offset(b, s, w.at);
     }
     if (for_data_kernel) // (uniform over the grid: every lane gets here)
         bank_silence_by_warp(b, s, w.start, (s < b.nstreams && w.at >= 0) ? w.gap : 0);
@@ -403,10 +451,7 @@ __device__ __forceinline__ void bank_repeat_stream(const BankState &b, uint64_t 
 {
     char *slot = b.capture_stage + s * b.period * 8;
     for (uint32_t i = lane; i < b.period && !capture_in_slot; i += 32) {
-        uint64_t z = sx_synth_frame(b.seed + s, first + i);
-        Pack<2> p;
-        p.w[0] = uint32_t(z);
-        p.w[1] = uint32_t(z >> 32);
+        const Pack<2> p = capture_frame(b.seed + s, first + i);
         st_stream<8>(slot + size_t(i) * 8, p);
     }
     __syncwarp(); // the slot is complete before any lane reads it back
@@ -430,27 +475,18 @@ __device__ __forceinline__ void bank_repeat_stream(const BankState &b, uint64_t 
 // (one round trip, all vectors in flight at once) instead of being produced here.
 // Needs an even period and 16-byte aligned CF32 blocks; a block that does not start on a period
 // boundary of the ring falls back to frame-wide stores for the ring side.
-template <int U, class Hook>
+template <class Hook>
 __device__ __forceinline__ void bank_repeat_stream_reg(const BankState &b, uint64_t s, char *cf32, uint64_t first,
                                                        long long at, long long gap, long long start, uint32_t lane,
                                                        bool capture_in_slot, const Hook &hook)
 {
+    constexpr int U = 4; // 16-byte vectors a lane has in flight: a 256-frame period in one go
     char *slot = b.capture_stage + s * b.period * 8;
     char *cf = cf32 + s * b.period * 8;
     const uint32_t nvec = b.period / 2;
 
-    if (at >= 0 && gap > 0) { // silence for a forwarded-over region (rare: late start, underrun)
-        long long g = gap, st0 = start;
-        if (g > (long long)b.ring) {
-            st0 += g - (long long)b.ring;
-            g = (long long)b.ring;
-        }
-        Pack<2> zero;
-        zero.w[0] = zero.w[1] = 0;
-        for (long long i = lane; i < g; i += 32)
-            st_stream<8>(ring_frame(b, s, uint64_t(st0 + i)), zero);
-        __syncwarp(); // a gap of a lap or more silences the slots the block is about to take
-    }
+    if (at >= 0 && gap > 0) // rare: late start, underrun
+        bank_silence_gap(b, s, start, gap, lane);
     // Streams in lock-step write whole period slices of the ring: 16-byte stores.  A block that
     // starts inside a slice goes frame by frame.
     const bool ring_vec = at >= 0 && uint64_t(at) % b.period == 0;
@@ -467,13 +503,8 @@ __device__ __forceinline__ void bank_repeat_stream_reg(const BankState &b, uint6
             }
         } else {
 #pragma unroll
-            for (int u = 0; u < U; u++) {
-                const uint32_t v = base + lane + 32 * u;
-                const uint64_t z0 = sx_synth_frame(b.seed + s, first + 2 * uint64_t(v));
-                const uint64_t z1 = sx_synth_frame(b.seed + s, first + 2 * uint64_t(v) + 1);
-                cap[u].w[0] = uint32_t(z0), cap[u].w[1] = uint32_t(z0 >> 32);
-                cap[u].w[2] = uint32_t(z1), cap[u].w[3] = uint32_t(z1 >> 32);
-            }
+            for (int u = 0; u < U; u++)
+                cap[u] = capture_pair(b.seed + s, first + 2 * uint64_t(base + lane + 32 * u));
         }
 #pragma unroll
         for (int u = 0; u < U; u++) {
@@ -490,14 +521,10 @@ __device__ __forceinline__ void bank_repeat_stream_reg(const BankState &b, uint6
             if (!capture_in_slot)
                 st_stream<16>(slot + size_t(v) * 16, cap[u]);
             st_stream<16>(cf + size_t(v) * 16, mid[u]);
-            if (ring_vec) {
+            if (ring_vec)
                 st_stream<16>(ring + size_t(v) * 16, out[u]);
-            } else if (at >= 0) {
-                Pack<2> f0, f1;
-                f0.w[0] = out[u].w[0], f0.w[1] = out[u].w[1], f1.w[0] = out[u].w[2], f1.w[1] = out[u].w[3];
-                st_stream<8>(ring_frame(b, s, uint64_t(at) + 2 * uint64_t(v)), f0);
-                st_stream<8>(ring_frame(b, s, uint64_t(at) + 2 * uint64_t(v) + 1), f1);
-            }
+            else if (at >= 0)
+                ring_store_pair(b, s, uint64_t(at) + 2 * uint64_t(v), out[u]);
         }
     }
 }
@@ -507,74 +534,6 @@ __device__ __forceinline__ void bank_repeat_stream_reg(const BankState &b, uint6
 struct IdentityHook {
     __device__ __forceinline__ void operator()(Pack<4> &, uint64_t, uint32_t) const {}
 };
-
-// Warp-per-K-streams schedule of the fused iteration, intermediates in registers (above).
-template <int K, class Hook>
-__global__ void __launch_bounds__(256) bank_repeat_reg_kernel(BankState b, char *cf32, long long rx_time_offset_ns,
-                                                              bool capture_in_slot, Hook hook)
-{
-    const uint32_t lane = threadIdx.x & 31, warps_per_cta = blockDim.x >> 5;
-    const uint64_t nwarps = uint64_t(gridDim.x) * warps_per_cta;
-    const uint64_t nchunks = (uint64_t(b.nstreams) + K - 1) / K;
-    for (uint64_t c = uint64_t(blockIdx.x) * warps_per_cta + (threadIdx.x >> 5); c < nchunks; c += nwarps) {
-        const uint64_t base = c * K;
-        const uint32_t count = uint32_t(b.nstreams - base < K ? b.nstreams - base : K);
-        long long my_first = 0, my_at = -1, my_gap = 0, my_start = 0;
-        if (lane < count) {
-            BankWritePlan w;
-            bank_plan_repeat(b, base + lane, cf32, rx_time_offset_ns, my_first, w);
-            my_at = w.at;
-            my_gap = w.gap;
-            my_start = w.start;
-        }
-#pragma unroll
-        for (uint32_t j = 0; j < K; j++) {
-            const uint64_t first = uint64_t(__shfl_sync(0xffffffffu, my_first, j));
-            const long long at = __shfl_sync(0xffffffffu, my_at, j);
-            const long long gap = __shfl_sync(0xffffffffu, my_gap, j);
-            const long long start = __shfl_sync(0xffffffffu, my_start, j);
-            if (j >= count)
-                break;
-            bank_repeat_stream_reg<4>(b, base + j, cf32, first, at, gap, start, lane, capture_in_slot, hook);
-        }
-    }
-}
-
-// CTA-per-32-streams schedule with the intermediates in registers: the first warp takes the 32
-// streams' decisions, one stream per lane (the timestamp arithmetic is double precision and runs
-// on one lane per stream: 32 lanes side by side cost what one does), hands them over in shared
-// memory, and each of the CTA's warps then produces, converts and stores its streams' blocks
-// without reading anything back.
-// U = 16-byte vectors a lane has in flight (4: a 256-frame period in one go, ~98 registers, two
-// CTAs per SM; 2: two passes per period, fewer registers, MINB CTAs per SM).
-template <int U, int MINB, class Hook>
-__global__ void __launch_bounds__(256, MINB) bank_repeat_group_reg_kernel(BankState b, char *cf32, long long rx_time_offset_ns,
-                                                                          bool capture_in_slot, Hook hook)
-{
-    __shared__ long long s_first[2][32], s_at[2][32], s_gap[2][32], s_start[2][32];
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps_per_cta = blockDim.x >> 5;
-    const uint64_t ngroups = (uint64_t(b.nstreams) + 31) / 32;
-    int buf = 0;
-    for (uint64_t g = blockIdx.x; g < ngroups; g += gridDim.x, buf ^= 1) {
-        const uint64_t base = g * 32;
-        const uint32_t count = uint32_t(b.nstreams - base < 32 ? b.nstreams - base : 32);
-        if (threadIdx.x < count) {
-            long long first;
-            BankWritePlan w;
-            bank_plan_repeat(b, base + threadIdx.x, cf32, rx_time_offset_ns, first, w);
-            s_first[buf][threadIdx.x] = first;
-            s_at[buf][threadIdx.x] = w.at;
-            s_gap[buf][threadIdx.x] = w.gap;
-            s_start[buf][threadIdx.x] = w.start;
-        }
-        // One barrier per group: the plans alternate between two buffers, so the first warp may
-        // plan the next group while the others are still moving this one's blocks.
-        __syncthreads();
-        for (uint32_t j = warp; j < count; j += warps_per_cta)
-            bank_repeat_stream_reg<U>(b, base + j, cf32, uint64_t(s_first[buf][j]), s_at[buf][j], s_gap[buf][j],
-                                      s_start[buf][j], lane, capture_in_slot, hook);
-    }
-}
 
 // The repeater iteration in one launch: readStream(period) on every stream, then
 // writeStream(period, HAS_TIME, that read's timestamp + rx_time_offset_ns) of the block just
@@ -620,10 +579,12 @@ __global__ void __launch_bounds__(256) bank_repeat_kernel(BankState b, char *cf3
 // lanes 0..K-1 take their decisions, and the warp then carries them through the three stages.
 // No shared memory, no CTA barrier, and K sets the granularity: small K spreads S streams more
 // evenly over the resident warps, large K spends fewer issue slots on the (one-lane-per-stream)
-// decisions.
-template <int K>
+// decisions.  IN_REGISTERS: each stream's stages keep their intermediates in registers and only
+// store (bank_repeat_stream_reg, the form with a hook point: even periods and 16-byte aligned
+// CF32 only); otherwise they go through memory stage by stage (bank_repeat_stream, no hook).
+template <int K, bool IN_REGISTERS = false, class Hook = IdentityHook>
 __global__ void __launch_bounds__(256) bank_repeat_warp_kernel(BankState b, char *cf32, long long rx_time_offset_ns,
-                                                               bool capture_in_slot)
+                                                               bool capture_in_slot, Hook hook)
 {
     const uint32_t lane = threadIdx.x & 31, warps_per_cta = blockDim.x >> 5;
     const uint64_t nwarps = uint64_t(gridDim.x) * warps_per_cta;
@@ -633,9 +594,8 @@ __global__ void __launch_bounds__(256) bank_repeat_warp_kernel(BankState b, char
         const uint32_t count = uint32_t(b.nstreams - base < K ? b.nstreams - base : K);
         long long my_first = 0, my_at = -1, my_gap = 0, my_start = 0;
         if (lane < count) {
-            const uint64_t s = base + lane;
             BankWritePlan w;
-            bank_plan_repeat(b, s, cf32, rx_time_offset_ns, my_first, w);
+            bank_plan_repeat(b, base + lane, cf32, rx_time_offset_ns, my_first, w);
             my_at = w.at;
             my_gap = w.gap;
             my_start = w.start;
@@ -648,7 +608,10 @@ __global__ void __launch_bounds__(256) bank_repeat_warp_kernel(BankState b, char
             const long long start = __shfl_sync(0xffffffffu, my_start, j);
             if (j >= count) // count is the same in every lane
                 break;
-            bank_repeat_stream(b, base + j, cf32, first, at, gap, start, lane, capture_in_slot);
+            if constexpr (IN_REGISTERS)
+                bank_repeat_stream_reg(b, base + j, cf32, first, at, gap, start, lane, capture_in_slot, hook);
+            else
+                bank_repeat_stream(b, base + j, cf32, first, at, gap, start, lane, capture_in_slot);
         }
     }
 }
@@ -702,9 +665,7 @@ __global__ void bank_plan_repeat_kernel(BankState b, char *cf32, long long rx_ti
     if (s < b.nstreams) {
         long long first;
         bank_plan_repeat(b, s, cf32, rx_time_offset_ns, first, w);
-        b.tx_ring_offset[s] = w.at >= 0 ? (long long)(ring_frame(b, s, uint64_t(w.at)) - b.playback_ring) +
-                                              (uint64_t(w.at) % b.period != 0 ? 1 : 0)
-                                        : -1;
+        b.tx_ring_offset[s] = bank_ring_offset(b, s, w.at);
     }
     bank_silence_by_warp(b, s, w.start, (s < b.nstreams && w.at >= 0) ? w.gap : 0);
 }
@@ -788,13 +749,8 @@ __global__ void __launch_bounds__(256) bank_repeat_data_kernel(BankState b, char
         const uint32_t j = pow2 ? local >> log2v : local / nvec;
         jj[u] = v0 + u * 256 + threadIdx.x < total ? j : 0;
         kk[u] = pow2 ? local & (nvec - 1) : local - j * nvec;
-        if (MODE != kBankModeWrite && !capture_in_slot) {
-            const uint64_t first = uint64_t(s_first[jj[u]]);
-            const uint64_t z0 = sx_synth_frame(b.seed + s0 + jj[u], first + 2 * uint64_t(kk[u]));
-            const uint64_t z1 = sx_synth_frame(b.seed + s0 + jj[u], first + 2 * uint64_t(kk[u]) + 1);
-            cap[u].w[0] = uint32_t(z0), cap[u].w[1] = uint32_t(z0 >> 32);
-            cap[u].w[2] = uint32_t(z1), cap[u].w[3] = uint32_t(z1 >> 32);
-        }
+        if (MODE != kBankModeWrite && !capture_in_slot)
+            cap[u] = capture_pair(b.seed + s0 + jj[u], uint64_t(s_first[jj[u]]) + 2 * uint64_t(kk[u]));
     }
 #pragma unroll
     for (int u = 0; u < U; u++) {
@@ -825,67 +781,10 @@ __global__ void __launch_bounds__(256) bank_repeat_data_kernel(BankState b, char
             // the block starts on a period boundary of the ring: one contiguous, 16-byte aligned span
             st_stream<16>(b.playback_ring + off + size_t(kk[u]) * 16, out[u]);
         } else {
-            // it straddles two slices of the time-major ring: frame by frame (rare: a stream out of step)
-            const uint64_t at = uint64_t(b.tx_write_position[s0 + jj[u]]);
-            Pack<2> f0, f1;
-            f0.w[0] = out[u].w[0], f0.w[1] = out[u].w[1], f1.w[0] = out[u].w[2], f1.w[1] = out[u].w[3];
-            st_stream<8>(ring_frame(b, s0 + jj[u], at + 2 * uint64_t(kk[u])), f0);
-            st_stream<8>(ring_frame(b, s0 + jj[u], at + 2 * uint64_t(kk[u]) + 1), f1);
+            // it straddles two slices of the time-major ring: frame by frame
+            ring_store_pair(b, s0 + jj[u], uint64_t(b.tx_write_position[s0 + jj[u]]) + 2 * uint64_t(kk[u]), out[u]);
         }
     }
-}
-
-// Launches the two kernels of the plan + data schedule on `st`: decisions by one thread per
-// stream, then the samples, the second as a programmatic dependent of the first so that its
-// launch and the first CTAs' set-up run under the decisions instead of after them.
-// U = 16-byte vectors per thread (2 or 4).  Returns the CUDA error of the launches.
-template <int U, class Hook>
-inline cudaError_t launch_bank_repeat_planned(const BankState &b, char *cf32, long long rx_time_offset_ns, bool capture_in_slot,
-                                              cudaStream_t st, const Hook &hook, bool programmatic = true)
-{
-    bank_plan_repeat_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, cf32, rx_time_offset_ns);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess)
-        return e;
-    const uint64_t vectors = uint64_t(b.nstreams) * (b.period / 2);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(unsigned((vectors + 256 * U - 1) / (256 * U)));
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = programmatic ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, bank_repeat_data_kernel<U, Hook>, b, cf32, capture_in_slot, hook);
-}
-
-// One half of the iteration (sxgpu_bank_read / sxgpu_bank_write on a large bank): the matching
-// plan kernel, then the data kernel in that mode as its programmatic dependent.
-template <int MODE>
-inline cudaError_t launch_bank_half_planned(const BankState &b, char *cf32, bool capture_in_slot, int flags,
-                                            const long long *time_ns, long long rx_time_offset_ns, cudaStream_t st,
-                                            bool programmatic = true)
-{
-    if (MODE == kBankModeRead)
-        bank_plan_read_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, cf32);
-    else
-        bank_plan_write_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, flags, time_ns, rx_time_offset_ns, true);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess)
-        return e;
-    constexpr int U = 4;
-    const uint64_t vectors = uint64_t(b.nstreams) * (b.period / 2);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(unsigned((vectors + 256 * U - 1) / (256 * U)));
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = programmatic ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, bank_repeat_data_kernel<U, IdentityHook, MODE>, b, cf32, capture_in_slot, IdentityHook());
 }
 
 // ---------------------------------------------------------------------------------------
@@ -954,6 +853,9 @@ __global__ void __launch_bounds__(kIirThreads) bank_repeat_iir_kernel(BankState 
                 if (capture_in_slot) {
                     cap = ld_stream<16>(slot);
                 } else {
+                    // capture_pair(b.seed + s0 + r, first) written out: through the helper the compiler
+                    // associates the seed's additions differently, and read mode ran 1 % slower at 64
+                    // streams (tools/bench_iir.py, B200 at a 1 000 W power limit)
                     const uint64_t first = uint64_t(s_first[r]) + t0 + 2 * m;
                     const uint64_t z0 = sx_synth_frame(b.seed + s0 + r, first), z1 = sx_synth_frame(b.seed + s0 + r, first + 1);
                     cap.w[0] = uint32_t(z0), cap.w[1] = uint32_t(z0 >> 32);
@@ -993,11 +895,7 @@ __global__ void __launch_bounds__(kIirThreads) bank_repeat_iir_kernel(BankState 
             if ((off & 1) == 0) {
                 st_stream<16>(b.playback_ring + off + v * 16, out);
             } else { // straddles two slices of the time-major ring: frame by frame
-                const uint64_t at = uint64_t(s_at[r]);
-                Pack<2> f0, f1;
-                f0.w[0] = out.w[0], f0.w[1] = out.w[1], f1.w[0] = out.w[2], f1.w[1] = out.w[3];
-                st_stream<8>(ring_frame(b, s0 + r, at + 2 * v), f0);
-                st_stream<8>(ring_frame(b, s0 + r, at + 2 * v + 1), f1);
+                ring_store_pair(b, s0 + r, uint64_t(s_at[r]) + 2 * v, out);
             }
         }
         __syncthreads(); // the next tile overwrites the rows
@@ -1022,52 +920,71 @@ inline const char *bank_repeat_iir_invalid(const BankState &b, const void *cf32,
     return nullptr;
 }
 
-// bank_plan_repeat_kernel, then bank_repeat_iir_kernel as its programmatic dependent.
-template <class Hook>
-inline cudaError_t launch_bank_repeat_iir(const BankState &b, char *cf32, long long rx_time_offset_ns, bool capture_in_slot,
-                                          const IirView &pre, const IirView &post, cudaStream_t st, const Hook &hook)
+// ---------------------------------------------------------------------------------------
+// Launchers of the plan + data schedules.  The data kernel is launched as a programmatic
+// dependent of the plan kernel, so that its launch and the first CTAs' set-up run under the
+// decisions instead of after them; it waits for them with pdl_wait() before it reads them.
+// ---------------------------------------------------------------------------------------
+template <class... Params, class... Args>
+inline cudaError_t launch_dependent(void (*kernel)(Params...), unsigned grid, unsigned block, cudaStream_t st,
+                                    const Args &...args)
 {
-    bank_plan_repeat_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, cf32, rx_time_offset_ns);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess)
-        return e;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(unsigned((uint64_t(b.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta));
-    cfg.blockDim = dim3(kIirThreads);
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(block);
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, bank_repeat_iir_kernel<Hook>, b, cf32, capture_in_slot, pre, post, hook);
+    return cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
-// One half with its filter (sxgpu_bank_read_filtered / sxgpu_bank_write_filtered): the matching
-// plan kernel, then bank_repeat_iir_kernel in that mode as its programmatic dependent.  One
-// schedule for every bank size, as for the whole iteration.
+// The decisions of the whole iteration (MODE = kBankModeRepeat: a timed write at the read's
+// timestamp + rx_time_offset_ns; `flags` and `time_ns` are not used) or of one half, one thread
+// per stream, for the data kernel that follows.
 template <int MODE>
-inline cudaError_t launch_bank_half_iir(const BankState &b, char *cf32, bool capture_in_slot, int flags, const long long *time_ns,
-                                        long long rx_time_offset_ns, const IirView &f, cudaStream_t st)
+inline cudaError_t launch_bank_plan(const BankState &b, char *cf32, int flags, const long long *time_ns,
+                                    long long rx_time_offset_ns, cudaStream_t st)
 {
-    if (MODE == kBankModeRead)
-        bank_plan_read_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, cf32);
+    const unsigned grid = (b.nstreams + 63) / 64;
+    if (MODE == kBankModeRepeat)
+        bank_plan_repeat_kernel<<<grid, 64, 0, st>>>(b, cf32, rx_time_offset_ns);
+    else if (MODE == kBankModeRead)
+        bank_plan_read_kernel<<<grid, 64, 0, st>>>(b, cf32);
     else
-        bank_plan_write_kernel<<<(b.nstreams + 63) / 64, 64, 0, st>>>(b, flags, time_ns, rx_time_offset_ns, true);
-    cudaError_t e = cudaGetLastError();
+        bank_plan_write_kernel<<<grid, 64, 0, st>>>(b, flags, time_ns, rx_time_offset_ns, true);
+    return cudaGetLastError();
+}
+
+// The iteration or one half of it on a large bank: the decisions, then bank_repeat_data_kernel in
+// that mode.  U = 16-byte vectors per thread (2 or 4).  Returns the CUDA error of the launches.
+template <int MODE, int U, class Hook>
+inline cudaError_t launch_bank_planned(const BankState &b, char *cf32, bool capture_in_slot, int flags, const long long *time_ns,
+                                       long long rx_time_offset_ns, cudaStream_t st, const Hook &hook)
+{
+    const cudaError_t e = launch_bank_plan<MODE>(b, cf32, flags, time_ns, rx_time_offset_ns, st);
     if (e != cudaSuccess)
         return e;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(unsigned((uint64_t(b.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta));
-    cfg.blockDim = dim3(kIirThreads);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, bank_repeat_iir_kernel<IdentityHook, MODE>, b, cf32, capture_in_slot, f, IirView{},
-                              IdentityHook());
+    const uint64_t vectors = uint64_t(b.nstreams) * (b.period / 2);
+    return launch_dependent(bank_repeat_data_kernel<U, Hook, MODE>, unsigned((vectors + 256 * U - 1) / (256 * U)), 256, st, b,
+                            cf32, capture_in_slot, hook);
+}
+
+// The iteration or one half of it with filters, every bank size: the decisions, then
+// bank_repeat_iir_kernel in that mode.  A half runs `pre` alone (`post` is not used).
+template <int MODE, class Hook>
+inline cudaError_t launch_bank_iir(const BankState &b, char *cf32, bool capture_in_slot, int flags, const long long *time_ns,
+                                   long long rx_time_offset_ns, const IirView &pre, const IirView &post, cudaStream_t st,
+                                   const Hook &hook)
+{
+    const cudaError_t e = launch_bank_plan<MODE>(b, cf32, flags, time_ns, rx_time_offset_ns, st);
+    if (e != cudaSuccess)
+        return e;
+    return launch_dependent(bank_repeat_iir_kernel<Hook, MODE>,
+                            unsigned((uint64_t(b.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta), kIirThreads, st, b,
+                            cf32, capture_in_slot, pre, post, hook);
 }
 
 __global__ void bank_advance_kernel(BankState b, long long frames)

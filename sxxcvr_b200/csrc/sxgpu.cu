@@ -113,8 +113,8 @@ struct sxgpu_ctx {
     int64_t loopback_variant = 0;           // 0 auto (= 2), 1 = vector accesses on a persistent grid, 2 = one tile per CTA, 3 = bulk-async
     int64_t warp_ctas_per_sm = 0;           // grid cap of the warp-per-block / warp-per-stream kernels: N CTAs per SM (persistent), 0 = one CTA per eight blocks
     int64_t bank_split_variant = 0;         // sxgpu_bank_read / _write on large banks: 0 auto (plan + data kernels), 1 = warp-per-stream kernels
-    int64_t bank_pdl = 1;                   // the plan + data schedule launches its data kernel as a programmatic dependent
-    int64_t bank_repeat_variant = 0;        // 0 auto; 1, 2, 4, 8 = K streams per warp round; 100 = 32 per CTA round
+    int64_t bank_repeat_variant = 0;        // 0 auto; 1, 2, 4 = K streams per warp round; 100 = 32 per CTA round;
+                                            // 201, 202, 204 = K per warp round in registers; 600, 604 = plan + data kernels
     int64_t bounce_threads = 0;             // threads copying a pageable caller's buffer: 0 auto, 1 = the caller alone
     int64_t numa_local_alloc = 1;           // place pinned host memory on the GPU's NUMA node
     int64_t numa_node = -1;                 // read-only: the GPU's NUMA node, -1 unknown / no NUMA
@@ -1320,7 +1320,6 @@ int64_t *option_slot(sxgpu_ctx *ctx, const char *key)
         {"resident_max_frames", &ctx->resident_max_frames},
         {"zero_copy_variant", &ctx->zero_copy_variant},
         {"bank_repeat_variant", &ctx->bank_repeat_variant},
-        {"bank_pdl", &ctx->bank_pdl},
         {"bank_split_variant", &ctx->bank_split_variant},
         {"warp_ctas_per_sm", &ctx->warp_ctas_per_sm},
         {"batch_variant", &ctx->batch_variant},
@@ -1841,8 +1840,8 @@ int sxgpu_bank_read(sxgpu_bank *bank, void *d_cf32, sxgpu_stream stream)
     if (bank_split_direct(ctx, b, d_cf32)) {
         // large banks: decisions by a thread per stream, then capture and RX conversion by CTAs that
         // take one chunk each (sx_bank.cuh, bank_repeat_data_kernel in read mode)
-        SX_CUDA(ctx, launch_bank_half_planned<kBankModeRead>(b, static_cast<char *>(d_cf32), bank->external_capture, 0, nullptr,
-                                                             0, st, ctx->bank_pdl != 0));
+        SX_CUDA(ctx, (launch_bank_planned<kBankModeRead, 4>(b, static_cast<char *>(d_cf32), bank->external_capture, 0, nullptr, 0,
+                                                            st, IdentityHook())));
         ctx->launches += 2;
         ctx->frames_rx += uint64_t(b.nstreams) * b.period;
         return SXGPU_OK;
@@ -1871,8 +1870,8 @@ int sxgpu_bank_write(sxgpu_bank *bank, const void *d_cf32, int flags, const long
     cudaStream_t st = bank_stream(bank, stream);
     const BankState &b = bank->st;
     if (bank_split_direct(ctx, b, d_cf32)) {
-        SX_CUDA(ctx, launch_bank_half_planned<kBankModeWrite>(b, const_cast<char *>(static_cast<const char *>(d_cf32)), false,
-                                                              flags, d_time_ns, rx_time_offset_ns, st, ctx->bank_pdl != 0));
+        SX_CUDA(ctx, (launch_bank_planned<kBankModeWrite, 4>(b, const_cast<char *>(static_cast<const char *>(d_cf32)), false, flags,
+                                                             d_time_ns, rx_time_offset_ns, st, IdentityHook())));
         ctx->launches += 2;
         ctx->frames_tx += uint64_t(b.nstreams) * b.period;
         return SXGPU_OK;
@@ -1903,22 +1902,15 @@ int sxgpu_bank_repeat(sxgpu_bank *bank, void *d_cf32, long long rx_time_offset_n
     const bool ext = bank->external_capture;
     auto warp_variant = [&](auto kernel, uint64_t k) {
         const uint64_t chunks = (uint64_t(b.nstreams) + k - 1) / k;
-        kernel<<<persistent_grid(ctx, kernel, 256, 0, (chunks + 7) / 8), 256, 0, st>>>(b, cf, rx_time_offset_ns, ext);
-    };
-    auto reg_variant = [&](auto kernel, uint64_t k) { // intermediates in registers, stores only
-        const uint64_t chunks = (uint64_t(b.nstreams) + k - 1) / k;
         kernel<<<persistent_grid(ctx, kernel, 256, 0, (chunks + 7) / 8), 256, 0, st>>>(b, cf, rx_time_offset_ns, ext,
                                                                                        IdentityHook());
     };
-    auto group_variant = [&](auto kernel) { // a CTA takes 32 streams per round, its first warp decides for all of them
-        const uint64_t groups = (uint64_t(b.nstreams) + kRepeatGroup - 1) / kRepeatGroup;
-        kernel<<<persistent_grid(ctx, kernel, 256, 0, groups), 256, 0, st>>>(b, cf, rx_time_offset_ns, ext);
-    };
     // Schedules.  K streams per warp round: lanes 0..K-1 take K streams' decisions side by side, so
     // a larger K spends fewer issue slots on the timestamp arithmetic; a smaller K spreads few
-    // streams over more warps.  1/2/4/8 and 100 carry each stream through memory stage by stage
-    // (each stage reading from L2 what the previous one wrote); 201/202/204 keep the stages'
-    // intermediates in registers and only store.  Measured crossovers: profiles/r02_summary.md.
+    // streams over more warps.  1/2/4 and 100 (a CTA takes 32 streams per round, its first warp
+    // decides for all of them) carry each stream through memory stage by stage (each stage reading
+    // from L2 what the previous one wrote); 201/202/204 keep the stages' intermediates in registers
+    // and only store.  Measured crossovers: profiles/r02_summary.md.
     const bool reg_ok = (b.period % 2 == 0) && reinterpret_cast<uintptr_t>(d_cf32) % 16 == 0;
     int64_t k = ctx->bank_repeat_variant;
     if (k == 0) {
@@ -1935,36 +1927,26 @@ int sxgpu_bank_repeat(sxgpu_bank *bank, void *d_cf32, long long rx_time_offset_n
     case 1: warp_variant(bank_repeat_warp_kernel<1>, 1); break;
     case 2: warp_variant(bank_repeat_warp_kernel<2>, 2); break;
     case 4: warp_variant(bank_repeat_warp_kernel<4>, 4); break;
-    case 8: warp_variant(bank_repeat_warp_kernel<8>, 8); break;
-    case 100: group_variant(bank_repeat_kernel); break;
-    case 201: reg_variant(bank_repeat_reg_kernel<1, IdentityHook>, 1); break;
-    case 202: reg_variant(bank_repeat_reg_kernel<2, IdentityHook>, 2); break;
-    case 204: reg_variant(bank_repeat_reg_kernel<4, IdentityHook>, 4); break;
-    case 300:   // a CTA takes 32 streams per round: first warp decides, every warp keeps its streams in registers
-    case 302:   // ... two vectors per lane in flight instead of four: fewer registers, three CTAs per SM
-    case 303: { // ... four CTAs per SM
-        const uint64_t groups = (uint64_t(b.nstreams) + 31) / 32;
-        auto go = [&](auto kernel) {
-            kernel<<<persistent_grid(ctx, kernel, 256, 0, groups), 256, 0, st>>>(b, cf, rx_time_offset_ns, ext, IdentityHook());
-        };
-        if (k == 300)
-            go(bank_repeat_group_reg_kernel<4, 1, IdentityHook>);
-        else if (k == 302)
-            go(bank_repeat_group_reg_kernel<2, 3, IdentityHook>);
-        else
-            go(bank_repeat_group_reg_kernel<2, 4, IdentityHook>);
+    case 100: {
+        const uint64_t groups = (uint64_t(b.nstreams) + kRepeatGroup - 1) / kRepeatGroup;
+        bank_repeat_kernel<<<persistent_grid(ctx, bank_repeat_kernel, 256, 0, groups), 256, 0, st>>>(b, cf, rx_time_offset_ns, ext);
         break;
     }
+    case 201: warp_variant(bank_repeat_warp_kernel<1, true>, 1); break;
+    case 202: warp_variant(bank_repeat_warp_kernel<2, true>, 2); break;
+    case 204: warp_variant(bank_repeat_warp_kernel<4, true>, 4); break;
     case 600:   // decisions by a thread-per-stream kernel, then the samples by hardware-scheduled CTAs (two vectors per thread)
     case 604: { // ... four vectors per thread
         if (b.period < 4)
             return ctx->invalid("the direct schedules need a period of at least four frames");
-        SX_CUDA(ctx, k == 600 ? launch_bank_repeat_planned<2>(b, cf, rx_time_offset_ns, ext, st, IdentityHook(), ctx->bank_pdl != 0)
-                              : launch_bank_repeat_planned<4>(b, cf, rx_time_offset_ns, ext, st, IdentityHook(), ctx->bank_pdl != 0));
+        SX_CUDA(ctx, (k == 600 ? launch_bank_planned<kBankModeRepeat, 2>(b, cf, ext, SX_HAS_TIME, nullptr, rx_time_offset_ns, st,
+                                                                          IdentityHook())
+                               : launch_bank_planned<kBankModeRepeat, 4>(b, cf, ext, SX_HAS_TIME, nullptr, rx_time_offset_ns, st,
+                                                                          IdentityHook())));
         ctx->launches++;
         break;
     }
-    default: return ctx->invalid("bank_repeat_variant must be 0 (auto), 1, 2, 4, 8, 100, 201, 202, 204, 300, 302, 303, 600 or 604");
+    default: return ctx->invalid("bank_repeat_variant must be 0 (auto), 1, 2, 4, 100, 201, 202, 204, 600 or 604");
     }
     SX_CUDA(ctx, cudaGetLastError());
     ctx->launches += 1;
@@ -2308,8 +2290,8 @@ int sxgpu_bank_repeat_filtered(sxgpu_bank *bank, sxgpu_iir *pre, sxgpu_iir *post
         return sxgpu_bank_repeat(bank, d_cf32, rx_time_offset_ns, stream);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const BankState &b = bank->st;
-    SX_CUDA(ctx, launch_bank_repeat_iir(b, static_cast<char *>(d_cf32), rx_time_offset_ns, bank->external_capture, vpre,
-                                        vpost, bank_stream(bank, stream), IdentityHook()));
+    SX_CUDA(ctx, launch_bank_iir<kBankModeRepeat>(b, static_cast<char *>(d_cf32), bank->external_capture, SX_HAS_TIME, nullptr,
+                                                  rx_time_offset_ns, vpre, vpost, bank_stream(bank, stream), IdentityHook()));
     ctx->launches += 2;
     ctx->frames_rx += uint64_t(b.nstreams) * b.period;
     ctx->frames_tx += uint64_t(b.nstreams) * b.period;
@@ -2330,8 +2312,8 @@ int sxgpu_bank_read_filtered(sxgpu_bank *bank, sxgpu_iir *f, void *d_cf32, sxgpu
         return sxgpu_bank_read(bank, d_cf32, stream);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const BankState &b = bank->st;
-    SX_CUDA(ctx, launch_bank_half_iir<kBankModeRead>(b, static_cast<char *>(d_cf32), bank->external_capture, 0, nullptr, 0, v,
-                                                     bank_stream(bank, stream)));
+    SX_CUDA(ctx, launch_bank_iir<kBankModeRead>(b, static_cast<char *>(d_cf32), bank->external_capture, 0, nullptr, 0, v,
+                                                IirView{}, bank_stream(bank, stream), IdentityHook()));
     ctx->launches += 2;
     ctx->frames_rx += uint64_t(b.nstreams) * b.period;
     return SXGPU_OK;
@@ -2353,8 +2335,9 @@ int sxgpu_bank_write_filtered(sxgpu_bank *bank, sxgpu_iir *f, const void *d_cf32
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const BankState &b = bank->st;
     // the kernel only loads from the block in this mode
-    SX_CUDA(ctx, launch_bank_half_iir<kBankModeWrite>(b, const_cast<char *>(static_cast<const char *>(d_cf32)), false, flags,
-                                                      d_time_ns, rx_time_offset_ns, v, bank_stream(bank, stream)));
+    SX_CUDA(ctx, launch_bank_iir<kBankModeWrite>(b, const_cast<char *>(static_cast<const char *>(d_cf32)), false, flags,
+                                                 d_time_ns, rx_time_offset_ns, v, IirView{}, bank_stream(bank, stream),
+                                                 IdentityHook()));
     ctx->launches += 2;
     ctx->frames_tx += uint64_t(b.nstreams) * b.period;
     return SXGPU_OK;

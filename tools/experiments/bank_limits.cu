@@ -626,25 +626,19 @@ int main(int argc, char **argv)
         report("data_kernel_u4", time_us([&](int) { bank_repeat_data_kernel<4, IdentityHook><<<unsigned((vectors + 1023) / 1024), 256>>>(b, cf, false, IdentityHook()); }, 50), bytes3);
         report("data_kernel_u2_external", time_us([&](int) { bank_repeat_data_kernel<2, IdentityHook><<<unsigned((vectors + 511) / 512), 256>>>(b, cf, true, IdentityHook()); }, 50), bytes3);
         report("data_kernel_u4_external", time_us([&](int) { bank_repeat_data_kernel<4, IdentityHook><<<unsigned((vectors + 1023) / 1024), 256>>>(b, cf, true, IdentityHook()); }, 50), bytes3);
-        report("plan_then_data_u2", time_us([&](int) { CK(launch_bank_repeat_planned<2>(b, cf, lat, false, 0, IdentityHook(), false)); }, 50), bytes3);
-        report("plan_then_data_u2_programmatic", time_us([&](int) { CK(launch_bank_repeat_planned<2>(b, cf, lat, false, 0, IdentityHook(), true)); }, 50), bytes3);
-        report("plan_then_data_u4_programmatic", time_us([&](int) { CK(launch_bank_repeat_planned<4>(b, cf, lat, false, 0, IdentityHook(), true)); }, 50), bytes3);
-        report("plan_then_data_u2_programmatic_external", time_us([&](int) { CK(launch_bank_repeat_planned<2>(b, cf, lat, true, 0, IdentityHook(), true)); }, 50), bytes3);
+        report("plan_then_data_u2_programmatic", time_us([&](int) { CK((launch_bank_planned<kBankModeRepeat, 2>(b, cf, false, SX_HAS_TIME, nullptr, lat, 0, IdentityHook()))); }, 50), bytes3);
+        report("plan_then_data_u4_programmatic", time_us([&](int) { CK((launch_bank_planned<kBankModeRepeat, 4>(b, cf, false, SX_HAS_TIME, nullptr, lat, 0, IdentityHook()))); }, 50), bytes3);
+        report("plan_then_data_u2_programmatic_external", time_us([&](int) { CK((launch_bank_planned<kBankModeRepeat, 2>(b, cf, true, SX_HAS_TIME, nullptr, lat, 0, IdentityHook()))); }, 50), bytes3);
         {
             cudaStream_t cs;
             CK(cudaStreamCreate(&cs));
             cudaGraph_t graph;
             cudaGraphExec_t exec;
             CK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-            CK(launch_bank_repeat_planned<2>(b, cf, lat, false, cs, IdentityHook(), true));
+            CK((launch_bank_planned<kBankModeRepeat, 2>(b, cf, false, SX_HAS_TIME, nullptr, lat, cs, IdentityHook())));
             CK(cudaStreamEndCapture(cs, &graph));
             CK(cudaGraphInstantiate(&exec, graph, 0));
             report("plan_then_data_u2_programmatic_graph", time_us([&](int) { CK(cudaGraphLaunch(exec, 0)); }, 50), bytes3);
-            CK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-            CK(launch_bank_repeat_planned<2>(b, cf, lat, false, cs, IdentityHook(), false));
-            CK(cudaStreamEndCapture(cs, &graph));
-            CK(cudaGraphInstantiate(&exec, graph, 0));
-            report("plan_then_data_u2_graph", time_us([&](int) { CK(cudaGraphLaunch(exec, 0)); }, 50), bytes3);
         }
         report("group_kernel_v100", time_us([&](int) { bank_repeat_kernel<<<740, 256>>>(b, cf, lat, false); }, 50), bytes3);
         return 0;

@@ -63,7 +63,7 @@ def main():
     for S in args.streams:
         cf = torch.empty(S * P * 2, dtype=torch.float32, device="cuda")
         schedules = [("read+write", None, 0)]
-        for variant in (0, 1, 2, 4, 8, 100):
+        for variant in (0, 1, 2, 4, 100):
             schedules.append(("repeat", variant, 0))
         for name, variant, ctas in schedules:
             if variant is not None:

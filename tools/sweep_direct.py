@@ -6,7 +6,7 @@ the library's own entry points on one B200 (run under gpurun; results -> gpurun_
   ext         CS16 / S16 extensions (12 B/frame) at 2^27 frames: 4 vs 3
   loopback    fused RX->TX: 2 (direct) vs 3 (bulk-async) vs 1 (vector, persistent), with and without the CF32 block
   batched     1 GiB as N blocks per launch: 2 (direct) vs 3 (bulk-async tiles) vs 1 (slices)
-  bank        one repeater iteration: 600 / 604 (plan + data kernels) vs 100 / 300, per launch and from a CUDA graph,
+  bank        one repeater iteration: 600 / 604 (plan + data kernels) vs 100, per launch and from a CUDA graph,
               synthetic and ingested capture, S in {1024 .. 65536}
 """
 import argparse
@@ -162,7 +162,7 @@ def sweep_bank(ctx, side, out):
     for S in (1024, 4096, 16384, 65536):
         cf = torch.empty(S * P * 2, dtype=torch.float32, device="cuda")
         row = {"streams": S}
-        for variant in (0, 600, 604, 100, 300, 201 if S <= 4096 else 2):
+        for variant in (0, 600, 604, 100, 201 if S <= 4096 else 2):
             ctx.set_option("bank_repeat_variant", variant)
             with Bank(ctx, S, P, rate, 0.0, 7) as bank:
                 sec = timed(lambda: bank.repeat(cf.data_ptr(), lat, st), side, 200, warm=5)
@@ -175,7 +175,7 @@ def sweep_bank(ctx, side, out):
                 assert ((txp - rxp) == 768).all()
             row[f"v{variant}_us"] = round(sec * 1e6, 2)
             row[f"v{variant}_graph_us"] = round(gsec * 1e6, 2)
-        for variant in (0, 600, 604, 100, 303):
+        for variant in (0, 600, 604, 100):
             ctx.set_option("bank_repeat_variant", variant)
             with Bank(ctx, S, P, rate, 0.0, 7) as bank:
                 bank.ingest(0, 0, None, st)

@@ -131,7 +131,7 @@ def sweep_bank(ctx, side, out):
     for S in (4096, 16384, 65536):
         cf = torch.empty(S * P * 2, dtype=torch.float32, device="cuda")
         row = {"streams": S}
-        for variant in (2, 100, 300, 302, 303, 600):
+        for variant in (2, 100, 600):
             ctx.set_option("bank_repeat_variant", variant)
             with Bank(ctx, S, P, rate, 0.0, 7) as bank:
                 sec = timed(lambda: bank.repeat(cf.data_ptr(), lat, st), side, 200, warm=5)
@@ -145,7 +145,7 @@ def sweep_bank(ctx, side, out):
             row[f"v{variant}_us"] = round(sec * 1e6, 2)
             row[f"v{variant}_graph_us"] = round(gsec * 1e6, 2)
         # frames from outside (sxgpu_bank_ingest): the capture slots are read, not synthesised
-        for variant in (100, 202, 300, 302, 303, 604):
+        for variant in (100, 202, 604):
             ctx.set_option("bank_repeat_variant", variant)
             with Bank(ctx, S, P, rate, 0.0, 7) as bank:
                 bank.ingest(0, 0, None, st)
