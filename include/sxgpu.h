@@ -238,6 +238,21 @@ int sxgpu_iir_get_state(sxgpu_iir *f, void *h_zf, sxgpu_stream stream);
 /* Filter d_cf32[nstreams][period] in place, carrying the state: sosfilt(sos, x, zi=state) per
  * stream.  1 <= period <= 65536; d_cf32 8-byte aligned device memory. */
 int sxgpu_iir_apply(sxgpu_iir *f, void *d_cf32, uint32_t period, sxgpu_stream stream);
+/* Filter d_cf32[nstreams][nframes] in place, carrying the state, for any nframes >= 1: a long block
+ * filtered in parallel along each stream, not only across streams.  Each stream is cut into chunks
+ * of L frames (the last may be shorter); L is 1024, halved while nstreams * ceil(nframes / L) <
+ * 65536 and L > 128, and depends on nothing else.  The chunks run from a zero state in float32,
+ * their start states are carried across in float64 (end = A^L start + end from zero, A the
+ * cascade's state matrix), and they run again from those starts, rounded to float32, in place
+ * (DESIGN.md §4).  Chunk 0 of every stream is sxgpu_iir_apply bit for bit, and a block of one
+ * chunk (nframes <= L) is exactly sxgpu_iir_apply.  Later chunks differ from it only through the
+ * rounding of their start state: within 5e-5 of the output's peak of sosfilt in float64, as the
+ * float32 filter is, and within a few 1e-6 of the peak of sosfilt in float32 (tests/sxiir_long.py
+ * restates the call bit for bit).  Refused: nframes 0, a NULL or unaligned d_cf32, a block whose
+ * size in bytes overflows 64 bits or needs more than 2^31 - 1 CTAs of 64 chunks.  Only kernels and
+ * stream-ordered scratch (cudaMallocAsync, about 136 B per chunk) are enqueued, so the call
+ * can be captured in a CUDA graph; each filter holds 128 KB of device tables for it. */
+int sxgpu_iir_apply_long(sxgpu_iir *f, void *d_cf32, uint64_t nframes, sxgpu_stream stream);
 /* The repeater iteration with its filters: read -> pre -> post -> CF32 block and timed write.
  * Same state, results, positions, CF32 block and playback ring, bit for bit, as sxgpu_bank_read,
  * sxgpu_iir_apply(pre), sxgpu_iir_apply(post), sxgpu_bank_write(bank, d_cf32, SOAPY_SDR_HAS_TIME,

@@ -84,6 +84,7 @@ SIGNATURES = {
     "sxgpu_iir_set_state": (C.c_int, [_P, _P, _P]),
     "sxgpu_iir_get_state": (C.c_int, [_P, _P, _P]),
     "sxgpu_iir_apply": (C.c_int, [_P, _P, C.c_uint32, _P]),
+    "sxgpu_iir_apply_long": (C.c_int, [_P, _P, C.c_uint64, _P]),
     "sxgpu_bank_repeat_filtered": (C.c_int, [_P, _P, _P, _P, C.c_longlong, _P]),
     "sxgpu_bank_read_filtered": (C.c_int, [_P, _P, _P, _P]),
     "sxgpu_bank_write_filtered": (C.c_int, [_P, _P, _P, C.c_int, _P, C.c_longlong, _P]),
@@ -428,6 +429,12 @@ class Iir:
     def apply(self, d_cf32, period, stream=None):
         """Filter d_cf32[nstreams][period] (complex64 on the device) in place."""
         self.ctx.check(self.lib.sxgpu_iir_apply(self.handle, d_cf32, period, stream), "sxgpu_iir_apply")
+
+    def apply_long(self, d_cf32, nframes, stream=None):
+        """Filter d_cf32[nstreams][nframes] in place for any nframes, in parallel along the block: bit
+        for bit `apply` on each stream's first chunk, within float32 rounding of it after that
+        (sxgpu_iir_apply_long in include/sxgpu.h)."""
+        self.ctx.check(self.lib.sxgpu_iir_apply_long(self.handle, d_cf32, nframes, stream), "sxgpu_iir_apply_long")
 
     def state(self, stream=None):
         """The state as scipy's zf: (nsections, nstreams, 2) complex64."""

@@ -2137,10 +2137,63 @@ int sxgpu_bank_playback(sxgpu_bank *bank, uint32_t index, int64_t position, size
 
 struct sxgpu_iir {
     sxgpu_ctx *ctx = nullptr;
-    IirView view = {}; // the state in device memory and the float32 coefficients
+    IirView view = {};        // the state in device memory and the float32 coefficients
+    double *powers = nullptr; // sxgpu_iir_apply_long's P_j = A^(2^j) (sx_iir.cuh), in device memory
 };
 
 namespace {
+
+// P_0 .. P_kIirPowers-1 of sx_iir.cuh's carry, [j][kIirDim][kIirDim] with zeros outside the
+// 2S x 2S corner: A column by column (one float64 step of the cascade on zero input from a unit
+// state), then repeated squaring, each entry summed left to right.  The build's -ffp-contract=off
+// keeps every operation one rounding, as on the device and in tests/sxiir_long.py.
+std::vector<double> iir_power_chain(const IirCoeffs &k)
+{
+    const int n = 2 * int(k.nsections);
+    constexpr size_t kMat = size_t(kIirDim) * kIirDim;
+    std::vector<double> p(kIirPowers * kMat, 0.0);
+    for (int col = 0; col < n; col++) {
+        double z[kIirDim] = {};
+        z[col] = 1.0;
+        double x = 0.0;
+        for (int q = 0; q < int(k.nsections); q++) {
+            const double b0 = k.b0[q], b1 = k.b1[q], b2 = k.b2[q], a1 = k.a1[q], a2 = k.a2[q];
+            const double y = b0 * x + z[2 * q];
+            const double z0 = (b1 * x - a1 * y) + z[2 * q + 1];
+            const double z1 = b2 * x - a2 * y;
+            z[2 * q] = z0;
+            z[2 * q + 1] = z1;
+            x = y;
+        }
+        for (int i = 0; i < n; i++)
+            p[size_t(i) * kIirDim + col] = z[i];
+    }
+    for (int j = 1; j < kIirPowers; j++) {
+        const double *a = &p[(j - 1) * kMat];
+        double *out = &p[j * kMat];
+        for (int i = 0; i < n; i++)
+            for (int col = 0; col < n; col++) {
+                double acc = a[size_t(i) * kIirDim] * a[col];
+                for (int m = 1; m < n; m++)
+                    acc = acc + a[size_t(i) * kIirDim + m] * a[size_t(m) * kIirDim + col];
+                out[size_t(i) * kIirDim + col] = acc;
+            }
+    }
+    return p;
+}
+
+// sxgpu_iir_apply_long's chunk length: a function of the shape alone, so that every GPU computes the
+// same bits.  The longest chunk that still gives about one wave of pass-1 CTAs (65536 rows is 1024
+// CTAs of 64 rows, 7 CTAs on each of the B200's 148 SMs), from 1024 down to 128 frames.
+uint32_t iir_chunk_len(uint64_t nstreams, uint64_t nframes)
+{
+    uint32_t len = 1024;
+    while (len > 128 && nstreams * ((nframes + len - 1) / len) < 65536)
+        len /= 2;
+    return len;
+}
+
+
 
 size_t iir_state_bytes(const IirView &v)
 {
@@ -2204,9 +2257,20 @@ int sxgpu_iir_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t nsections, cons
         return ctx->fail(e, "cudaMemset(filter state)");
     }
     v.state = static_cast<float *>(state);
+    const std::vector<double> chain = iir_power_chain(v.k);
+    void *powers = nullptr;
+    e = cudaMalloc(&powers, chain.size() * sizeof(double));
+    if (e == cudaSuccess)
+        e = cudaMemcpy(powers, chain.data(), chain.size() * sizeof(double), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) {
+        cudaFree(powers);
+        cudaFree(state);
+        return ctx->fail(e, "filter tables");
+    }
     sxgpu_iir *f = new sxgpu_iir();
     f->ctx = ctx;
     f->view = v;
+    f->powers = static_cast<double *>(powers);
     ctx->live_iirs++;
     *out = f;
     return SXGPU_OK;
@@ -2223,6 +2287,7 @@ int sxgpu_iir_destroy(sxgpu_iir *f)
     }
     cudaDeviceSynchronize();
     cudaFree(f->view.state);
+    cudaFree(f->powers);
     f->ctx->live_iirs--;
     delete f;
     return SXGPU_OK;
@@ -2267,9 +2332,79 @@ int sxgpu_iir_apply(sxgpu_iir *f, void *d_cf32, uint32_t period, sxgpu_stream st
         return ctx->invalid("the period is 1 to 65536 frames");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const unsigned grid = unsigned((uint64_t(f->view.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta);
-    iir_apply_kernel<<<grid, kIirThreads, 0, iir_stream(f, stream)>>>(f->view, static_cast<char *>(d_cf32), period);
+    iir_apply_kernel<<<grid, kIirThreads, 0, iir_stream(f, stream)>>>(f->view, static_cast<char *>(d_cf32), period, IirChunks{});
     SX_CUDA(ctx, cudaGetLastError());
     ctx->launches++;
+    return SXGPU_OK;
+}
+
+int sxgpu_iir_apply_long(sxgpu_iir *f, void *d_cf32, uint64_t nframes, sxgpu_stream stream)
+{
+    if (!f)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = f->ctx;
+    if (!d_cf32 || reinterpret_cast<uintptr_t>(d_cf32) % 8)
+        return ctx->invalid("CF32 buffer must be 8-byte aligned device memory");
+    if (nframes == 0)
+        return ctx->invalid("sxgpu_iir_apply_long: a block has at least one frame");
+    const uint64_t nstreams = f->view.nstreams;
+    if (nframes > UINT64_MAX / 8 / nstreams)
+        return ctx->invalid("sxgpu_iir_apply_long: nstreams * nframes * 8 bytes overflows 64 bits");
+    const uint32_t len = iir_chunk_len(nstreams, nframes);
+    const uint64_t chunks = (nframes + len - 1) / len;
+    const uint64_t ctas = (nstreams * chunks + kIirStreamsPerCta - 1) / kIirStreamsPerCta;
+    if (ctas > uint64_t(INT32_MAX))
+        return ctx->invalid("sxgpu_iir_apply_long: the block needs more CTAs than a grid holds");
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = iir_stream(f, stream);
+    char *cf32 = static_cast<char *>(d_cf32);
+    if (chunks == 1) { // the whole block is chunk 0: exactly sxgpu_iir_apply
+        const unsigned grid = unsigned((nstreams + kIirStreamsPerCta - 1) / kIirStreamsPerCta);
+        iir_apply_kernel<<<grid, kIirThreads, 0, st>>>(f->view, cf32, uint32_t(nframes), IirChunks{});
+        SX_CUDA(ctx, cudaGetLastError());
+        ctx->launches++;
+        return SXGPU_OK;
+    }
+    const uint64_t groups = (chunks + kIirGroup - 1) / kIirGroup, sequences = nstreams * groups * 2;
+    const size_t edge_bytes = size_t(nstreams * chunks) * 2 * kIirDim * sizeof(float);
+    const size_t total_bytes = size_t(sequences) * kIirDim * sizeof(double);
+    void *scratch = nullptr;
+    SX_CUDA(ctx, cudaMallocAsync(&scratch, edge_bytes + 2 * total_bytes, st));
+    double *totals[2] = {reinterpret_cast<double *>(static_cast<char *>(scratch) + edge_bytes),
+                         reinterpret_cast<double *>(static_cast<char *>(scratch) + edge_bytes + total_bytes)};
+    IirChunks ch = {nframes, chunks, nstreams * (chunks - 1), len, static_cast<float *>(scratch)};
+    IirCarry a = {f->powers, ch, nullptr, totals[0], groups, sequences, 0};
+    while ((1u << a.log2_len) < len)
+        a.log2_len++;
+    const unsigned carry_grid = unsigned((sequences * 16 + 127) / 128);
+    int launches = 0;
+    cudaError_t e = cudaSuccess;
+    auto launched = [&]() {
+        if (e == cudaSuccess)
+            e = cudaGetLastError();
+        launches++;
+    };
+    iir_apply_kernel<kIirRowsChunkEnds>
+        <<<unsigned((ch.rows + kIirStreamsPerCta - 1) / kIirStreamsPerCta), kIirThreads, 0, st>>>(f->view, cf32, 0, ch);
+    launched();
+    iir_carry_reduce_kernel<<<carry_grid, 128, 0, st>>>(f->view, a);
+    launched();
+    for (uint32_t level = 0; (uint64_t(1) << level) < groups; level++) {
+        a.in = a.out;
+        a.out = totals[a.out == totals[0] ? 1 : 0];
+        iir_carry_scan_kernel<<<carry_grid, 128, 0, st>>>(f->view, a, level);
+        launched();
+    }
+    a.in = a.out;
+    iir_carry_fixup_kernel<<<carry_grid, 128, 0, st>>>(f->view, a);
+    launched();
+    ch.rows = nstreams * chunks;
+    iir_apply_kernel<kIirRowsChunkOut><<<unsigned(ctas), kIirThreads, 0, st>>>(f->view, cf32, 0, ch);
+    launched();
+    cudaFreeAsync(scratch, st);
+    if (e != cudaSuccess)
+        return ctx->fail(e, "sxgpu_iir_apply_long");
+    ctx->launches += launches;
     return SXGPU_OK;
 }
 
