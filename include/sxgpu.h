@@ -280,6 +280,46 @@ int sxgpu_bank_write_filtered(sxgpu_bank *bank, sxgpu_iir *f, const void *d_cf32
  * sx::IirView).  out_bytes must be sizeof(sx::IirView). */
 int sxgpu_iir_device_view(sxgpu_iir *f, void *out, size_t out_bytes);
 
+/* ---- stateful FIR filters and rational resamplers for streams ------------------------------ */
+
+/* Linear-phase channel filters (firwin, remez, Kaiser designs) and sample-rate changes by up/down:
+ * real taps h[0..ntaps-1] applied to I and Q independently, with the last inputs carried from call
+ * to call, one history per stream.  A stream fed X frames in total, over any sequence of calls, has
+ * emitted exactly the first ceil(X up / down) outputs of scipy.signal.upfirdn(h, x, up, down) with
+ * h rounded to float32 and x complex64, bit for bit (DESIGN.md, "Parity policy"; tests/sxfir.py
+ * restates it).  Polyphase, hp = ceil(ntaps / up) taps per phase: output n is the float32 sum,
+ * oldest input first from +0, of x[(n down) div up - j] * h[(n down) mod up + up j] over
+ * j = hp-1 .. 0, every product and sum rounded on its own (no FMA).  upfirdn's flush tail is what
+ * feeding zeros gives.  Every stream of a filter is fed the same number of frames per call. */
+#define SXGPU_FIR_MAX_TAPS 4096
+#define SXGPU_FIR_MAX_FACTOR 256
+typedef struct sxgpu_fir sxgpu_fir;
+/* h: ntaps taps as double, rounded to float32 once, here.  Refused: nstreams 0, ntaps 0 or above
+ * SXGPU_FIR_MAX_TAPS, up or down 0 or above SXGPU_FIR_MAX_FACTOR, a NULL h, a tap that is not
+ * finite.  The history starts at zero and the phase at 0.  sxgpu_destroy of the context refuses
+ * while a filter is alive. */
+int sxgpu_fir_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t ntaps, const double *h, uint32_t up,
+                     uint32_t down, sxgpu_fir **out);
+int sxgpu_fir_destroy(sxgpu_fir *f);
+/* The frames each stream's next apply of nin frames emits: ceil((p + nin) up / down) -
+ * ceil(p up / down), p the phase.  Host arithmetic, no GPU work. */
+int sxgpu_fir_output_frames(sxgpu_fir *f, uint64_t nin, uint64_t *nout);
+/* d_in[nstreams][nin] -> d_out[nstreams][*nout], CF32, the history and the phase carried; *nout
+ * (may be NULL) is written on return.  The phase, X mod down, lives on the host and is all the call
+ * depends on besides the buffers, so a call with nin a multiple of down (which leaves the phase as
+ * it was) may be captured in a CUDA graph and replayed; other calls must not be.  Only kernels are
+ * enqueued: fir_apply_kernel when the call emits at least one frame, then fir_history_kernel when
+ * hp > 1 (the new history, written after every read of the old one), so 2 launches per call at most.
+ * Refused: nin 0, a NULL or not 8-byte aligned buffer, byte sizes that overflow 64 bits, d_in and
+ * d_out overlapping, a grid of more than 2^31 - 1 CTAs. */
+int sxgpu_fir_apply(sxgpu_fir *f, const void *d_in, uint64_t nin, void *d_out, uint64_t *nout,
+                    sxgpu_stream stream);
+/* The history, [nstreams][hp - 1] complex64 on the host, oldest frame first (nothing when hp = 1),
+ * and the phase.  get: either pointer may be NULL.  set: NULL h_hist = zeros; a phase of down or
+ * more is refused.  Both synchronise with `stream`. */
+int sxgpu_fir_get_state(sxgpu_fir *f, void *h_hist, uint32_t *phase, sxgpu_stream stream);
+int sxgpu_fir_set_state(sxgpu_fir *f, const void *h_hist, uint32_t phase, sxgpu_stream stream);
+
 /* ---- the hot path, host buffers ---------------------------------------------------------- */
 
 /* Same contracts as the two converters above, but src and dest are HOST memory, as they

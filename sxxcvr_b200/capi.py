@@ -89,6 +89,12 @@ SIGNATURES = {
     "sxgpu_bank_read_filtered": (C.c_int, [_P, _P, _P, _P]),
     "sxgpu_bank_write_filtered": (C.c_int, [_P, _P, _P, C.c_int, _P, C.c_longlong, _P]),
     "sxgpu_iir_device_view": (C.c_int, [_P, _P, _S]),
+    "sxgpu_fir_create": (C.c_int, [_P, C.c_uint32, C.c_uint32, _P, C.c_uint32, C.c_uint32, C.POINTER(_P)]),
+    "sxgpu_fir_destroy": (C.c_int, [_P]),
+    "sxgpu_fir_output_frames": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "sxgpu_fir_apply": (C.c_int, [_P, _P, C.c_uint64, _P, C.POINTER(C.c_uint64), _P]),
+    "sxgpu_fir_get_state": (C.c_int, [_P, _P, C.POINTER(C.c_uint32), _P]),
+    "sxgpu_fir_set_state": (C.c_int, [_P, _P, C.c_uint32, _P]),
     "sxgpu_convert_rx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S]),
     "sxgpu_convert_rx_buffer_host_gated": (C.c_int, [_P, _P, _S, _P, _S, _S, _P, _P]),
     "sxgpu_convert_tx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S, _F]),
@@ -451,6 +457,68 @@ class Iir:
                 raise ValueError(f"zi must have shape {(self.nsections, self.nstreams, 2)}, got {zi.shape}")
             ptr = zi.ctypes.data
         self.ctx.check(self.lib.sxgpu_iir_set_state(self.handle, ptr, stream), "sxgpu_iir_set_state")
+
+
+class Fir:
+    """Real FIR taps with an up/down rate change and one history per stream (sxgpu_fir_* in
+    include/sxgpu.h): scipy.signal.upfirdn(taps, x, up, down) on each stream's concatenated input,
+    bit for bit, carried from call to call.  up = down = 1 is a plain FIR filter."""
+
+    def __init__(self, ctx: Context, nstreams: int, taps, up: int = 1, down: int = 1):
+        import numpy as np
+        self.np = np
+        self.ctx, self.lib = ctx, ctx.lib
+        self.handle = None
+        taps = np.ascontiguousarray(np.asarray(taps, dtype=np.float64))
+        if taps.ndim != 1:
+            raise ValueError(f"taps must be one-dimensional, got shape {taps.shape}")
+        h = _P()
+        ctx.check(self.lib.sxgpu_fir_create(ctx.handle, nstreams, taps.size, taps.ctypes.data if taps.size else None,
+                                            up, down, C.byref(h)), "sxgpu_fir_create")
+        self.handle, self.nstreams, self.ntaps, self.up, self.down = h, nstreams, taps.size, up, down
+        self.hp = -(-taps.size // up)
+
+    def close(self):
+        if self.handle:
+            self.lib.sxgpu_fir_destroy(self.handle)
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def output_frames(self, nin) -> int:
+        """Frames each stream's next apply of nin frames emits."""
+        n = C.c_uint64()
+        self.ctx.check(self.lib.sxgpu_fir_output_frames(self.handle, nin, C.byref(n)), "sxgpu_fir_output_frames")
+        return n.value
+
+    def apply(self, d_in, nin, d_out, stream=None) -> int:
+        """d_in[nstreams][nin] -> d_out[nstreams][nout] (complex64 on the device); returns nout."""
+        n = C.c_uint64()
+        self.ctx.check(self.lib.sxgpu_fir_apply(self.handle, d_in, nin, d_out, C.byref(n), stream), "sxgpu_fir_apply")
+        return n.value
+
+    def state(self, stream=None):
+        """(history, phase): the last hp - 1 inputs of each stream, (nstreams, hp - 1) complex64 oldest
+        first, and the frames fed so far mod down."""
+        hist = self.np.empty((self.nstreams, self.hp - 1), self.np.complex64)
+        phase = C.c_uint32()
+        self.ctx.check(self.lib.sxgpu_fir_get_state(self.handle, hist.ctypes.data, C.byref(phase), stream),
+                       "sxgpu_fir_get_state")
+        return hist, phase.value
+
+    def set_state(self, hist=None, phase=0, stream=None):
+        """Set the history, (nstreams, hp - 1) complex64 (None = zeros), and the phase."""
+        ptr = None
+        if hist is not None:
+            hist = self.np.ascontiguousarray(hist, dtype=self.np.complex64)
+            if hist.shape != (self.nstreams, self.hp - 1):
+                raise ValueError(f"hist must have shape {(self.nstreams, self.hp - 1)}, got {hist.shape}")
+            ptr = hist.ctypes.data
+        self.ctx.check(self.lib.sxgpu_fir_set_state(self.handle, ptr, phase, stream), "sxgpu_fir_set_state")
 
 
 class Multi:

@@ -9,6 +9,7 @@
 #include "sx_kernels.cuh"
 #include "sx_bank.cuh"
 #include "sx_iir.cuh"
+#include "sx_fir.cuh"
 #include "sx_resident.cuh"
 #include "host/par_copy.hpp"
 #include "host/worker_pool.hpp"
@@ -126,6 +127,7 @@ struct sxgpu_ctx {
     std::atomic<uint64_t> resident_launches{0}, resident_calls{0}, flagged_calls{0};
     std::atomic<int> live_banks{0}; // banks keep a pointer to their context
     std::atomic<int> live_iirs{0};  // so do filters
+    std::atomic<int> live_firs{0};
     bool l2_carveout_set = false;   // sxgpu_bank_repeat_begin sets the persisting-L2 limit once
 
     // host pipeline: lane 0 serves the RX conversions, lane 1 the TX conversions
@@ -1462,7 +1464,7 @@ int sxgpu_destroy(sxgpu_ctx *ctx)
         return SXGPU_ERR_INVALID;
     if (ctx->live_banks.load() != 0)
         return ctx->invalid("destroy the context's stream banks first");
-    if (ctx->live_iirs.load() != 0)
+    if (ctx->live_iirs.load() != 0 || ctx->live_firs.load() != 0)
         return ctx->invalid("destroy the context's filters first");
     cudaSetDevice(ctx->device);
     for (HostLane &lane : ctx->lanes) {
@@ -2485,6 +2487,257 @@ int sxgpu_iir_device_view(sxgpu_iir *f, void *out, size_t out_bytes)
     if (out_bytes != sizeof(IirView))
         return f->ctx->invalid("sxgpu_iir_device_view: size mismatch (header and library disagree)");
     std::memcpy(out, &f->view, sizeof(IirView));
+    return SXGPU_OK;
+}
+
+// ---- stateful FIR filters and rational resamplers (sx_fir.cuh) ------------------------------------
+} // extern "C"
+
+struct sxgpu_fir {
+    sxgpu_ctx *ctx = nullptr;
+    uint32_t nstreams = 0, up = 1, down = 1, g = 1, up1 = 1, down1 = 1, hp = 1, rows = 1;
+    uint32_t phase = 0;       // frames fed so far mod down: the only state kept on the host
+    float4 *taps = nullptr;   // [up][rows] tap tables (FirCall::taps), device memory
+    float2 *hist = nullptr;   // [nstreams][hp - 1], device memory; NULL when hp == 1
+};
+
+namespace {
+
+constexpr size_t kFirWindowBytes = 200 * 1024; // fir_apply_kernel's window stays below the 227 KB of an SM
+
+// Outputs a call of nin frames emits from phase r: ceil((r + nin) U / D) - ceil(r U / D), or
+// UINT64_MAX if that does not fit.
+uint64_t fir_outputs(const sxgpu_fir *f, uint32_t r, uint64_t nin)
+{
+    const unsigned __int128 up = f->up, down = f->down;
+    const unsigned __int128 end = ((r + (unsigned __int128)nin) * up + down - 1) / down;
+    const unsigned __int128 n = end - (r * up + down - 1) / down;
+    return n > UINT64_MAX ? UINT64_MAX : uint64_t(n);
+}
+
+size_t fir_hist_bytes(const sxgpu_fir *f)
+{
+    return size_t(f->nstreams) * (f->hp - 1) * sizeof(float2);
+}
+
+cudaStream_t fir_stream(sxgpu_fir *f, sxgpu_stream stream)
+{
+    return stream ? static_cast<cudaStream_t>(stream) : f->ctx->stream;
+}
+
+} // namespace
+
+extern "C" {
+
+int sxgpu_fir_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t ntaps, const double *h, uint32_t up, uint32_t down,
+                     sxgpu_fir **out)
+{
+    if (!ctx || !out)
+        return SXGPU_ERR_INVALID;
+    *out = nullptr;
+    if (nstreams == 0 || nstreams > uint32_t(INT32_MAX))
+        return ctx->invalid("a FIR filter has 1 to 2^31 - 1 streams (one CTA each for the history)");
+    if (ntaps < 1 || ntaps > SXGPU_FIR_MAX_TAPS || !h)
+        return ctx->invalid("a FIR filter has 1 to SXGPU_FIR_MAX_TAPS taps");
+    if (up < 1 || up > SXGPU_FIR_MAX_FACTOR || down < 1 || down > SXGPU_FIR_MAX_FACTOR)
+        return ctx->invalid("up and down are 1 to SXGPU_FIR_MAX_FACTOR");
+    for (uint32_t i = 0; i < ntaps; i++)
+        if (!std::isfinite(h[i]))
+            return ctx->invalid("every FIR tap must be finite");
+    std::unique_ptr<sxgpu_fir> f(new sxgpu_fir());
+    f->ctx = ctx;
+    f->nstreams = nstreams;
+    f->up = up;
+    f->down = down;
+    uint32_t g = up, d = down;
+    while (d) {
+        const uint32_t t = g % d;
+        g = d;
+        d = t;
+    }
+    f->g = g;
+    f->up1 = up / g;
+    f->down1 = down / g;
+    f->hp = (ntaps + up - 1) / up;
+    f->rows = (kFirBlock - 1) * f->down1 + f->hp;
+    // Row q of phase t's table holds, for i < kFirBlock, tap s = q - i D' of the phase in
+    // accumulation order, h[t + U (hp - 1 - s)] (0 past the taps, and where that s does not exist).
+    std::vector<float> taps(size_t(up) * f->rows * 4, 0.0f);
+    for (uint32_t t = 0; t < up; t++)
+        for (uint32_t q = 0; q < f->rows; q++)
+            for (uint32_t i = 0; i < uint32_t(kFirBlock); i++) {
+                if (q < i * f->down1 || q - i * f->down1 >= f->hp)
+                    continue;
+                const uint64_t j = t + uint64_t(up) * (f->hp - 1 - (q - i * f->down1));
+                taps[(size_t(t) * f->rows + q) * 4 + i] = j < ntaps ? float(h[j]) : 0.0f;
+            }
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t smem = std::min<size_t>(kFirWindowBytes, ctx->prop.sharedMemPerBlockOptin);
+    SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    void *d_taps = nullptr, *d_hist = nullptr;
+    cudaError_t e = cudaMalloc(&d_taps, taps.size() * sizeof(float));
+    if (e == cudaSuccess)
+        e = cudaMemcpy(d_taps, taps.data(), taps.size() * sizeof(float), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && f->hp > 1) {
+        e = cudaMalloc(&d_hist, fir_hist_bytes(f.get()));
+        if (e == cudaSuccess)
+            e = cudaMemsetAsync(d_hist, 0, fir_hist_bytes(f.get()), ctx->stream);
+        if (e == cudaSuccess)
+            e = cudaStreamSynchronize(ctx->stream);
+    }
+    if (e != cudaSuccess) {
+        cudaFree(d_hist);
+        cudaFree(d_taps);
+        return ctx->fail(e, "cudaMalloc(FIR filter)");
+    }
+    f->taps = static_cast<float4 *>(d_taps);
+    f->hist = static_cast<float2 *>(d_hist);
+    ctx->live_firs++;
+    *out = f.release();
+    return SXGPU_OK;
+}
+
+int sxgpu_fir_destroy(sxgpu_fir *f)
+{
+    if (!f)
+        return SXGPU_ERR_INVALID;
+    cudaSetDevice(f->ctx->device);
+    for (HostLane &lane : f->ctx->lanes) { // a resident converter would hold the device-wide sync up
+        std::lock_guard<std::mutex> lock(lane.mutex);
+        resident_stop(f->ctx, lane);
+    }
+    cudaDeviceSynchronize();
+    cudaFree(f->hist);
+    cudaFree(f->taps);
+    f->ctx->live_firs--;
+    delete f;
+    return SXGPU_OK;
+}
+
+int sxgpu_fir_output_frames(sxgpu_fir *f, uint64_t nin, uint64_t *nout)
+{
+    if (!f || !nout)
+        return SXGPU_ERR_INVALID;
+    const uint64_t n = fir_outputs(f, f->phase, nin);
+    if (n == UINT64_MAX)
+        return f->ctx->invalid("sxgpu_fir_output_frames: the output count overflows 64 bits");
+    *nout = n;
+    return SXGPU_OK;
+}
+
+int sxgpu_fir_apply(sxgpu_fir *f, const void *d_in, uint64_t nin, void *d_out, uint64_t *nout, sxgpu_stream stream)
+{
+    if (!f)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = f->ctx;
+    if (!d_in || !d_out || reinterpret_cast<uintptr_t>(d_in) % 8 || reinterpret_cast<uintptr_t>(d_out) % 8)
+        return ctx->invalid("sxgpu_fir_apply: input and output must be 8-byte aligned device memory");
+    if (nin == 0)
+        return ctx->invalid("sxgpu_fir_apply: a block has at least one frame");
+    const uint64_t nstreams = f->nstreams;
+    if (nin > UINT64_MAX / 8 / nstreams)
+        return ctx->invalid("sxgpu_fir_apply: nstreams * nin * 8 bytes overflows 64 bits");
+    const uint64_t n = fir_outputs(f, f->phase, nin);
+    if (n > UINT64_MAX / 8 / nstreams)
+        return ctx->invalid("sxgpu_fir_apply: nstreams * nout * 8 bytes overflows 64 bits");
+    const uintptr_t in0 = reinterpret_cast<uintptr_t>(d_in), out0 = reinterpret_cast<uintptr_t>(d_out);
+    const uint64_t in_bytes = nstreams * nin * 8, out_bytes = nstreams * n * 8;
+    if (out_bytes && (in0 >= out0 ? in0 - out0 < out_bytes : out0 - in0 < in_bytes))
+        return ctx->invalid("sxgpu_fir_apply: input and output overlap");
+
+    FirCall a = {};
+    a.in = static_cast<const float2 *>(d_in);
+    a.out = static_cast<float2 *>(d_out);
+    a.hist = f->hist;
+    a.taps = f->taps;
+    a.nin = nin;
+    a.nout = n;
+    a.c0 = (uint64_t(f->phase) * f->up + f->down - 1) / f->down;
+    a.a_lo = a.c0 / f->up1;
+    a.hp = f->hp;
+    a.rows = f->rows;
+    a.g = f->g;
+    a.up1 = f->up1;
+    a.down1 = f->down1;
+    a.phase = f->phase;
+    int block = 0; // R of fir_apply_kernel
+    size_t smem = 0;
+    if (n) {
+        const uint64_t classes = (a.c0 + n - 1) / f->up1 - a.a_lo + 1; // class indices a the call covers
+        const uint32_t e_max = (f->up1 - 1) * f->down1 / f->up1;
+        for (block = classes >= 128 ? 4 : classes >= 64 ? 2 : 1;; block /= 2) {
+            const uint32_t seg = uint32_t(block) * f->down1;
+            a.win_len = 32 * seg + e_max + f->hp;
+            a.pad = seg % 2 == 0;
+            smem = (a.win_len + (a.pad ? a.win_len / seg : 0)) * sizeof(float2);
+            if (smem <= kFirWindowBytes || block == 1)
+                break;
+        }
+        a.chunks = (classes + 32 * block - 1) / (32 * block);
+        if (a.chunks > uint64_t(INT32_MAX) / nstreams)
+            return ctx->invalid("sxgpu_fir_apply: the block needs more CTAs than a grid holds");
+    }
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = fir_stream(f, stream);
+    int launches = 0;
+    if (n) {
+        const unsigned grid = unsigned(nstreams * a.chunks);
+        if (block == 4)
+            fir_apply_kernel<4><<<grid, 32, smem, st>>>(a);
+        else if (block == 2)
+            fir_apply_kernel<2><<<grid, 32, smem, st>>>(a);
+        else
+            fir_apply_kernel<1><<<grid, 32, smem, st>>>(a);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
+    if (f->hp > 1) {
+        fir_history_kernel<<<unsigned(nstreams), kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(a);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
+    ctx->launches += launches;
+    f->phase = uint32_t((f->phase + nin % f->down) % f->down);
+    if (nout)
+        *nout = n;
+    return SXGPU_OK;
+}
+
+int sxgpu_fir_get_state(sxgpu_fir *f, void *h_hist, uint32_t *phase, sxgpu_stream stream)
+{
+    if (!f)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = f->ctx;
+    if (h_hist && f->hp > 1) {
+        SX_CUDA(ctx, cudaSetDevice(ctx->device));
+        cudaStream_t st = fir_stream(f, stream);
+        SX_CUDA(ctx, cudaMemcpyAsync(h_hist, f->hist, fir_hist_bytes(f), cudaMemcpyDeviceToHost, st));
+        SX_CUDA(ctx, cudaStreamSynchronize(st));
+    }
+    if (phase)
+        *phase = f->phase;
+    return SXGPU_OK;
+}
+
+int sxgpu_fir_set_state(sxgpu_fir *f, const void *h_hist, uint32_t phase, sxgpu_stream stream)
+{
+    if (!f)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = f->ctx;
+    if (phase >= f->down)
+        return ctx->invalid("sxgpu_fir_set_state: the phase is below down");
+    if (f->hp > 1) {
+        SX_CUDA(ctx, cudaSetDevice(ctx->device));
+        cudaStream_t st = fir_stream(f, stream);
+        if (h_hist)
+            SX_CUDA(ctx, cudaMemcpyAsync(f->hist, h_hist, fir_hist_bytes(f), cudaMemcpyHostToDevice, st));
+        else
+            SX_CUDA(ctx, cudaMemsetAsync(f->hist, 0, fir_hist_bytes(f), st));
+        SX_CUDA(ctx, cudaStreamSynchronize(st));
+    }
+    f->phase = phase;
     return SXGPU_OK;
 }
 
