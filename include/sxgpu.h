@@ -319,6 +319,39 @@ int sxgpu_fir_apply(sxgpu_fir *f, const void *d_in, uint64_t nin, void *d_out, u
  * more is refused.  Both synchronise with `stream`. */
 int sxgpu_fir_get_state(sxgpu_fir *f, void *h_hist, uint32_t *phase, sxgpu_stream stream);
 int sxgpu_fir_set_state(sxgpu_fir *f, const void *h_hist, uint32_t phase, sxgpu_stream stream);
+/* The bank's two halves with a FIR filter or resampler fused in: a bank of receivers that decimates
+ * every stream to its channel rate, a bank of transmitters that interpolates each stream's
+ * channel-rate block up to the bank's rate, without the full-rate CF32 block in memory.  The split
+ * repeater around channel-rate DSP is read_fir(F, decimating), the caller's kernels on d_out, then
+ * write_fir(G, interpolating, SOAPY_SDR_HAS_TIME, NULL, rx_time_offset_ns), as read_filtered /
+ * write_filtered are for IIR filters.
+ * Both need f of this context with the bank's stream count and an 8-byte aligned device buffer
+ * (frames are stored one at a time: no even-period or 16-byte requirement).  Refused with
+ * SXGPU_ERR_INVALID and nothing enqueued: a NULL or foreign filter, a stream-count mismatch, a NULL
+ * or unaligned buffer, byte sizes that overflow 64 bits, a data kernel of more than 2^31 - 1 CTAs,
+ * and (write only) an nin from which f does not emit exactly one period.
+ * Only kernels are enqueued: the bank's plan kernel, then the FIR data kernel as its programmatic
+ * dependent when the filter emits at least one frame (always, for the write), then
+ *   read:  bank_fir_read_tail_kernel when hp > 1 or the capture is synthetic (the new history and
+ *          the capture slot);
+ *   write: fir_history_kernel when hp > 1;
+ * so 3 launches per call at most, counted in "launches".  Each adds to frames_rx / frames_tx as the
+ * plain call does.  A call whose frames fed to the filter (period for the read, nin for the write)
+ * are a multiple of down leaves the phase as it was and may be captured in a CUDA graph, as for
+ * sxgpu_fir_apply.
+ * sxgpu_bank_read, then sxgpu_fir_apply(f, that block, period, d_out, nout): the same positions,
+ * results, capture slots, filter history and phase and d_out[nstreams][*nout] (nout may be NULL),
+ * with *nout = sxgpu_fir_output_frames(f, period) before the call; bit for bit, for synthetic and
+ * ingested capture, through overruns, and when the call emits nothing. */
+int sxgpu_bank_read_fir(sxgpu_bank *bank, sxgpu_fir *f, void *d_out, uint64_t *nout, sxgpu_stream stream);
+/* sxgpu_fir_apply(f, d_in, nin, tmp, &n), then sxgpu_bank_write(bank, tmp, flags, d_time_ns,
+ * rx_time_offset_ns): the same positions, results, playback rings and filter history and phase, bit
+ * for bit.  d_in[nstreams][nin] is not modified.  The filter advances also when a stream's write is
+ * dropped as late.  f must emit exactly `period` frames from nin at its current phase, by the
+ * arithmetic of sxgpu_fir_output_frames: for an interpolator by up, nin = period / up; for up'/down'
+ * in lowest terms, nin = period down' / up' always does when up' divides the period. */
+int sxgpu_bank_write_fir(sxgpu_bank *bank, sxgpu_fir *f, const void *d_in, uint64_t nin, int flags,
+                         const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream);
 
 /* ---- the hot path, host buffers ---------------------------------------------------------- */
 

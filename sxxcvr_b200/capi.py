@@ -95,6 +95,8 @@ SIGNATURES = {
     "sxgpu_fir_apply": (C.c_int, [_P, _P, C.c_uint64, _P, C.POINTER(C.c_uint64), _P]),
     "sxgpu_fir_get_state": (C.c_int, [_P, _P, C.POINTER(C.c_uint32), _P]),
     "sxgpu_fir_set_state": (C.c_int, [_P, _P, C.c_uint32, _P]),
+    "sxgpu_bank_read_fir": (C.c_int, [_P, _P, _P, C.POINTER(C.c_uint64), _P]),
+    "sxgpu_bank_write_fir": (C.c_int, [_P, _P, _P, C.c_uint64, C.c_int, _P, C.c_longlong, _P]),
     "sxgpu_convert_rx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S]),
     "sxgpu_convert_rx_buffer_host_gated": (C.c_int, [_P, _P, _S, _P, _S, _S, _P, _P]),
     "sxgpu_convert_tx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S, _F]),
@@ -360,6 +362,19 @@ class Bank:
         """write() of d_cf32 filtered by f, in one pass that leaves d_cf32 as it was (f None: write)."""
         self.ctx.check(self.lib.sxgpu_bank_write_filtered(self.handle, f.handle if f else None, d_cf32, flags, d_time_ns,
                                                           rx_time_offset_ns, stream), "sxgpu_bank_write_filtered")
+
+    def read_fir(self, f: "Fir", d_out, stream=None) -> int:
+        """read() then f.apply(that block, period, d_out) in one call, without the full-rate block;
+        returns nout, the frames per stream written to d_out."""
+        n = C.c_uint64()
+        self.ctx.check(self.lib.sxgpu_bank_read_fir(self.handle, f.handle if f else None, d_out, C.byref(n), stream),
+                       "sxgpu_bank_read_fir")
+        return n.value
+
+    def write_fir(self, f: "Fir", d_in, nin, flags=4, d_time_ns=None, rx_time_offset_ns=0, stream=None):
+        """write() of f.apply(d_in, nin), which must be one period, in one call that leaves d_in as it was."""
+        self.ctx.check(self.lib.sxgpu_bank_write_fir(self.handle, f.handle if f else None, d_in, nin, flags, d_time_ns,
+                                                     rx_time_offset_ns, stream), "sxgpu_bank_write_fir")
 
     def repeat_begin(self, d_cf32, stream=None):
         self.ctx.check(self.lib.sxgpu_bank_repeat_begin(self.handle, d_cf32, stream), "sxgpu_bank_repeat_begin")

@@ -37,11 +37,17 @@
 //     bank_plan_{repeat,read,write}_kernel, then bank_repeat_iir_kernel<Hook, MODE>: whole
 //                             streams per CTA through shared-memory tiles, as a programmatic
 //                             dependent of the plan kernel
+// and a half with a FIR filter or resampler (every bank size) as:
+//     bank_plan_{read,write}_kernel, then bank_fir_kernel<R, MODE>: fir_apply_kernel's polyphase
+//                             tiles with the frames taken from the capture or stored into the
+//                             ring, as a programmatic dependent of the plan kernel, then
+//                             bank_fir_read_tail_kernel / fir_history_kernel
 // The virtual clock follows the same rule as the host-side ALSA stand-in: it moves when a
 // blocking transfer must wait (by exactly the deficit) or when the owner advances it.
 #pragma once
 
 #include "host/stream_plan.hpp"
+#include "sx_fir.cuh"
 #include "sx_iir.cuh"
 #include "sx_kernels.cuh"
 #include "sx_time.h"
@@ -926,12 +932,13 @@ inline const char *bank_repeat_iir_invalid(const BankState &b, const void *cf32,
 // decisions instead of after them; it waits for them with pdl_wait() before it reads them.
 // ---------------------------------------------------------------------------------------
 template <class... Params, class... Args>
-inline cudaError_t launch_dependent(void (*kernel)(Params...), unsigned grid, unsigned block, cudaStream_t st,
+inline cudaError_t launch_dependent(void (*kernel)(Params...), unsigned grid, unsigned block, size_t smem, cudaStream_t st,
                                     const Args &...args)
 {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(block);
+    cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -968,7 +975,7 @@ inline cudaError_t launch_bank_planned(const BankState &b, char *cf32, bool capt
     if (e != cudaSuccess)
         return e;
     const uint64_t vectors = uint64_t(b.nstreams) * (b.period / 2);
-    return launch_dependent(bank_repeat_data_kernel<U, Hook, MODE>, unsigned((vectors + 256 * U - 1) / (256 * U)), 256, st, b,
+    return launch_dependent(bank_repeat_data_kernel<U, Hook, MODE>, unsigned((vectors + 256 * U - 1) / (256 * U)), 256, 0, st, b,
                             cf32, capture_in_slot, hook);
 }
 
@@ -983,8 +990,101 @@ inline cudaError_t launch_bank_iir(const BankState &b, char *cf32, bool capture_
     if (e != cudaSuccess)
         return e;
     return launch_dependent(bank_repeat_iir_kernel<Hook, MODE>,
-                            unsigned((uint64_t(b.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta), kIirThreads, st, b,
+                            unsigned((uint64_t(b.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta), kIirThreads, 0, st, b,
                             cf32, capture_in_slot, pre, post, hook);
+}
+
+// ---------------------------------------------------------------------------------------
+// A half with a FIR filter or resampler (sxgpu_bank_read_fir, sxgpu_bank_write_fir): the same
+// state, results, capture, ring, filter history and outputs as the plain half and sxgpu_fir_apply
+// one after the other, without the full-rate CF32 block in memory.
+//
+// bank_fir_kernel<R, MODE> is fir_apply_kernel<R> (sx_fir.cuh: one warp per CTA, one tile of
+// 32 R class indices of one stream per CTA, same grid, same window, same arithmetic) after the
+// plan kernel, with the frames and the outputs moved:
+//   read mode (after bank_plan_read_kernel): input frame i of stream s is RxCf32 of capture frame
+//     i of the period -- sx_synth_frame(seed + s, rx_first_frame[s] + i), or the ingested slot --
+//     and the outputs go to the caller's block as in fir_apply_kernel.  The capture slot and the
+//     new history are bank_fir_read_tail_kernel's.
+//   write mode (after bank_plan_write_kernel(..., for_data_kernel = true), which has written the
+//     silence of forwarded-over gaps): input frames come from the caller's block, and output k,
+//     through TxCf32, goes to the ring at frame tx_write_position[s] + k: at byte offset
+//     tx_ring_offset[s] + 8 k when the block starts on a period boundary of the ring, frame by
+//     frame through ring_frame() when it straddles two slices, nowhere when the write was dropped
+//     as late.  The new history is fir_history_kernel's, from the caller's block as for apply.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ float2 rx_frame(const Pack<2> &cap)
+{
+    Pack<2> f;
+    RxCf32::apply<1>(cap, f, 0.0f);
+    return make_float2(__uint_as_float(f.w[0]), __uint_as_float(f.w[1]));
+}
+
+template <int R, int MODE>
+__global__ void __launch_bounds__(32) bank_fir_kernel(BankState b, const __grid_constant__ FirCall a, bool capture_in_slot)
+{
+    extern __shared__ __align__(16) float2 win[];
+    const uint64_t stream = blockIdx.x / a.chunks, chunk = blockIdx.x % a.chunks;
+    pdl_wait(); // the decisions, and everything before them on the stream, are in memory
+    if constexpr (MODE == kBankModeRead) {
+        auto out = [&](uint64_t k, float2 v) { a.out[stream * a.nout + k] = v; };
+        if (capture_in_slot) {
+            const char *slot = b.capture_stage + stream * b.period * 8;
+            fir_tile<R>(a, threadIdx.x, stream, chunk, win, [&](const float2 *, uint64_t i) { return rx_frame(ld_stream<8>(slot + i * 8)); }, out);
+        } else {
+            const uint64_t seed = b.seed + stream, first = uint64_t(b.rx_first_frame[stream]);
+            fir_tile<R>(a, threadIdx.x, stream, chunk, win, [&](const float2 *, uint64_t i) { return rx_frame(capture_frame(seed, first + i)); }, out);
+        }
+    } else {
+        const long long off = b.tx_ring_offset[stream];
+        if (off < 0)
+            return; // dropped as late: nothing is stored (the history still advances, fir_history_kernel)
+        const long long at = b.tx_write_position[stream];
+        fir_tile<R>(a, threadIdx.x, stream, chunk, win, [](const float2 *row, uint64_t i) { return row[i]; }, [&](uint64_t k, float2 v) {
+            Pack<2> f, w;
+            f.w[0] = __float_as_uint(v.x), f.w[1] = __float_as_uint(v.y);
+            TxCf32::apply<1>(f, w, b.thr2);
+            st_stream<8>((off & 1) == 0 ? b.playback_ring + off + k * 8 : ring_frame(b, stream, uint64_t(at) + k), w);
+        });
+    }
+}
+
+// After a read's bank_fir_kernel (or straight after the plan when the call emits nothing), one CTA
+// per stream: the new history, the last hp - 1 frames of old history ++ RX(capture), read before
+// any of it is overwritten as in fir_history_kernel; and with synthetic capture the whole capture
+// slot, every frame once with the value sxgpu_bank_read stores.  (The data kernel's CTAs stage
+// overlapping windows, so none of them owns the slot's frames; here they are written in order.)
+__global__ void __launch_bounds__(kFirHistoryThreads) bank_fir_read_tail_kernel(BankState b, const __grid_constant__ FirCall a,
+                                                                                bool capture_in_slot)
+{
+    extern __shared__ __align__(16) float2 keep[]; // [hp - 1]
+    const uint32_t n = a.hp - 1;
+    const uint64_t s = blockIdx.x;
+    char *slot = b.capture_stage + s * b.period * 8;
+    const uint64_t seed = b.seed + s, first = capture_in_slot ? 0 : uint64_t(b.rx_first_frame[s]);
+    float2 *hist = a.hist + s * n;
+    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads) {
+        const uint64_t k = a.nin + i; // buffer frame
+        keep[i] = k < n ? hist[k] : rx_frame(capture_in_slot ? ld_stream<8>(slot + (k - n) * 8) : capture_frame(seed, first + k - n));
+    }
+    for (uint32_t i = threadIdx.x; i < b.period && !capture_in_slot; i += kFirHistoryThreads)
+        st_stream<8>(slot + size_t(i) * 8, capture_frame(seed, first + i));
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads)
+        hist[i] = keep[i];
+}
+
+// The data kernel of a FIR half in its R, as a programmatic dependent of the plan kernel.
+template <int MODE>
+inline cudaError_t launch_bank_fir(const BankState &b, const FirCall &a, int block, size_t smem, bool capture_in_slot,
+                                   cudaStream_t st)
+{
+    const unsigned grid = unsigned(uint64_t(b.nstreams) * a.chunks);
+    if (block == 4)
+        return launch_dependent(bank_fir_kernel<4, MODE>, grid, 32, smem, st, b, a, capture_in_slot);
+    if (block == 2)
+        return launch_dependent(bank_fir_kernel<2, MODE>, grid, 32, smem, st, b, a, capture_in_slot);
+    return launch_dependent(bank_fir_kernel<1, MODE>, grid, 32, smem, st, b, a, capture_in_slot);
 }
 
 __global__ void bank_advance_kernel(BankState b, long long frames)

@@ -59,12 +59,16 @@ constexpr int kFirBlock = 4; // the largest R: consecutive outputs a lane keeps 
 // two ends only the outputs whose window holds frame q add, so no product of a tap with a frame
 // outside an output's own window is ever formed.  Lanes are R D' frames apart; a padding frame
 // after every R D' frames makes that stride odd, so the loads of a step are conflict-free.
-template <int R>
-__global__ void __launch_bounds__(32) fir_apply_kernel(const __grid_constant__ FirCall a)
+//
+// fir_tile is that walk for one CTA, with the block's frames and the outputs' destination left to
+// the kernel: in(row, i) gives input frame i < nin of the stream (row = the stream's row of a.in),
+// out(k, v) stores output k of the call.
+// fir_apply_kernel reads a.in and stores to a.out; the stream bank's FIR calls (sx_bank.cuh) take
+// the frames from the capture and store into the playback ring.
+template <int R, class In, class Out>
+__device__ __forceinline__ void fir_tile(const FirCall &a, uint32_t lane, uint64_t stream, uint64_t chunk, float2 *win,
+                                         const In &in, const Out &out)
 {
-    extern __shared__ __align__(16) float2 win[];
-    const uint32_t lane = threadIdx.x;
-    const uint64_t stream = blockIdx.x / a.chunks, chunk = blockIdx.x % a.chunks;
     const uint64_t a_first = a.a_lo + chunk * (32 * R);
     const uint32_t d1 = a.down1, hp = a.hp, seg = R * d1, pad = a.pad;
     const uint64_t buf_len = a.nin + hp - 1;
@@ -74,12 +78,12 @@ __global__ void __launch_bounds__(32) fir_apply_kernel(const __grid_constant__ F
     // frames come from the history, frames outside the buffer are never read by a stored output
     // and are staged as zeros.
     const float2 *hist = a.hist + stream * (hp - 1);
-    const float2 *in = a.in + stream * a.nin;
+    const float2 *row = a.in + stream * a.nin;
     for (uint32_t o = lane; o < a.win_len; o += 32) {
         const int64_t b = wb0 + int64_t(o);
         float2 v = make_float2(0.0f, 0.0f);
         if (b >= 0 && uint64_t(b) < buf_len)
-            v = uint64_t(b) < hp - 1 ? hist[b] : in[uint64_t(b) - (hp - 1)];
+            v = uint64_t(b) < hp - 1 ? hist[b] : in(row, uint64_t(b) - (hp - 1));
         win[o + (pad ? o / seg : 0)] = v;
     }
     __syncwarp();
@@ -132,9 +136,19 @@ __global__ void __launch_bounds__(32) fir_apply_kernel(const __grid_constant__ F
         for (int i = 0; i < R; i++) {
             const uint64_t kk = (a_first + R * lane + i) * a.up1 + c;
             if (kk >= a.c0 && kk - a.c0 < a.nout)
-                a.out[stream * a.nout + (kk - a.c0)] = make_float2(acc_re[i], acc_im[i]);
+                out(kk - a.c0, make_float2(acc_re[i], acc_im[i]));
         }
     }
+}
+
+template <int R>
+__global__ void __launch_bounds__(32) fir_apply_kernel(const __grid_constant__ FirCall a)
+{
+    extern __shared__ __align__(16) float2 win[];
+    const uint32_t lane = threadIdx.x;
+    const uint64_t stream = blockIdx.x / a.chunks, chunk = blockIdx.x % a.chunks;
+    fir_tile<R>(a, lane, stream, chunk, win, [](const float2 *row, uint64_t i) { return row[i]; },
+                [&](uint64_t k, float2 v) { a.out[stream * a.nout + k] = v; });
 }
 
 // The new history, hist = buf[nin .. nin + hp - 2], after fir_apply_kernel has read the old one

@@ -2515,6 +2515,43 @@ uint64_t fir_outputs(const sxgpu_fir *f, uint32_t r, uint64_t nin)
     return n > UINT64_MAX ? UINT64_MAX : uint64_t(n);
 }
 
+// The geometry of a call of nin frames that emits n = fir_outputs(f, f->phase, nin) frames, without
+// its buffers; `block` is the R of the data kernel (0 when n is 0) and `smem` its window in bytes.
+// False when the data kernel's grid would not fit.
+bool fir_call(const sxgpu_fir *f, uint64_t nin, uint64_t n, FirCall &a, int &block, size_t &smem)
+{
+    a.hist = f->hist;
+    a.taps = f->taps;
+    a.nin = nin;
+    a.nout = n;
+    a.c0 = (uint64_t(f->phase) * f->up + f->down - 1) / f->down;
+    a.a_lo = a.c0 / f->up1;
+    a.hp = f->hp;
+    a.rows = f->rows;
+    a.g = f->g;
+    a.up1 = f->up1;
+    a.down1 = f->down1;
+    a.phase = f->phase;
+    block = 0;
+    smem = 0;
+    if (n) {
+        const uint64_t classes = (a.c0 + n - 1) / f->up1 - a.a_lo + 1; // class indices a the call covers
+        const uint32_t e_max = (f->up1 - 1) * f->down1 / f->up1;
+        for (block = classes >= 128 ? 4 : classes >= 64 ? 2 : 1;; block /= 2) {
+            const uint32_t seg = uint32_t(block) * f->down1;
+            a.win_len = 32 * seg + e_max + f->hp;
+            a.pad = seg % 2 == 0;
+            smem = (a.win_len + (a.pad ? a.win_len / seg : 0)) * sizeof(float2);
+            if (smem <= kFirWindowBytes || block == 1)
+                break;
+        }
+        a.chunks = (classes + 32 * block - 1) / (32 * block);
+        if (a.chunks > uint64_t(INT32_MAX) / f->nstreams)
+            return false;
+    }
+    return true;
+}
+
 size_t fir_hist_bytes(const sxgpu_fir *f)
 {
     return size_t(f->nstreams) * (f->hp - 1) * sizeof(float2);
@@ -2576,6 +2613,12 @@ int sxgpu_fir_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t ntaps, const do
     SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<1, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<2, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<4, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<1, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<2, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<4, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     void *d_taps = nullptr, *d_hist = nullptr;
     cudaError_t e = cudaMalloc(&d_taps, taps.size() * sizeof(float));
     if (e == cudaSuccess)
@@ -2648,37 +2691,12 @@ int sxgpu_fir_apply(sxgpu_fir *f, const void *d_in, uint64_t nin, void *d_out, u
         return ctx->invalid("sxgpu_fir_apply: input and output overlap");
 
     FirCall a = {};
+    int block = 0;
+    size_t smem = 0;
+    if (!fir_call(f, nin, n, a, block, smem))
+        return ctx->invalid("sxgpu_fir_apply: the block needs more CTAs than a grid holds");
     a.in = static_cast<const float2 *>(d_in);
     a.out = static_cast<float2 *>(d_out);
-    a.hist = f->hist;
-    a.taps = f->taps;
-    a.nin = nin;
-    a.nout = n;
-    a.c0 = (uint64_t(f->phase) * f->up + f->down - 1) / f->down;
-    a.a_lo = a.c0 / f->up1;
-    a.hp = f->hp;
-    a.rows = f->rows;
-    a.g = f->g;
-    a.up1 = f->up1;
-    a.down1 = f->down1;
-    a.phase = f->phase;
-    int block = 0; // R of fir_apply_kernel
-    size_t smem = 0;
-    if (n) {
-        const uint64_t classes = (a.c0 + n - 1) / f->up1 - a.a_lo + 1; // class indices a the call covers
-        const uint32_t e_max = (f->up1 - 1) * f->down1 / f->up1;
-        for (block = classes >= 128 ? 4 : classes >= 64 ? 2 : 1;; block /= 2) {
-            const uint32_t seg = uint32_t(block) * f->down1;
-            a.win_len = 32 * seg + e_max + f->hp;
-            a.pad = seg % 2 == 0;
-            smem = (a.win_len + (a.pad ? a.win_len / seg : 0)) * sizeof(float2);
-            if (smem <= kFirWindowBytes || block == 1)
-                break;
-        }
-        a.chunks = (classes + 32 * block - 1) / (32 * block);
-        if (a.chunks > uint64_t(INT32_MAX) / nstreams)
-            return ctx->invalid("sxgpu_fir_apply: the block needs more CTAs than a grid holds");
-    }
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = fir_stream(f, stream);
     int launches = 0;
@@ -2702,6 +2720,94 @@ int sxgpu_fir_apply(sxgpu_fir *f, const void *d_in, uint64_t nin, void *d_out, u
     f->phase = uint32_t((f->phase + nin % f->down) % f->down);
     if (nout)
         *nout = n;
+    return SXGPU_OK;
+}
+
+// Why a FIR half's filter is refused (nullptr: it is not).
+static const char *bank_fir_invalid(const sxgpu_bank *bank, const sxgpu_fir *f)
+{
+    if (!f || f->ctx != bank->ctx)
+        return "the FIR filter is NULL or belongs to another context";
+    if (f->nstreams != bank->st.nstreams)
+        return "a filter must have as many streams as the bank";
+    return nullptr;
+}
+
+int sxgpu_bank_read_fir(sxgpu_bank *bank, sxgpu_fir *f, void *d_out, uint64_t *nout, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = bank->ctx;
+    if (const char *why = bank_fir_invalid(bank, f))
+        return ctx->invalid(why);
+    if (!d_out || reinterpret_cast<uintptr_t>(d_out) % 8)
+        return ctx->invalid("sxgpu_bank_read_fir: the output must be 8-byte aligned device memory");
+    const BankState &b = bank->st;
+    const uint64_t n = fir_outputs(f, f->phase, b.period);
+    if (n > UINT64_MAX / 8 / b.nstreams)
+        return ctx->invalid("sxgpu_bank_read_fir: nstreams * nout * 8 bytes overflows 64 bits");
+    FirCall a = {};
+    int block = 0;
+    size_t smem = 0;
+    if (!fir_call(f, b.period, n, a, block, smem))
+        return ctx->invalid("sxgpu_bank_read_fir: the period needs more CTAs than a grid holds");
+    a.out = static_cast<float2 *>(d_out);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = bank_stream(bank, stream);
+    const bool ext = bank->external_capture;
+    SX_CUDA(ctx, launch_bank_plan<kBankModeRead>(b, nullptr, 0, nullptr, 0, st));
+    int launches = 1;
+    if (n) {
+        SX_CUDA(ctx, launch_bank_fir<kBankModeRead>(b, a, block, smem, ext, st));
+        launches++;
+    }
+    if (f->hp > 1 || !ext) {
+        bank_fir_read_tail_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(b, a, ext);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
+    ctx->launches += launches;
+    ctx->frames_rx += uint64_t(b.nstreams) * b.period;
+    f->phase = uint32_t((f->phase + b.period % f->down) % f->down);
+    if (nout)
+        *nout = n;
+    return SXGPU_OK;
+}
+
+int sxgpu_bank_write_fir(sxgpu_bank *bank, sxgpu_fir *f, const void *d_in, uint64_t nin, int flags,
+                         const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = bank->ctx;
+    if (const char *why = bank_fir_invalid(bank, f))
+        return ctx->invalid(why);
+    if (!d_in || reinterpret_cast<uintptr_t>(d_in) % 8)
+        return ctx->invalid("sxgpu_bank_write_fir: the input must be 8-byte aligned device memory");
+    const BankState &b = bank->st;
+    if (nin > UINT64_MAX / 8 / b.nstreams)
+        return ctx->invalid("sxgpu_bank_write_fir: nstreams * nin * 8 bytes overflows 64 bits");
+    if (fir_outputs(f, f->phase, nin) != b.period)
+        return ctx->invalid("sxgpu_bank_write_fir: the filter must emit exactly one period from nin frames");
+    FirCall a = {};
+    int block = 0;
+    size_t smem = 0;
+    if (!fir_call(f, nin, b.period, a, block, smem))
+        return ctx->invalid("sxgpu_bank_write_fir: the block needs more CTAs than a grid holds");
+    a.in = static_cast<const float2 *>(d_in);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = bank_stream(bank, stream);
+    SX_CUDA(ctx, launch_bank_plan<kBankModeWrite>(b, nullptr, flags, d_time_ns, rx_time_offset_ns, st));
+    SX_CUDA(ctx, launch_bank_fir<kBankModeWrite>(b, a, block, smem, false, st));
+    int launches = 2;
+    if (f->hp > 1) {
+        fir_history_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(a);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
+    ctx->launches += launches;
+    ctx->frames_tx += uint64_t(b.nstreams) * b.period;
+    f->phase = uint32_t((f->phase + nin % f->down) % f->down);
     return SXGPU_OK;
 }
 
