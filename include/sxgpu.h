@@ -353,6 +353,66 @@ int sxgpu_bank_read_fir(sxgpu_bank *bank, sxgpu_fir *f, void *d_out, uint64_t *n
 int sxgpu_bank_write_fir(sxgpu_bank *bank, sxgpu_fir *f, const void *d_in, uint64_t nin, int flags,
                          const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream);
 
+/* ---- numerically controlled oscillators: per-stream frequency translation ------------------ */
+
+/* Selecting a channel that is not at DC of the front-end's band: mix it down to DC, then low-pass
+ * and decimate with real taps (a digital down-converter); a transmitter interpolates and then
+ * mixes up (a digital up-converter).  Per stream, a 32-bit phase phi_s and a 32-bit increment
+ * inc_s, both in device memory (so every call may be captured in a CUDA graph).  Frame k of a call
+ * is multiplied by e^{+j 2 pi phi / 2^32} with phi = phi_s + (k mod 2^32) inc_s (mod 2^32); a call
+ * of n frames then adds n inc_s to phi_s (mod 2^32).  To bring a channel at +f0 to DC, tune to -f0.
+ * A frequency f in cycles per sample (-0.5 <= f <= 0.5) becomes inc = rint(f 2^32) mod 2^32, round
+ * half to even: a resolution of fs / 2^32.
+ * The phasor, bit for bit (tests/sxnco.py restates it): u = ((phi + 2048) mod 2^32) >> 12,
+ * A = e^{j 2 pi (u >> 10) / 1024} and B = e^{j 2 pi (u & 1023) / 2^20}, each part libm's double cos or
+ * sin of 2.0 * pi * k / 1024.0 (/ 1048576.0) rounded once to float32; c = A.re B.re - A.im B.im,
+ * s = A.im B.re + A.re B.im; y.re = x.re c - x.im s, y.im = x.re s + x.im c; every product and sum
+ * one float32 rounding (no FMA).  The phasor is within 3.1e-6 of e^{j 2 pi phi / 2^32}. */
+typedef struct sxgpu_nco sxgpu_nco;
+/* freq: one frequency per stream (NULL: all 0).  The phases start at 0.  Refused: nstreams 0 or
+ * above 2^31 - 1, a frequency that is not finite or has |f| > 0.5.  sxgpu_destroy of the context
+ * refuses while an oscillator is alive. */
+int sxgpu_nco_create(sxgpu_ctx *ctx, uint32_t nstreams, const double *freq, sxgpu_nco **out);
+int sxgpu_nco_destroy(sxgpu_nco *n);
+/* d_cf32[nstreams][nframes], CF32, mixed in place; every phase advances by nframes inc_s.  Any
+ * nframes >= 1.  Only kernels are enqueued: nco_apply_kernel, then nco_advance_kernel (the new
+ * phases, after every read of the old ones), so 2 launches, counted in "launches".  Refused:
+ * nframes 0, a NULL or not 8-byte aligned buffer, byte sizes that overflow 64 bits, a grid of more
+ * than 2^31 - 1 CTAs. */
+int sxgpu_nco_apply(sxgpu_nco *n, void *d_cf32, uint64_t nframes, sxgpu_stream stream);
+/* Retunes every stream (h_freq on the host, NULL: all 0) and keeps the phases, so each stream's
+ * phase is continuous.  Refused as sxgpu_nco_create refuses a frequency.  Synchronises with
+ * `stream`. */
+int sxgpu_nco_set_frequencies(sxgpu_nco *n, const double *h_freq, sxgpu_stream stream);
+/* The phases and increments, [nstreams] each on the host.  get: either pointer may be NULL.  set:
+ * NULL leaves that array as it is.  Both synchronise with `stream`. */
+int sxgpu_nco_get_state(sxgpu_nco *n, uint32_t *h_phase, uint32_t *h_inc, sxgpu_stream stream);
+int sxgpu_nco_set_state(sxgpu_nco *n, const uint32_t *h_phase, const uint32_t *h_inc, sxgpu_stream stream);
+/* The FIR halves with the oscillator fused in: a bank of receivers that each select their own
+ * channel (read_ddc), a bank of transmitters that each place theirs (write_duc), without the
+ * full-rate CF32 block in memory.  Both need nco and f of this context with the bank's stream
+ * count, and refuse, with SXGPU_ERR_INVALID and nothing enqueued, what sxgpu_bank_read_fir /
+ * sxgpu_bank_write_fir refuse and a NULL or foreign oscillator or a stream-count mismatch.
+ * Only kernels are enqueued: the bank's plan kernel, then the data kernel (bank_nco_fir_kernel) as
+ * its programmatic dependent when the filter emits at least one frame (always, for the write),
+ * then the tail kernel (bank_nco_fir_read_tail_kernel / bank_nco_fir_write_tail_kernel: the
+ * filter's new history and, for a synthetic read, the capture slot; the phases advanced by the
+ * period), which always runs: so 3 launches per call at most (read: 2 when the call emits
+ * nothing; write: always 3), counted in "launches".  The oscillator never prevents graph capture;
+ * a call whose filter keeps its phase may be captured, as for sxgpu_bank_read_fir.
+ * read_ddc: sxgpu_bank_read(tmp), sxgpu_nco_apply(nco, tmp, period), then sxgpu_fir_apply(f, tmp,
+ * period, d_out, nout), bit for bit: positions, results, capture slots, the filter's history and
+ * phase, the oscillator's phases, d_out; for synthetic and ingested capture, through overruns (the
+ * oscillator counts delivered frames, a period per call), and when the call emits nothing. */
+int sxgpu_bank_read_ddc(sxgpu_bank *bank, sxgpu_nco *nco, sxgpu_fir *f, void *d_out, uint64_t *nout,
+                        sxgpu_stream stream);
+/* write_duc: sxgpu_fir_apply(f, d_in, nin, tmp), sxgpu_nco_apply(nco, tmp, period), then
+ * sxgpu_bank_write(bank, tmp, flags, d_time_ns, rx_time_offset_ns), bit for bit.  d_in is not
+ * modified.  The filter and the oscillator advance also when a stream's write is dropped as late.
+ * f must emit exactly one period from nin, as for sxgpu_bank_write_fir. */
+int sxgpu_bank_write_duc(sxgpu_bank *bank, sxgpu_fir *f, sxgpu_nco *nco, const void *d_in, uint64_t nin, int flags,
+                         const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream);
+
 /* ---- the hot path, host buffers ---------------------------------------------------------- */
 
 /* Same contracts as the two converters above, but src and dest are HOST memory, as they

@@ -31,7 +31,7 @@ NVCC_FLAGS = [
 ]
 
 GPU_SOURCES = [CSRC / "sxgpu.cu"]
-GPU_DEPS = GPU_SOURCES + [CSRC / "sx_kernels.cuh", CSRC / "sx_bank.cuh", CSRC / "sx_iir.cuh", CSRC / "sx_fir.cuh", CSRC / "sx_resident.cuh", CSRC / "sx_synth.h", CSRC / "sx_time.h",
+GPU_DEPS = GPU_SOURCES + [CSRC / "sx_kernels.cuh", CSRC / "sx_bank.cuh", CSRC / "sx_iir.cuh", CSRC / "sx_fir.cuh", CSRC / "sx_nco.cuh", CSRC / "sx_resident.cuh", CSRC / "sx_synth.h", CSRC / "sx_time.h",
                           CSRC / "host" / "stream_plan.hpp", CSRC / "host" / "par_copy.hpp", ROOT / "include" / "sxgpu.h"]
 
 SOAPY_SOURCES = [
@@ -103,7 +103,7 @@ def build_hook_example(force: bool = False) -> Path:
     """examples/repeater_hook.cu: user DSP compiled into the fused bank iteration (include/sx_hook.cuh)."""
     build_gpu_library()
     src = ROOT / "examples" / "repeater_hook.cu"
-    deps = [src, ROOT / "include" / "sx_hook.cuh", CSRC / "sx_bank.cuh", CSRC / "sx_iir.cuh", CSRC / "sx_kernels.cuh", GPU_LIB]
+    deps = [src, ROOT / "include" / "sx_hook.cuh", CSRC / "sx_bank.cuh", CSRC / "sx_iir.cuh", CSRC / "sx_fir.cuh", CSRC / "sx_nco.cuh", CSRC / "sx_kernels.cuh", GPU_LIB]
     if force or _stale(HOOK_EXAMPLE_LIB, deps):
         _run([_find_nvcc(), *NVCC_FLAGS, "-o", HOOK_EXAMPLE_LIB, src, "-L", LIB, "-lsxgpu",
               "-Xlinker", "-rpath,$ORIGIN"])

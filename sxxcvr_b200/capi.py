@@ -97,6 +97,14 @@ SIGNATURES = {
     "sxgpu_fir_set_state": (C.c_int, [_P, _P, C.c_uint32, _P]),
     "sxgpu_bank_read_fir": (C.c_int, [_P, _P, _P, C.POINTER(C.c_uint64), _P]),
     "sxgpu_bank_write_fir": (C.c_int, [_P, _P, _P, C.c_uint64, C.c_int, _P, C.c_longlong, _P]),
+    "sxgpu_nco_create": (C.c_int, [_P, C.c_uint32, _P, C.POINTER(_P)]),
+    "sxgpu_nco_destroy": (C.c_int, [_P]),
+    "sxgpu_nco_apply": (C.c_int, [_P, _P, C.c_uint64, _P]),
+    "sxgpu_nco_set_frequencies": (C.c_int, [_P, _P, _P]),
+    "sxgpu_nco_get_state": (C.c_int, [_P, _P, _P, _P]),
+    "sxgpu_nco_set_state": (C.c_int, [_P, _P, _P, _P]),
+    "sxgpu_bank_read_ddc": (C.c_int, [_P, _P, _P, _P, C.POINTER(C.c_uint64), _P]),
+    "sxgpu_bank_write_duc": (C.c_int, [_P, _P, _P, _P, C.c_uint64, C.c_int, _P, C.c_longlong, _P]),
     "sxgpu_convert_rx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S]),
     "sxgpu_convert_rx_buffer_host_gated": (C.c_int, [_P, _P, _S, _P, _S, _S, _P, _P]),
     "sxgpu_convert_tx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S, _F]),
@@ -376,6 +384,20 @@ class Bank:
         self.ctx.check(self.lib.sxgpu_bank_write_fir(self.handle, f.handle if f else None, d_in, nin, flags, d_time_ns,
                                                      rx_time_offset_ns, stream), "sxgpu_bank_write_fir")
 
+    def read_ddc(self, nco: "Nco", f: "Fir", d_out, stream=None) -> int:
+        """read(), nco.apply(that block, period), then f.apply(it, period, d_out) in one call, without
+        the full-rate block; returns nout, the frames per stream written to d_out."""
+        n = C.c_uint64()
+        self.ctx.check(self.lib.sxgpu_bank_read_ddc(self.handle, nco.handle if nco else None, f.handle if f else None,
+                                                    d_out, C.byref(n), stream), "sxgpu_bank_read_ddc")
+        return n.value
+
+    def write_duc(self, f: "Fir", nco: "Nco", d_in, nin, flags=4, d_time_ns=None, rx_time_offset_ns=0, stream=None):
+        """write() of nco.apply(f.apply(d_in, nin), period), in one call that leaves d_in as it was."""
+        self.ctx.check(self.lib.sxgpu_bank_write_duc(self.handle, f.handle if f else None, nco.handle if nco else None,
+                                                     d_in, nin, flags, d_time_ns, rx_time_offset_ns, stream),
+                       "sxgpu_bank_write_duc")
+
     def repeat_begin(self, d_cf32, stream=None):
         self.ctx.check(self.lib.sxgpu_bank_repeat_begin(self.handle, d_cf32, stream), "sxgpu_bank_repeat_begin")
 
@@ -534,6 +556,70 @@ class Fir:
                 raise ValueError(f"hist must have shape {(self.nstreams, self.hp - 1)}, got {hist.shape}")
             ptr = hist.ctypes.data
         self.ctx.check(self.lib.sxgpu_fir_set_state(self.handle, ptr, phase, stream), "sxgpu_fir_set_state")
+
+
+class Nco:
+    """One numerically controlled oscillator per stream (sxgpu_nco_* in include/sxgpu.h): each
+    frame multiplied by exp(+2j pi phase / 2^32), the 32-bit phase advancing by the increment
+    rint(f 2^32) per frame, carried from call to call.  `freqs` in cycles per sample, -0.5 .. 0.5
+    (None: all 0); to bring a channel at +f0 to DC, use -f0."""
+
+    def __init__(self, ctx: Context, nstreams: int, freqs=None):
+        import numpy as np
+        self.np = np
+        self.ctx, self.lib = ctx, ctx.lib
+        self.handle = None
+        f = self._freqs(nstreams, freqs)
+        h = _P()
+        ctx.check(self.lib.sxgpu_nco_create(ctx.handle, nstreams, f.ctypes.data if f is not None else None, C.byref(h)),
+                  "sxgpu_nco_create")
+        self.handle, self.nstreams = h, nstreams
+
+    def _freqs(self, nstreams, freqs):
+        if freqs is None:
+            return None
+        return self.np.ascontiguousarray(self.np.broadcast_to(self.np.asarray(freqs, dtype=self.np.float64), (nstreams,)))
+
+    def close(self):
+        if self.handle:
+            self.lib.sxgpu_nco_destroy(self.handle)
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def apply(self, d_cf32, nframes, stream=None):
+        """Mix d_cf32[nstreams][nframes] (complex64 on the device) in place."""
+        self.ctx.check(self.lib.sxgpu_nco_apply(self.handle, d_cf32, nframes, stream), "sxgpu_nco_apply")
+
+    def set_frequencies(self, freqs, stream=None):
+        """Retune every stream (one frequency, or one per stream; None: all 0), the phases kept."""
+        f = self._freqs(self.nstreams, freqs)
+        self.ctx.check(self.lib.sxgpu_nco_set_frequencies(self.handle, f.ctypes.data if f is not None else None, stream),
+                       "sxgpu_nco_set_frequencies")
+
+    def state(self, stream=None):
+        """(phases, increments), each (nstreams,) uint32."""
+        ph, inc = self.np.empty(self.nstreams, self.np.uint32), self.np.empty(self.nstreams, self.np.uint32)
+        self.ctx.check(self.lib.sxgpu_nco_get_state(self.handle, ph.ctypes.data, inc.ctypes.data, stream),
+                       "sxgpu_nco_get_state")
+        return ph, inc
+
+    def set_state(self, phases=None, incs=None, stream=None):
+        """Set the phases and/or the increments, (nstreams,) uint32 each; None leaves that one as it is."""
+        ptrs = []
+        for a in (phases, incs):
+            if a is None:
+                ptrs.append((None, None))
+                continue
+            a = self.np.ascontiguousarray(a, dtype=self.np.uint32)
+            if a.shape != (self.nstreams,):
+                raise ValueError(f"phases and incs must have shape {(self.nstreams,)}, got {a.shape}")
+            ptrs.append((a, a.ctypes.data))
+        self.ctx.check(self.lib.sxgpu_nco_set_state(self.handle, ptrs[0][1], ptrs[1][1], stream), "sxgpu_nco_set_state")
 
 
 class Multi:

@@ -42,6 +42,9 @@
 //                             tiles with the frames taken from the capture or stored into the
 //                             ring, as a programmatic dependent of the plan kernel, then
 //                             bank_fir_read_tail_kernel / fir_history_kernel
+// and the same with an oscillator mixing the full-rate frames (digital down- and up-conversion):
+//     bank_plan_{read,write}_kernel, then bank_nco_fir_kernel<R, MODE>, then
+//                             bank_nco_fir_{read,write}_tail_kernel, which also advance the phases
 // The virtual clock follows the same rule as the host-side ALSA stand-in: it moves when a
 // blocking transfer must wait (by exactly the deficit) or when the owner advances it.
 #pragma once
@@ -50,6 +53,7 @@
 #include "sx_fir.cuh"
 #include "sx_iir.cuh"
 #include "sx_kernels.cuh"
+#include "sx_nco.cuh"
 #include "sx_time.h"
 
 namespace sx {
@@ -1074,6 +1078,94 @@ __global__ void __launch_bounds__(kFirHistoryThreads) bank_fir_read_tail_kernel(
         hist[i] = keep[i];
 }
 
+// ---------------------------------------------------------------------------------------
+// The FIR halves with an oscillator (sxgpu_bank_read_ddc, sxgpu_bank_write_duc): the kernels above
+// with the full-rate frames mixed (sx_nco.cuh), so that the same state, results, capture, ring,
+// filter history, phases and outputs come out as from the plain half, sxgpu_nco_apply and
+// sxgpu_fir_apply one after the other.
+//   read:  input frame i of the filter is capture frame i of the period through RxCf32, mixed with
+//          phi_s + i inc_s; bank_nco_fir_read_tail_kernel mixes the history's new frames the same
+//          way, writes the capture slot as bank_fir_read_tail_kernel does, and advances phi_s.
+//   write: output k of the filter is mixed with phi_s + k inc_s before TxCf32 and the ring;
+//          bank_nco_fir_write_tail_kernel writes the filter's history as fir_history_kernel does
+//          and advances phi_s, also for a stream whose write was dropped as late.
+// Every read of phi_s is in the data kernel or before the tail kernel's barrier, and the phase
+// advances after it.
+// ---------------------------------------------------------------------------------------
+template <int R, int MODE>
+__global__ void __launch_bounds__(32) bank_nco_fir_kernel(BankState b, const __grid_constant__ FirCall a, bool capture_in_slot,
+                                                          NcoView nco)
+{
+    extern __shared__ __align__(16) float2 win[];
+    const uint64_t stream = blockIdx.x / a.chunks, chunk = blockIdx.x % a.chunks;
+    pdl_wait(); // the decisions, and everything before them on the stream, are in memory
+    const NcoStream mix = nco_stream(nco, stream);
+    if constexpr (MODE == kBankModeRead) {
+        auto out = [&](uint64_t k, float2 v) { a.out[stream * a.nout + k] = v; };
+        if (capture_in_slot) {
+            const char *slot = b.capture_stage + stream * b.period * 8;
+            fir_tile<R>(a, threadIdx.x, stream, chunk, win, [&](const float2 *, uint64_t i) { return mix(i, rx_frame(ld_stream<8>(slot + i * 8))); }, out);
+        } else {
+            const uint64_t seed = b.seed + stream, first = uint64_t(b.rx_first_frame[stream]);
+            fir_tile<R>(a, threadIdx.x, stream, chunk, win, [&](const float2 *, uint64_t i) { return mix(i, rx_frame(capture_frame(seed, first + i))); }, out);
+        }
+    } else {
+        const long long off = b.tx_ring_offset[stream];
+        if (off < 0)
+            return; // dropped as late: nothing is stored (the history and the phase still advance, in the tail kernel)
+        const long long at = b.tx_write_position[stream];
+        fir_tile<R>(a, threadIdx.x, stream, chunk, win, [](const float2 *row, uint64_t i) { return row[i]; }, [&](uint64_t k, float2 v) {
+            const float2 m = mix(k, v);
+            Pack<2> f, w;
+            f.w[0] = __float_as_uint(m.x), f.w[1] = __float_as_uint(m.y);
+            TxCf32::apply<1>(f, w, b.thr2);
+            st_stream<8>((off & 1) == 0 ? b.playback_ring + off + k * 8 : ring_frame(b, stream, uint64_t(at) + k), w);
+        });
+    }
+}
+
+__global__ void __launch_bounds__(kFirHistoryThreads) bank_nco_fir_read_tail_kernel(BankState b, const __grid_constant__ FirCall a,
+                                                                                    bool capture_in_slot, NcoView nco)
+{
+    extern __shared__ __align__(16) float2 keep[]; // [hp - 1]
+    const uint32_t n = a.hp - 1;
+    const uint64_t s = blockIdx.x;
+    char *slot = b.capture_stage + s * b.period * 8;
+    const uint64_t seed = b.seed + s, first = capture_in_slot ? 0 : uint64_t(b.rx_first_frame[s]);
+    float2 *hist = a.hist + s * n;
+    const NcoStream mix = nco_stream(nco, s);
+    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads) {
+        const uint64_t k = a.nin + i; // buffer frame
+        keep[i] = k < n ? hist[k] : mix(k - n, rx_frame(capture_in_slot ? ld_stream<8>(slot + (k - n) * 8) : capture_frame(seed, first + k - n)));
+    }
+    for (uint32_t i = threadIdx.x; i < b.period && !capture_in_slot; i += kFirHistoryThreads)
+        st_stream<8>(slot + size_t(i) * 8, capture_frame(seed, first + i));
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads)
+        hist[i] = keep[i];
+    if (threadIdx.x == 0)
+        nco_advance(nco, s, b.period);
+}
+
+__global__ void __launch_bounds__(kFirHistoryThreads) bank_nco_fir_write_tail_kernel(const __grid_constant__ FirCall a, NcoView nco,
+                                                                                     uint32_t period)
+{
+    extern __shared__ __align__(16) float2 keep[]; // [hp - 1]
+    const uint32_t n = a.hp - 1;
+    const uint64_t s = blockIdx.x;
+    float2 *hist = a.hist + s * n;
+    const float2 *in = a.in + s * a.nin;
+    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads) {
+        const uint64_t k = a.nin + i; // buffer frame
+        keep[i] = k < n ? hist[k] : in[k - n];
+    }
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads)
+        hist[i] = keep[i];
+    if (threadIdx.x == 0)
+        nco_advance(nco, s, period);
+}
+
 // The data kernel of a FIR half in its R, as a programmatic dependent of the plan kernel.
 template <int MODE>
 inline cudaError_t launch_bank_fir(const BankState &b, const FirCall &a, int block, size_t smem, bool capture_in_slot,
@@ -1085,6 +1177,19 @@ inline cudaError_t launch_bank_fir(const BankState &b, const FirCall &a, int blo
     if (block == 2)
         return launch_dependent(bank_fir_kernel<2, MODE>, grid, 32, smem, st, b, a, capture_in_slot);
     return launch_dependent(bank_fir_kernel<1, MODE>, grid, 32, smem, st, b, a, capture_in_slot);
+}
+
+// The same with the oscillator.
+template <int MODE>
+inline cudaError_t launch_bank_nco_fir(const BankState &b, const FirCall &a, int block, size_t smem, bool capture_in_slot,
+                                       const NcoView &nco, cudaStream_t st)
+{
+    const unsigned grid = unsigned(uint64_t(b.nstreams) * a.chunks);
+    if (block == 4)
+        return launch_dependent(bank_nco_fir_kernel<4, MODE>, grid, 32, smem, st, b, a, capture_in_slot, nco);
+    if (block == 2)
+        return launch_dependent(bank_nco_fir_kernel<2, MODE>, grid, 32, smem, st, b, a, capture_in_slot, nco);
+    return launch_dependent(bank_nco_fir_kernel<1, MODE>, grid, 32, smem, st, b, a, capture_in_slot, nco);
 }
 
 __global__ void bank_advance_kernel(BankState b, long long frames)

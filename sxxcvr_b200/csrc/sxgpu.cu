@@ -10,6 +10,7 @@
 #include "sx_bank.cuh"
 #include "sx_iir.cuh"
 #include "sx_fir.cuh"
+#include "sx_nco.cuh"
 #include "sx_resident.cuh"
 #include "host/par_copy.hpp"
 #include "host/worker_pool.hpp"
@@ -128,6 +129,7 @@ struct sxgpu_ctx {
     std::atomic<int> live_banks{0}; // banks keep a pointer to their context
     std::atomic<int> live_iirs{0};  // so do filters
     std::atomic<int> live_firs{0};
+    std::atomic<int> live_ncos{0};
     bool l2_carveout_set = false;   // sxgpu_bank_repeat_begin sets the persisting-L2 limit once
 
     // host pipeline: lane 0 serves the RX conversions, lane 1 the TX conversions
@@ -1466,6 +1468,8 @@ int sxgpu_destroy(sxgpu_ctx *ctx)
         return ctx->invalid("destroy the context's stream banks first");
     if (ctx->live_iirs.load() != 0 || ctx->live_firs.load() != 0)
         return ctx->invalid("destroy the context's filters first");
+    if (ctx->live_ncos.load() != 0)
+        return ctx->invalid("destroy the context's oscillators first");
     cudaSetDevice(ctx->device);
     for (HostLane &lane : ctx->lanes) {
         std::lock_guard<std::mutex> lock(lane.mutex);
@@ -2844,6 +2848,265 @@ int sxgpu_fir_set_state(sxgpu_fir *f, const void *h_hist, uint32_t phase, sxgpu_
         SX_CUDA(ctx, cudaStreamSynchronize(st));
     }
     f->phase = phase;
+    return SXGPU_OK;
+}
+
+// ---- numerically controlled oscillators (sx_nco.cuh) ---------------------------------------------
+} // extern "C"
+
+struct sxgpu_nco {
+    sxgpu_ctx *ctx = nullptr;
+    uint32_t nstreams = 0;
+    void *mem = nullptr; // one allocation: the tables, then the phases, then the increments
+    NcoView view = {};
+};
+
+namespace {
+
+// inc = rint(f 2^32) mod 2^32 for every stream (f NULL: all 0), or why a frequency is refused.
+const char *nco_increments(uint32_t nstreams, const double *freq, std::vector<uint32_t> &inc)
+{
+    inc.assign(nstreams, 0);
+    for (uint32_t s = 0; freq && s < nstreams; s++) {
+        if (!std::isfinite(freq[s]) || std::fabs(freq[s]) > 0.5)
+            return "an oscillator's frequency is finite and within -0.5 .. 0.5 cycles per sample";
+        inc[s] = uint32_t(uint64_t(std::llrint(freq[s] * 4294967296.0)));
+    }
+    return nullptr;
+}
+
+cudaStream_t nco_stream(sxgpu_nco *n, sxgpu_stream stream)
+{
+    return stream ? static_cast<cudaStream_t>(stream) : n->ctx->stream;
+}
+
+} // namespace
+
+extern "C" {
+
+int sxgpu_nco_create(sxgpu_ctx *ctx, uint32_t nstreams, const double *freq, sxgpu_nco **out)
+{
+    if (!ctx || !out)
+        return SXGPU_ERR_INVALID;
+    *out = nullptr;
+    if (nstreams == 0 || nstreams > uint32_t(INT32_MAX))
+        return ctx->invalid("an oscillator has 1 to 2^31 - 1 streams");
+    std::vector<uint32_t> inc;
+    if (const char *why = nco_increments(nstreams, freq, inc))
+        return ctx->invalid(why);
+    // A[k] = e^{j 2 pi k / 1024}, B[k] = e^{j 2 pi k / 2^20}: libm's double cos and sin, rounded once.
+    std::vector<float2> tab(2 * kNcoTableSize);
+    for (int k = 0; k < kNcoTableSize; k++) {
+        const double a = 2.0 * M_PI * k / 1024.0, b = 2.0 * M_PI * k / 1048576.0;
+        tab[k] = make_float2(float(std::cos(a)), float(std::sin(a)));
+        tab[kNcoTableSize + k] = make_float2(float(std::cos(b)), float(std::sin(b)));
+    }
+    const size_t tab_bytes = tab.size() * sizeof(float2), state_bytes = size_t(nstreams) * sizeof(uint32_t);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const size_t smem = std::min<size_t>(kFirWindowBytes, ctx->prop.sharedMemPerBlockOptin);
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<1, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<2, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<4, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<1, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<2, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<4, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    std::unique_ptr<sxgpu_nco> n(new sxgpu_nco());
+    n->ctx = ctx;
+    n->nstreams = nstreams;
+    cudaError_t e = cudaMalloc(&n->mem, tab_bytes + 2 * state_bytes);
+    if (e != cudaSuccess)
+        return ctx->fail(e, "cudaMalloc(oscillator)");
+    char *mem = static_cast<char *>(n->mem);
+    n->view.tab = reinterpret_cast<const float2 *>(mem);
+    n->view.phase = reinterpret_cast<uint32_t *>(mem + tab_bytes);
+    n->view.inc = reinterpret_cast<uint32_t *>(mem + tab_bytes + state_bytes);
+    e = cudaMemcpy(mem, tab.data(), tab_bytes, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess)
+        e = cudaMemcpy(n->view.inc, inc.data(), state_bytes, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess)
+        e = cudaMemsetAsync(n->view.phase, 0, state_bytes, ctx->stream);
+    if (e == cudaSuccess)
+        e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) {
+        cudaFree(n->mem);
+        return ctx->fail(e, "cudaMemcpy(oscillator)");
+    }
+    ctx->live_ncos++;
+    *out = n.release();
+    return SXGPU_OK;
+}
+
+int sxgpu_nco_destroy(sxgpu_nco *n)
+{
+    if (!n)
+        return SXGPU_ERR_INVALID;
+    cudaSetDevice(n->ctx->device);
+    for (HostLane &lane : n->ctx->lanes) { // a resident converter would hold the device-wide sync up
+        std::lock_guard<std::mutex> lock(lane.mutex);
+        resident_stop(n->ctx, lane);
+    }
+    cudaDeviceSynchronize();
+    cudaFree(n->mem);
+    n->ctx->live_ncos--;
+    delete n;
+    return SXGPU_OK;
+}
+
+int sxgpu_nco_apply(sxgpu_nco *n, void *d_cf32, uint64_t nframes, sxgpu_stream stream)
+{
+    if (!n)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = n->ctx;
+    if (!d_cf32 || reinterpret_cast<uintptr_t>(d_cf32) % 8)
+        return ctx->invalid("sxgpu_nco_apply: the block must be 8-byte aligned device memory");
+    if (nframes == 0)
+        return ctx->invalid("sxgpu_nco_apply: a block has at least one frame");
+    if (nframes > UINT64_MAX / 8 / n->nstreams)
+        return ctx->invalid("sxgpu_nco_apply: nstreams * nframes * 8 bytes overflows 64 bits");
+    const uint64_t total = uint64_t(n->nstreams) * nframes, ctas = (total + kNcoTile - 1) / kNcoTile;
+    if (ctas > uint64_t(INT32_MAX))
+        return ctx->invalid("sxgpu_nco_apply: the block needs more CTAs than a grid holds");
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = nco_stream(n, stream);
+    nco_apply_kernel<<<unsigned(ctas), kNcoThreads, 0, st>>>(n->view, static_cast<float2 *>(d_cf32), nframes, total,
+                                                             1.0 / double(nframes));
+    SX_CUDA(ctx, cudaGetLastError());
+    nco_advance_kernel<<<per_stream_grid(n->nstreams, 256), 256, 0, st>>>(n->view, n->nstreams, uint32_t(nframes));
+    SX_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 2;
+    return SXGPU_OK;
+}
+
+int sxgpu_nco_set_frequencies(sxgpu_nco *n, const double *h_freq, sxgpu_stream stream)
+{
+    if (!n)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = n->ctx;
+    std::vector<uint32_t> inc;
+    if (const char *why = nco_increments(n->nstreams, h_freq, inc))
+        return ctx->invalid(why);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = nco_stream(n, stream);
+    SX_CUDA(ctx, cudaMemcpyAsync(n->view.inc, inc.data(), inc.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    SX_CUDA(ctx, cudaStreamSynchronize(st));
+    return SXGPU_OK;
+}
+
+int sxgpu_nco_get_state(sxgpu_nco *n, uint32_t *h_phase, uint32_t *h_inc, sxgpu_stream stream)
+{
+    if (!n)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = n->ctx;
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = nco_stream(n, stream);
+    const size_t bytes = size_t(n->nstreams) * sizeof(uint32_t);
+    if (h_phase)
+        SX_CUDA(ctx, cudaMemcpyAsync(h_phase, n->view.phase, bytes, cudaMemcpyDeviceToHost, st));
+    if (h_inc)
+        SX_CUDA(ctx, cudaMemcpyAsync(h_inc, n->view.inc, bytes, cudaMemcpyDeviceToHost, st));
+    SX_CUDA(ctx, cudaStreamSynchronize(st));
+    return SXGPU_OK;
+}
+
+int sxgpu_nco_set_state(sxgpu_nco *n, const uint32_t *h_phase, const uint32_t *h_inc, sxgpu_stream stream)
+{
+    if (!n)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = n->ctx;
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = nco_stream(n, stream);
+    const size_t bytes = size_t(n->nstreams) * sizeof(uint32_t);
+    if (h_phase)
+        SX_CUDA(ctx, cudaMemcpyAsync(n->view.phase, h_phase, bytes, cudaMemcpyHostToDevice, st));
+    if (h_inc)
+        SX_CUDA(ctx, cudaMemcpyAsync(n->view.inc, h_inc, bytes, cudaMemcpyHostToDevice, st));
+    SX_CUDA(ctx, cudaStreamSynchronize(st));
+    return SXGPU_OK;
+}
+
+// Why a half's oscillator is refused (nullptr: it is not).
+static const char *bank_nco_invalid(const sxgpu_bank *bank, const sxgpu_nco *n)
+{
+    if (!n || n->ctx != bank->ctx)
+        return "the oscillator is NULL or belongs to another context";
+    if (n->nstreams != bank->st.nstreams)
+        return "an oscillator must have as many streams as the bank";
+    return nullptr;
+}
+
+int sxgpu_bank_read_ddc(sxgpu_bank *bank, sxgpu_nco *nco, sxgpu_fir *f, void *d_out, uint64_t *nout, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = bank->ctx;
+    if (const char *why = bank_nco_invalid(bank, nco))
+        return ctx->invalid(why);
+    if (const char *why = bank_fir_invalid(bank, f))
+        return ctx->invalid(why);
+    if (!d_out || reinterpret_cast<uintptr_t>(d_out) % 8)
+        return ctx->invalid("sxgpu_bank_read_ddc: the output must be 8-byte aligned device memory");
+    const BankState &b = bank->st;
+    const uint64_t n = fir_outputs(f, f->phase, b.period);
+    if (n > UINT64_MAX / 8 / b.nstreams)
+        return ctx->invalid("sxgpu_bank_read_ddc: nstreams * nout * 8 bytes overflows 64 bits");
+    FirCall a = {};
+    int block = 0;
+    size_t smem = 0;
+    if (!fir_call(f, b.period, n, a, block, smem))
+        return ctx->invalid("sxgpu_bank_read_ddc: the period needs more CTAs than a grid holds");
+    a.out = static_cast<float2 *>(d_out);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = bank_stream(bank, stream);
+    const bool ext = bank->external_capture;
+    SX_CUDA(ctx, launch_bank_plan<kBankModeRead>(b, nullptr, 0, nullptr, 0, st));
+    int launches = 1;
+    if (n) {
+        SX_CUDA(ctx, launch_bank_nco_fir<kBankModeRead>(b, a, block, smem, ext, nco->view, st));
+        launches++;
+    }
+    bank_nco_fir_read_tail_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(b, a, ext, nco->view);
+    SX_CUDA(ctx, cudaGetLastError());
+    launches++;
+    ctx->launches += launches;
+    ctx->frames_rx += uint64_t(b.nstreams) * b.period;
+    f->phase = uint32_t((f->phase + b.period % f->down) % f->down);
+    if (nout)
+        *nout = n;
+    return SXGPU_OK;
+}
+
+int sxgpu_bank_write_duc(sxgpu_bank *bank, sxgpu_fir *f, sxgpu_nco *nco, const void *d_in, uint64_t nin, int flags,
+                         const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = bank->ctx;
+    if (const char *why = bank_fir_invalid(bank, f))
+        return ctx->invalid(why);
+    if (const char *why = bank_nco_invalid(bank, nco))
+        return ctx->invalid(why);
+    if (!d_in || reinterpret_cast<uintptr_t>(d_in) % 8)
+        return ctx->invalid("sxgpu_bank_write_duc: the input must be 8-byte aligned device memory");
+    const BankState &b = bank->st;
+    if (nin > UINT64_MAX / 8 / b.nstreams)
+        return ctx->invalid("sxgpu_bank_write_duc: nstreams * nin * 8 bytes overflows 64 bits");
+    if (fir_outputs(f, f->phase, nin) != b.period)
+        return ctx->invalid("sxgpu_bank_write_duc: the filter must emit exactly one period from nin frames");
+    FirCall a = {};
+    int block = 0;
+    size_t smem = 0;
+    if (!fir_call(f, nin, b.period, a, block, smem))
+        return ctx->invalid("sxgpu_bank_write_duc: the block needs more CTAs than a grid holds");
+    a.in = static_cast<const float2 *>(d_in);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = bank_stream(bank, stream);
+    SX_CUDA(ctx, launch_bank_plan<kBankModeWrite>(b, nullptr, flags, d_time_ns, rx_time_offset_ns, st));
+    SX_CUDA(ctx, launch_bank_nco_fir<kBankModeWrite>(b, a, block, smem, false, nco->view, st));
+    bank_nco_fir_write_tail_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(a, nco->view, b.period);
+    SX_CUDA(ctx, cudaGetLastError());
+    ctx->launches += 3;
+    ctx->frames_tx += uint64_t(b.nstreams) * b.period;
+    f->phase = uint32_t((f->phase + nin % f->down) % f->down);
     return SXGPU_OK;
 }
 
