@@ -413,6 +413,63 @@ int sxgpu_bank_read_ddc(sxgpu_bank *bank, sxgpu_nco *nco, sxgpu_fir *f, void *d_
 int sxgpu_bank_write_duc(sxgpu_bank *bank, sxgpu_fir *f, sxgpu_nco *nco, const void *d_in, uint64_t nin, int flags,
                          const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream);
 
+/* ---- polyphase DFT channelizers: every channel of a stream at once ------------------------- */
+
+/* A receiver that monitors every channel of its band: each stream split into M channel-rate
+ * streams with one prototype low-pass, in one pass, instead of M copies each mixed and decimated.
+ * M = channels, a power of two from 2 to SXGPU_CHAN_MAX_CHANNELS; D = down divides M (D = M is
+ * critically sampled, D = M/2 oversampled by 2).  Channel k is centred at k / M cycles per input
+ * sample (k >= M/2: the negative frequency (k - M) / M, numpy's fft order); its rate is fs / D.
+ * X counts the frames a stream has been fed since creation or set_state; frames before the first
+ * are 0.  Output m of channel k, m = 0 .. ceil(X / D) - 1, is
+ *     y_k[m] = sum_{j < ntaps} h[j] x[m D - j] e^{-j 2 pi k (m D - j) / M},
+ * i.e. sxgpu_nco_apply at -k / M (phase counted from frame 0), then sxgpu_fir_apply(h, up 1, down D),
+ * up to rounding.  Bit for bit (tests/sxchan.py restates it), with N = m D, h rounded to float32
+ * once, I and Q separately and every product and sum one float32 rounding (no FMA):
+ *   1. branch sums, r < M, P_r = ceil((ntaps - r) / M) (0 when r >= ntaps):
+ *        u_r = +0;  for p = P_r - 1 down to 0:  u_r = u_r + x[N - p M - r] * h[p M + r];
+ *   2. a[i] = u_{(N - rev(i)) mod M}, rev reversing the log2 M bits of i;
+ *   3. radix-2 decimation-in-time stages h = 1, 2, .. M/2: for every i with (i mod 2h) < h,
+ *        w = T[(i mod 2h) M / (2h)], p = a[i], q = a[i+h],
+ *        t.re = q.re w.re - q.im w.im, t.im = q.re w.im + q.im w.re, a[i] = p + t, a[i+h] = p - t,
+ *      every butterfly multiplied by its twiddle, T[0] included; T[j] = (A.re, -A.im) of the
+ *      oscillators' coarse table entry A[j 1024 / M] (libm's double cos / sin of
+ *      2.0 * pi * q / 1024.0, rounded once);
+ *   4. y_k[m] = a[k]. */
+#define SXGPU_CHAN_MAX_CHANNELS 1024
+#define SXGPU_CHAN_MAX_TAPS 16384 /* and ntaps <= 32 * channels */
+typedef struct sxgpu_chan sxgpu_chan;
+/* h: ntaps real taps as double, rounded to float32 once, here.  Refused: nstreams 0 or
+ * nstreams * channels above 2^31 - 1 (so the output is always a valid block of that many streams
+ * for the other calls), channels not a power of two in 2 .. SXGPU_CHAN_MAX_CHANNELS, down 0 or not
+ * dividing channels, ntaps 0 or above 32 * channels or SXGPU_CHAN_MAX_TAPS, a NULL h, a tap that
+ * is not finite.  The history starts at zero and the phase at 0.  sxgpu_destroy of the context
+ * refuses while a channelizer is alive. */
+int sxgpu_chan_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t channels, uint32_t down, uint32_t ntaps,
+                      const double *h, sxgpu_chan **out);
+int sxgpu_chan_destroy(sxgpu_chan *c);
+/* The frames each channel's next apply of nin frames emits: ceil((X + nin) / D) - ceil(X / D).
+ * Host arithmetic, no GPU work. */
+int sxgpu_chan_output_frames(sxgpu_chan *c, uint64_t nin, uint64_t *nout);
+/* d_in[nstreams][nin] -> d_out[nstreams][channels][*nout], CF32: nstreams * channels rows of nout
+ * frames, the block sxgpu_fir_apply, sxgpu_nco_apply and sxgpu_iir_apply take with
+ * nstreams * channels streams.  The history and the phase are carried; *nout (may be NULL) is
+ * written on return.  The phase, X mod channels, lives on the host and is all the call depends on
+ * besides the buffers, so a call with nin a multiple of channels (which leaves the phase as it was)
+ * may be captured in a CUDA graph and replayed; other calls must not be.  Only kernels are
+ * enqueued: chan_apply_kernel when the call emits at least one frame, then fir_history_kernel when
+ * ntaps > 1 (the new history, written after every read of the old one), so 2 launches per call at
+ * most, counted in "launches".  Refused: nin 0, a NULL or not 8-byte aligned buffer, byte sizes
+ * that overflow 64 bits, d_in and d_out overlapping, a grid of more than 2^31 - 1 CTAs. */
+int sxgpu_chan_apply(sxgpu_chan *c, const void *d_in, uint64_t nin, void *d_out, uint64_t *nout,
+                     sxgpu_stream stream);
+/* The history, [nstreams][ntaps - 1] complex64 on the host, the last inputs of each stream oldest
+ * first (nothing when ntaps = 1), and the phase X mod channels.  get: either pointer may be NULL.
+ * set: NULL h_hist = zeros; a phase of channels or more is refused.  Both synchronise with
+ * `stream`. */
+int sxgpu_chan_get_state(sxgpu_chan *c, void *h_hist, uint32_t *phase, sxgpu_stream stream);
+int sxgpu_chan_set_state(sxgpu_chan *c, const void *h_hist, uint32_t phase, sxgpu_stream stream);
+
 /* ---- the hot path, host buffers ---------------------------------------------------------- */
 
 /* Same contracts as the two converters above, but src and dest are HOST memory, as they

@@ -31,7 +31,7 @@ NVCC_FLAGS = [
 ]
 
 GPU_SOURCES = [CSRC / "sxgpu.cu"]
-GPU_DEPS = GPU_SOURCES + [CSRC / "sx_kernels.cuh", CSRC / "sx_bank.cuh", CSRC / "sx_iir.cuh", CSRC / "sx_fir.cuh", CSRC / "sx_nco.cuh", CSRC / "sx_resident.cuh", CSRC / "sx_synth.h", CSRC / "sx_time.h",
+GPU_DEPS = GPU_SOURCES + [CSRC / "sx_kernels.cuh", CSRC / "sx_bank.cuh", CSRC / "sx_iir.cuh", CSRC / "sx_fir.cuh", CSRC / "sx_nco.cuh", CSRC / "sx_chan.cuh", CSRC / "sx_resident.cuh", CSRC / "sx_synth.h", CSRC / "sx_time.h",
                           CSRC / "host" / "stream_plan.hpp", CSRC / "host" / "par_copy.hpp", ROOT / "include" / "sxgpu.h"]
 
 SOAPY_SOURCES = [

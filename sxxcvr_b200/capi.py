@@ -105,6 +105,12 @@ SIGNATURES = {
     "sxgpu_nco_set_state": (C.c_int, [_P, _P, _P, _P]),
     "sxgpu_bank_read_ddc": (C.c_int, [_P, _P, _P, _P, C.POINTER(C.c_uint64), _P]),
     "sxgpu_bank_write_duc": (C.c_int, [_P, _P, _P, _P, C.c_uint64, C.c_int, _P, C.c_longlong, _P]),
+    "sxgpu_chan_create": (C.c_int, [_P, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, _P, C.POINTER(_P)]),
+    "sxgpu_chan_destroy": (C.c_int, [_P]),
+    "sxgpu_chan_output_frames": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "sxgpu_chan_apply": (C.c_int, [_P, _P, C.c_uint64, _P, C.POINTER(C.c_uint64), _P]),
+    "sxgpu_chan_get_state": (C.c_int, [_P, _P, C.POINTER(C.c_uint32), _P]),
+    "sxgpu_chan_set_state": (C.c_int, [_P, _P, C.c_uint32, _P]),
     "sxgpu_convert_rx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S]),
     "sxgpu_convert_rx_buffer_host_gated": (C.c_int, [_P, _P, _S, _P, _S, _S, _P, _P]),
     "sxgpu_convert_tx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S, _F]),
@@ -620,6 +626,69 @@ class Nco:
                 raise ValueError(f"phases and incs must have shape {(self.nstreams,)}, got {a.shape}")
             ptrs.append((a, a.ctypes.data))
         self.ctx.check(self.lib.sxgpu_nco_set_state(self.handle, ptrs[0][1], ptrs[1][1], stream), "sxgpu_nco_set_state")
+
+
+class Chan:
+    """A polyphase DFT channelizer per stream (sxgpu_chan_* in include/sxgpu.h): each stream split
+    into `channels` channel-rate streams, channel k centred at k / channels cycles per sample (numpy's
+    fft order), low-passed by the real prototype `taps` and decimated by `down` (default: channels,
+    critically sampled), the last inputs carried from call to call."""
+
+    def __init__(self, ctx: Context, nstreams: int, taps, channels: int, down: int | None = None):
+        import numpy as np
+        self.np = np
+        self.ctx, self.lib = ctx, ctx.lib
+        self.handle = None
+        down = channels if down is None else down
+        taps = np.ascontiguousarray(np.asarray(taps, dtype=np.float64))
+        if taps.ndim != 1:
+            raise ValueError(f"taps must be one-dimensional, got shape {taps.shape}")
+        h = _P()
+        ctx.check(self.lib.sxgpu_chan_create(ctx.handle, nstreams, channels, down, taps.size,
+                                             taps.ctypes.data if taps.size else None, C.byref(h)), "sxgpu_chan_create")
+        self.handle, self.nstreams, self.ntaps, self.channels, self.down = h, nstreams, taps.size, channels, down
+
+    def close(self):
+        if self.handle:
+            self.lib.sxgpu_chan_destroy(self.handle)
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def output_frames(self, nin) -> int:
+        """Frames each channel's next apply of nin frames emits."""
+        n = C.c_uint64()
+        self.ctx.check(self.lib.sxgpu_chan_output_frames(self.handle, nin, C.byref(n)), "sxgpu_chan_output_frames")
+        return n.value
+
+    def apply(self, d_in, nin, d_out, stream=None) -> int:
+        """d_in[nstreams][nin] -> d_out[nstreams][channels][nout] (complex64 on the device); returns nout."""
+        n = C.c_uint64()
+        self.ctx.check(self.lib.sxgpu_chan_apply(self.handle, d_in, nin, d_out, C.byref(n), stream), "sxgpu_chan_apply")
+        return n.value
+
+    def state(self, stream=None):
+        """(history, phase): the last ntaps - 1 inputs of each stream, (nstreams, ntaps - 1) complex64
+        oldest first, and the frames fed so far mod channels."""
+        hist = self.np.empty((self.nstreams, self.ntaps - 1), self.np.complex64)
+        phase = C.c_uint32()
+        self.ctx.check(self.lib.sxgpu_chan_get_state(self.handle, hist.ctypes.data, C.byref(phase), stream),
+                       "sxgpu_chan_get_state")
+        return hist, phase.value
+
+    def set_state(self, hist=None, phase=0, stream=None):
+        """Set the history, (nstreams, ntaps - 1) complex64 (None = zeros), and the phase."""
+        ptr = None
+        if hist is not None:
+            hist = self.np.ascontiguousarray(hist, dtype=self.np.complex64)
+            if hist.shape != (self.nstreams, self.ntaps - 1):
+                raise ValueError(f"hist must have shape {(self.nstreams, self.ntaps - 1)}, got {hist.shape}")
+            ptr = hist.ctypes.data
+        self.ctx.check(self.lib.sxgpu_chan_set_state(self.handle, ptr, phase, stream), "sxgpu_chan_set_state")
 
 
 class Multi:

@@ -11,6 +11,7 @@
 #include "sx_iir.cuh"
 #include "sx_fir.cuh"
 #include "sx_nco.cuh"
+#include "sx_chan.cuh"
 #include "sx_resident.cuh"
 #include "host/par_copy.hpp"
 #include "host/worker_pool.hpp"
@@ -130,6 +131,7 @@ struct sxgpu_ctx {
     std::atomic<int> live_iirs{0};  // so do filters
     std::atomic<int> live_firs{0};
     std::atomic<int> live_ncos{0};
+    std::atomic<int> live_chans{0};
     bool l2_carveout_set = false;   // sxgpu_bank_repeat_begin sets the persisting-L2 limit once
 
     // host pipeline: lane 0 serves the RX conversions, lane 1 the TX conversions
@@ -1470,6 +1472,8 @@ int sxgpu_destroy(sxgpu_ctx *ctx)
         return ctx->invalid("destroy the context's filters first");
     if (ctx->live_ncos.load() != 0)
         return ctx->invalid("destroy the context's oscillators first");
+    if (ctx->live_chans.load() != 0)
+        return ctx->invalid("destroy the context's channelizers first");
     cudaSetDevice(ctx->device);
     for (HostLane &lane : ctx->lanes) {
         std::lock_guard<std::mutex> lock(lane.mutex);
@@ -2875,6 +2879,19 @@ const char *nco_increments(uint32_t nstreams, const double *freq, std::vector<ui
     return nullptr;
 }
 
+// A[k] = e^{j 2 pi k / 1024}, then B[k] = e^{j 2 pi k / 2^20}: libm's double cos and sin, rounded
+// once.  The channelizers' twiddles are A conjugated.
+std::vector<float2> nco_tables()
+{
+    std::vector<float2> tab(2 * kNcoTableSize);
+    for (int k = 0; k < kNcoTableSize; k++) {
+        const double a = 2.0 * M_PI * k / 1024.0, b = 2.0 * M_PI * k / 1048576.0;
+        tab[k] = make_float2(float(std::cos(a)), float(std::sin(a)));
+        tab[kNcoTableSize + k] = make_float2(float(std::cos(b)), float(std::sin(b)));
+    }
+    return tab;
+}
+
 cudaStream_t nco_stream(sxgpu_nco *n, sxgpu_stream stream)
 {
     return stream ? static_cast<cudaStream_t>(stream) : n->ctx->stream;
@@ -2894,13 +2911,7 @@ int sxgpu_nco_create(sxgpu_ctx *ctx, uint32_t nstreams, const double *freq, sxgp
     std::vector<uint32_t> inc;
     if (const char *why = nco_increments(nstreams, freq, inc))
         return ctx->invalid(why);
-    // A[k] = e^{j 2 pi k / 1024}, B[k] = e^{j 2 pi k / 2^20}: libm's double cos and sin, rounded once.
-    std::vector<float2> tab(2 * kNcoTableSize);
-    for (int k = 0; k < kNcoTableSize; k++) {
-        const double a = 2.0 * M_PI * k / 1024.0, b = 2.0 * M_PI * k / 1048576.0;
-        tab[k] = make_float2(float(std::cos(a)), float(std::sin(a)));
-        tab[kNcoTableSize + k] = make_float2(float(std::cos(b)), float(std::sin(b)));
-    }
+    const std::vector<float2> tab = nco_tables();
     const size_t tab_bytes = tab.size() * sizeof(float2), state_bytes = size_t(nstreams) * sizeof(uint32_t);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t smem = std::min<size_t>(kFirWindowBytes, ctx->prop.sharedMemPerBlockOptin);
@@ -3107,6 +3118,259 @@ int sxgpu_bank_write_duc(sxgpu_bank *bank, sxgpu_fir *f, sxgpu_nco *nco, const v
     ctx->launches += 3;
     ctx->frames_tx += uint64_t(b.nstreams) * b.period;
     f->phase = uint32_t((f->phase + nin % f->down) % f->down);
+    return SXGPU_OK;
+}
+
+// ---- polyphase DFT channelizers (sx_chan.cuh) -------------------------------------------------
+} // extern "C"
+
+struct sxgpu_chan {
+    sxgpu_ctx *ctx = nullptr;
+    uint32_t nstreams = 0, m = 2, log2m = 1, down = 1, ntaps = 1;
+    uint32_t phase = 0;     // frames fed so far mod M: the only state kept on the host
+    void *mem = nullptr;    // one allocation: the twiddles [1024], then the taps [ntaps]
+    float2 *hist = nullptr; // [nstreams][ntaps - 1], device memory; NULL when ntaps == 1
+};
+
+namespace {
+
+constexpr size_t kChanSmemBytes = 200 * 1024; // chan_apply_kernel's shared memory, below the 227 KB of an SM
+constexpr uint32_t kChanTargetThreads = 512;
+
+// ceil((r + nin) / D) - ceil(r / D): with D dividing M, what a stream whose frame count is r mod M emits.
+uint64_t chan_outputs(const sxgpu_chan *c, uint32_t r, uint64_t nin)
+{
+    const unsigned __int128 d = c->down;
+    return uint64_t((r + (unsigned __int128)nin + d - 1) / d - (r + d - 1) / d);
+}
+
+// The geometry of a call of nin frames emitting n = chan_outputs(c, c->phase, nin) frames, without
+// its buffers, and the kernel's threads and shared memory.  False when the grid would not fit.
+bool chan_call(const sxgpu_chan *c, uint64_t nin, uint64_t n, ChanCall &a, uint32_t &threads, size_t &smem)
+{
+    const uint32_t M = c->m, D = c->down;
+    a.hist = c->hist;
+    a.tw = static_cast<const float2 *>(c->mem);
+    a.taps = reinterpret_cast<const float *>(static_cast<const float2 *>(c->mem) + kNcoTableSize);
+    a.nin = nin;
+    a.nout = n;
+    a.m = M;
+    a.log2m = c->log2m;
+    a.down = D;
+    a.ntaps = c->ntaps;
+    a.e0 = (D - c->phase % D) % D;
+    a.rot0 = (c->phase + a.e0) % M;
+    threads = 0;
+    smem = 0;
+    if (n == 0)
+        return true;
+    // As many groups as fill the target thread count (a whole branch set when M is above it),
+    // fewer when the call has fewer outputs or the window would not fit.
+    uint32_t g = std::max<uint32_t>(1, kChanTargetThreads / M);
+    while (g > 1 && uint64_t(kChanBlock) * (g / 2) >= n)
+        g /= 2;
+    for (;; g /= 2) {
+        const uint32_t t = kChanBlock * g;
+        a.win_len = (t - 1) * D + c->ntaps;
+        smem = size_t(std::max<uint64_t>(a.win_len, uint64_t(t) * (M + 1))) * sizeof(float2);
+        if (smem <= kChanSmemBytes || g == 1)
+            break;
+    }
+    a.groups = g;
+    threads = M * g;
+    const uint64_t t = kChanBlock * g;
+    a.tiles = (n + t - 1) / t;
+    return a.tiles <= uint64_t(INT32_MAX) / c->nstreams;
+}
+
+size_t chan_hist_bytes(const sxgpu_chan *c)
+{
+    return size_t(c->nstreams) * (c->ntaps - 1) * sizeof(float2);
+}
+
+cudaStream_t chan_stream(sxgpu_chan *c, sxgpu_stream stream)
+{
+    return stream ? static_cast<cudaStream_t>(stream) : c->ctx->stream;
+}
+
+} // namespace
+
+extern "C" {
+
+int sxgpu_chan_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t channels, uint32_t down, uint32_t ntaps,
+                      const double *h, sxgpu_chan **out)
+{
+    if (!ctx || !out)
+        return SXGPU_ERR_INVALID;
+    *out = nullptr;
+    if (channels < 2 || channels > SXGPU_CHAN_MAX_CHANNELS || (channels & (channels - 1)))
+        return ctx->invalid("a channelizer has a power of two of 2 to SXGPU_CHAN_MAX_CHANNELS channels");
+    if (nstreams == 0 || uint64_t(nstreams) * channels > uint64_t(INT32_MAX))
+        return ctx->invalid("a channelizer has 1 to (2^31 - 1) / channels streams");
+    if (down == 0 || channels % down)
+        return ctx->invalid("a channelizer's decimation divides its channel count");
+    if (ntaps < 1 || ntaps > SXGPU_CHAN_MAX_TAPS || ntaps > 32 * channels || !h)
+        return ctx->invalid("a channelizer has 1 to min(SXGPU_CHAN_MAX_TAPS, 32 channels) taps");
+    for (uint32_t i = 0; i < ntaps; i++)
+        if (!std::isfinite(h[i]))
+            return ctx->invalid("every channelizer tap must be finite");
+    std::unique_ptr<sxgpu_chan> c(new sxgpu_chan());
+    c->ctx = ctx;
+    c->nstreams = nstreams;
+    c->m = channels;
+    while ((1u << c->log2m) < channels)
+        c->log2m++;
+    c->down = down;
+    c->ntaps = ntaps;
+    // The twiddles: the oscillator's coarse table conjugated, then the taps rounded once.
+    std::vector<float2> tw = nco_tables();
+    tw.resize(kNcoTableSize);
+    for (float2 &w : tw)
+        w.y = -w.y;
+    std::vector<float> taps(ntaps);
+    for (uint32_t i = 0; i < ntaps; i++)
+        taps[i] = float(h[i]);
+    const size_t tw_bytes = tw.size() * sizeof(float2), taps_bytes = taps.size() * sizeof(float);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    SX_CUDA(ctx, cudaFuncSetAttribute(chan_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      int(std::min<size_t>(kChanSmemBytes, ctx->prop.sharedMemPerBlockOptin))));
+    SX_CUDA(ctx, cudaFuncSetAttribute(fir_history_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      int((kChanMaxTaps - 1) * sizeof(float2))));
+    cudaError_t e = cudaMalloc(&c->mem, tw_bytes + taps_bytes);
+    if (e == cudaSuccess)
+        e = cudaMemcpy(c->mem, tw.data(), tw_bytes, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess)
+        e = cudaMemcpy(static_cast<char *>(c->mem) + tw_bytes, taps.data(), taps_bytes, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && ntaps > 1) {
+        void *d_hist = nullptr;
+        e = cudaMalloc(&d_hist, chan_hist_bytes(c.get()));
+        c->hist = static_cast<float2 *>(d_hist);
+        if (e == cudaSuccess)
+            e = cudaMemsetAsync(d_hist, 0, chan_hist_bytes(c.get()), ctx->stream);
+        if (e == cudaSuccess)
+            e = cudaStreamSynchronize(ctx->stream);
+    }
+    if (e != cudaSuccess) {
+        cudaFree(c->hist);
+        cudaFree(c->mem);
+        return ctx->fail(e, "cudaMalloc(channelizer)");
+    }
+    ctx->live_chans++;
+    *out = c.release();
+    return SXGPU_OK;
+}
+
+int sxgpu_chan_destroy(sxgpu_chan *c)
+{
+    if (!c)
+        return SXGPU_ERR_INVALID;
+    cudaSetDevice(c->ctx->device);
+    for (HostLane &lane : c->ctx->lanes) { // a resident converter would hold the device-wide sync up
+        std::lock_guard<std::mutex> lock(lane.mutex);
+        resident_stop(c->ctx, lane);
+    }
+    cudaDeviceSynchronize();
+    cudaFree(c->hist);
+    cudaFree(c->mem);
+    c->ctx->live_chans--;
+    delete c;
+    return SXGPU_OK;
+}
+
+int sxgpu_chan_output_frames(sxgpu_chan *c, uint64_t nin, uint64_t *nout)
+{
+    if (!c || !nout)
+        return SXGPU_ERR_INVALID;
+    *nout = chan_outputs(c, c->phase, nin);
+    return SXGPU_OK;
+}
+
+int sxgpu_chan_apply(sxgpu_chan *c, const void *d_in, uint64_t nin, void *d_out, uint64_t *nout, sxgpu_stream stream)
+{
+    if (!c)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = c->ctx;
+    if (!d_in || !d_out || reinterpret_cast<uintptr_t>(d_in) % 8 || reinterpret_cast<uintptr_t>(d_out) % 8)
+        return ctx->invalid("sxgpu_chan_apply: input and output must be 8-byte aligned device memory");
+    if (nin == 0)
+        return ctx->invalid("sxgpu_chan_apply: a block has at least one frame");
+    const uint64_t nstreams = c->nstreams, rows = nstreams * c->m;
+    if (nin > UINT64_MAX / 8 / nstreams)
+        return ctx->invalid("sxgpu_chan_apply: nstreams * nin * 8 bytes overflows 64 bits");
+    const uint64_t n = chan_outputs(c, c->phase, nin);
+    if (n > UINT64_MAX / 8 / rows)
+        return ctx->invalid("sxgpu_chan_apply: nstreams * channels * nout * 8 bytes overflows 64 bits");
+    const uintptr_t in0 = reinterpret_cast<uintptr_t>(d_in), out0 = reinterpret_cast<uintptr_t>(d_out);
+    const uint64_t in_bytes = nstreams * nin * 8, out_bytes = rows * n * 8;
+    if (out_bytes && (in0 >= out0 ? in0 - out0 < out_bytes : out0 - in0 < in_bytes))
+        return ctx->invalid("sxgpu_chan_apply: input and output overlap");
+
+    ChanCall a = {};
+    uint32_t threads = 0;
+    size_t smem = 0;
+    if (!chan_call(c, nin, n, a, threads, smem))
+        return ctx->invalid("sxgpu_chan_apply: the block needs more CTAs than a grid holds");
+    a.in = static_cast<const float2 *>(d_in);
+    a.out = static_cast<float2 *>(d_out);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = chan_stream(c, stream);
+    int launches = 0;
+    if (n) {
+        chan_apply_kernel<<<unsigned(nstreams * a.tiles), threads, smem, st>>>(a);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
+    if (c->ntaps > 1) {
+        // fir_history_kernel keeps the last hp - 1 frames of buf = hist ++ in: the same history.
+        FirCall hc = {};
+        hc.in = a.in;
+        hc.hist = c->hist;
+        hc.nin = nin;
+        hc.hp = c->ntaps;
+        fir_history_kernel<<<unsigned(nstreams), kFirHistoryThreads, (c->ntaps - 1) * sizeof(float2), st>>>(hc);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
+    ctx->launches += launches;
+    c->phase = uint32_t((c->phase + nin % c->m) % c->m);
+    if (nout)
+        *nout = n;
+    return SXGPU_OK;
+}
+
+int sxgpu_chan_get_state(sxgpu_chan *c, void *h_hist, uint32_t *phase, sxgpu_stream stream)
+{
+    if (!c)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = c->ctx;
+    if (h_hist && c->ntaps > 1) {
+        SX_CUDA(ctx, cudaSetDevice(ctx->device));
+        cudaStream_t st = chan_stream(c, stream);
+        SX_CUDA(ctx, cudaMemcpyAsync(h_hist, c->hist, chan_hist_bytes(c), cudaMemcpyDeviceToHost, st));
+        SX_CUDA(ctx, cudaStreamSynchronize(st));
+    }
+    if (phase)
+        *phase = c->phase;
+    return SXGPU_OK;
+}
+
+int sxgpu_chan_set_state(sxgpu_chan *c, const void *h_hist, uint32_t phase, sxgpu_stream stream)
+{
+    if (!c)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = c->ctx;
+    if (phase >= c->m)
+        return ctx->invalid("sxgpu_chan_set_state: the phase is below the channel count");
+    if (c->ntaps > 1) {
+        SX_CUDA(ctx, cudaSetDevice(ctx->device));
+        cudaStream_t st = chan_stream(c, stream);
+        if (h_hist)
+            SX_CUDA(ctx, cudaMemcpyAsync(c->hist, h_hist, chan_hist_bytes(c), cudaMemcpyHostToDevice, st));
+        else
+            SX_CUDA(ctx, cudaMemsetAsync(c->hist, 0, chan_hist_bytes(c), st));
+        SX_CUDA(ctx, cudaStreamSynchronize(st));
+    }
+    c->phase = phase;
     return SXGPU_OK;
 }
 
