@@ -393,9 +393,9 @@ int sxgpu_nco_set_state(sxgpu_nco *n, const uint32_t *h_phase, const uint32_t *h
  * full-rate CF32 block in memory.  Both need nco and f of this context with the bank's stream
  * count, and refuse, with SXGPU_ERR_INVALID and nothing enqueued, what sxgpu_bank_read_fir /
  * sxgpu_bank_write_fir refuse and a NULL or foreign oscillator or a stream-count mismatch.
- * Only kernels are enqueued: the bank's plan kernel, then the data kernel (bank_nco_fir_kernel) as
+ * Only kernels are enqueued: the bank's plan kernel, then the data kernel (bank_fir_kernel, mixing) as
  * its programmatic dependent when the filter emits at least one frame (always, for the write),
- * then the tail kernel (bank_nco_fir_read_tail_kernel / bank_nco_fir_write_tail_kernel: the
+ * then the tail kernel (bank_fir_read_tail_kernel / fir_history_kernel, mixing and advancing: the
  * filter's new history and, for a synthetic read, the capture slot; the phases advanced by the
  * period), which always runs: so 3 launches per call at most (read: 2 when the call emits
  * nothing; write: always 3), counted in "launches".  The oscillator never prevents graph capture;

@@ -168,8 +168,29 @@ def load_library(build: bool = True) -> C.CDLL:
     return _lib
 
 
-class Context:
+class _Owned:
+    """An object behind a C handle: `close` (also on leaving a `with` block) frees it with the type's
+    destroy function, named by `_destroy`, once."""
+
+    handle = None
+    _destroy = ""
+
+    def close(self):
+        if self.handle:
+            getattr(self.lib, self._destroy)(self.handle)
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class Context(_Owned):
     """One sxgpu context = one GPU.  Thin, checked wrappers over the C ABI."""
+
+    _destroy = "sxgpu_destroy"
 
     def __init__(self, device: int = 0):
         self.lib = load_library()
@@ -179,17 +200,6 @@ class Context:
             raise SxGpuError(rc, "sxgpu_init", self.lib.sxgpu_strerror(rc).decode())
         self.handle = h
         self.device = device
-
-    def close(self):
-        if self.handle:
-            self.lib.sxgpu_destroy(self.handle)
-            self.handle = None
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def check(self, rc: int, what: str) -> None:
         if rc != SXGPU_OK:
@@ -317,8 +327,10 @@ class Context:
         return out
 
 
-class Bank:
+class Bank(_Owned):
     """A bank of HBM-resident stream pairs (sxgpu_bank_* in include/sxgpu.h)."""
+
+    _destroy = "sxgpu_bank_destroy"
 
     def __init__(self, ctx: Context, nstreams: int, period: int = 0, sample_rate: float = 75000.0,
                  tx_threshold2: float = 1.0e-6, seed: int = 0x53581255):
@@ -333,17 +345,6 @@ class Bank:
         self.lib.sxgpu_bank_ring_frames(h, C.byref(r))
         self.ring = r.value
         self.period = period if 0 < period <= 65536 else (256 if period == 0 else 65536)
-
-    def close(self):
-        if self.handle:
-            self.lib.sxgpu_bank_destroy(self.handle)
-            self.handle = None
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def advance(self, frames, stream=None):
         self.ctx.check(self.lib.sxgpu_bank_advance(self.handle, frames, stream), "sxgpu_bank_advance")
@@ -446,16 +447,17 @@ class Bank:
         return out
 
 
-class Iir:
+class Iir(_Owned):
     """A cascade of second-order sections with one state per stream (sxgpu_iir_* in include/sxgpu.h):
     scipy.signal.sosfilt(sos, x, zi=state) along each stream's block, carried from call to call.
     `sos` is what scipy's filter design functions return with output="sos": (nsections, 6)."""
+
+    _destroy = "sxgpu_iir_destroy"
 
     def __init__(self, ctx: Context, nstreams: int, sos):
         import numpy as np
         self.np = np
         self.ctx, self.lib = ctx, ctx.lib
-        self.handle = None
         sos = np.ascontiguousarray(np.asarray(sos, dtype=np.float64))
         if sos.ndim != 2 or sos.shape[1] != 6:
             raise ValueError(f"sos must have shape (nsections, 6), got {sos.shape}")
@@ -463,17 +465,6 @@ class Iir:
         ctx.check(self.lib.sxgpu_iir_create(ctx.handle, nstreams, sos.shape[0], sos.ctypes.data, C.byref(h)),
                   "sxgpu_iir_create")
         self.handle, self.nstreams, self.nsections = h, nstreams, sos.shape[0]
-
-    def close(self):
-        if self.handle:
-            self.lib.sxgpu_iir_destroy(self.handle)
-            self.handle = None
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def apply(self, d_cf32, period, stream=None):
         """Filter d_cf32[nstreams][period] (complex64 on the device) in place."""
@@ -502,16 +493,17 @@ class Iir:
         self.ctx.check(self.lib.sxgpu_iir_set_state(self.handle, ptr, stream), "sxgpu_iir_set_state")
 
 
-class Fir:
+class Fir(_Owned):
     """Real FIR taps with an up/down rate change and one history per stream (sxgpu_fir_* in
     include/sxgpu.h): scipy.signal.upfirdn(taps, x, up, down) on each stream's concatenated input,
     bit for bit, carried from call to call.  up = down = 1 is a plain FIR filter."""
+
+    _destroy = "sxgpu_fir_destroy"
 
     def __init__(self, ctx: Context, nstreams: int, taps, up: int = 1, down: int = 1):
         import numpy as np
         self.np = np
         self.ctx, self.lib = ctx, ctx.lib
-        self.handle = None
         taps = np.ascontiguousarray(np.asarray(taps, dtype=np.float64))
         if taps.ndim != 1:
             raise ValueError(f"taps must be one-dimensional, got shape {taps.shape}")
@@ -520,17 +512,6 @@ class Fir:
                                             up, down, C.byref(h)), "sxgpu_fir_create")
         self.handle, self.nstreams, self.ntaps, self.up, self.down = h, nstreams, taps.size, up, down
         self.hp = -(-taps.size // up)
-
-    def close(self):
-        if self.handle:
-            self.lib.sxgpu_fir_destroy(self.handle)
-            self.handle = None
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def output_frames(self, nin) -> int:
         """Frames each stream's next apply of nin frames emits."""
@@ -564,17 +545,18 @@ class Fir:
         self.ctx.check(self.lib.sxgpu_fir_set_state(self.handle, ptr, phase, stream), "sxgpu_fir_set_state")
 
 
-class Nco:
+class Nco(_Owned):
     """One numerically controlled oscillator per stream (sxgpu_nco_* in include/sxgpu.h): each
     frame multiplied by exp(+2j pi phase / 2^32), the 32-bit phase advancing by the increment
     rint(f 2^32) per frame, carried from call to call.  `freqs` in cycles per sample, -0.5 .. 0.5
     (None: all 0); to bring a channel at +f0 to DC, use -f0."""
 
+    _destroy = "sxgpu_nco_destroy"
+
     def __init__(self, ctx: Context, nstreams: int, freqs=None):
         import numpy as np
         self.np = np
         self.ctx, self.lib = ctx, ctx.lib
-        self.handle = None
         f = self._freqs(nstreams, freqs)
         h = _P()
         ctx.check(self.lib.sxgpu_nco_create(ctx.handle, nstreams, f.ctypes.data if f is not None else None, C.byref(h)),
@@ -585,17 +567,6 @@ class Nco:
         if freqs is None:
             return None
         return self.np.ascontiguousarray(self.np.broadcast_to(self.np.asarray(freqs, dtype=self.np.float64), (nstreams,)))
-
-    def close(self):
-        if self.handle:
-            self.lib.sxgpu_nco_destroy(self.handle)
-            self.handle = None
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def apply(self, d_cf32, nframes, stream=None):
         """Mix d_cf32[nstreams][nframes] (complex64 on the device) in place."""
@@ -628,17 +599,18 @@ class Nco:
         self.ctx.check(self.lib.sxgpu_nco_set_state(self.handle, ptrs[0][1], ptrs[1][1], stream), "sxgpu_nco_set_state")
 
 
-class Chan:
+class Chan(_Owned):
     """A polyphase DFT channelizer per stream (sxgpu_chan_* in include/sxgpu.h): each stream split
     into `channels` channel-rate streams, channel k centred at k / channels cycles per sample (numpy's
     fft order), low-passed by the real prototype `taps` and decimated by `down` (default: channels,
     critically sampled), the last inputs carried from call to call."""
 
+    _destroy = "sxgpu_chan_destroy"
+
     def __init__(self, ctx: Context, nstreams: int, taps, channels: int, down: int | None = None):
         import numpy as np
         self.np = np
         self.ctx, self.lib = ctx, ctx.lib
-        self.handle = None
         down = channels if down is None else down
         taps = np.ascontiguousarray(np.asarray(taps, dtype=np.float64))
         if taps.ndim != 1:
@@ -647,17 +619,6 @@ class Chan:
         ctx.check(self.lib.sxgpu_chan_create(ctx.handle, nstreams, channels, down, taps.size,
                                              taps.ctypes.data if taps.size else None, C.byref(h)), "sxgpu_chan_create")
         self.handle, self.nstreams, self.ntaps, self.channels, self.down = h, nstreams, taps.size, channels, down
-
-    def close(self):
-        if self.handle:
-            self.lib.sxgpu_chan_destroy(self.handle)
-            self.handle = None
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     def output_frames(self, nin) -> int:
         """Frames each channel's next apply of nin frames emits."""

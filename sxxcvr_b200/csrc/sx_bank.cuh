@@ -37,14 +37,13 @@
 //     bank_plan_{repeat,read,write}_kernel, then bank_repeat_iir_kernel<Hook, MODE>: whole
 //                             streams per CTA through shared-memory tiles, as a programmatic
 //                             dependent of the plan kernel
-// and a half with a FIR filter or resampler (every bank size) as:
-//     bank_plan_{read,write}_kernel, then bank_fir_kernel<R, MODE>: fir_apply_kernel's polyphase
-//                             tiles with the frames taken from the capture or stored into the
-//                             ring, as a programmatic dependent of the plan kernel, then
-//                             bank_fir_read_tail_kernel / fir_history_kernel
-// and the same with an oscillator mixing the full-rate frames (digital down- and up-conversion):
-//     bank_plan_{read,write}_kernel, then bank_nco_fir_kernel<R, MODE>, then
-//                             bank_nco_fir_{read,write}_tail_kernel, which also advance the phases
+// and a half with a FIR filter or resampler (every bank size), with or without an oscillator
+// mixing the full-rate frames (digital down- and up-conversion), as:
+//     bank_plan_{read,write}_kernel, then bank_fir_kernel<R, MODE, Nco>: fir_apply_kernel's
+//                             polyphase tiles with the frames taken from the capture or stored
+//                             into the ring, as a programmatic dependent of the plan kernel, then
+//                             bank_fir_read_tail_kernel<Nco> / fir_history_kernel<Nco>, which also
+//                             advance the phases when Nco is NcoView
 // The virtual clock follows the same rule as the host-side ALSA stand-in: it moves when a
 // blocking transfer must wait (by exactly the deficit) or when the owner advances it.
 #pragma once
@@ -1016,6 +1015,18 @@ inline cudaError_t launch_bank_iir(const BankState &b, char *cf32, bool capture_
 //     tx_ring_offset[s] + 8 k when the block starts on a period boundary of the ring, frame by
 //     frame through ring_frame() when it straddles two slices, nowhere when the write was dropped
 //     as late.  The new history is fir_history_kernel's, from the caller's block as for apply.
+//
+// With an oscillator (sxgpu_bank_read_ddc, sxgpu_bank_write_duc) the full-rate frames are mixed
+// (sx_nco.cuh), so that the same state, results, capture, ring, filter history, phases and outputs
+// come out as from the plain half, sxgpu_nco_apply and sxgpu_fir_apply one after the other:
+//   read:  input frame i of the filter is capture frame i of the period through RxCf32, mixed with
+//          phi_s + i inc_s; the read tail mixes the history's new frames the same way and advances
+//          phi_s.
+//   write: output k of the filter is mixed with phi_s + k inc_s before TxCf32 and the ring;
+//          fir_history_kernel advances phi_s, also for a stream whose write was dropped as late.
+// Every read of phi_s is in the data kernel or before the tail kernel's barrier, and the phase
+// advances after it.  Each kernel takes the oscillator as its template parameter Nco: NoNco for
+// the plain half, NcoView with one.
 // ---------------------------------------------------------------------------------------
 __device__ __forceinline__ float2 rx_frame(const Pack<2> &cap)
 {
@@ -1024,82 +1035,13 @@ __device__ __forceinline__ float2 rx_frame(const Pack<2> &cap)
     return make_float2(__uint_as_float(f.w[0]), __uint_as_float(f.w[1]));
 }
 
-template <int R, int MODE>
-__global__ void __launch_bounds__(32) bank_fir_kernel(BankState b, const __grid_constant__ FirCall a, bool capture_in_slot)
+template <int R, int MODE, class Nco>
+__global__ void __launch_bounds__(32) bank_fir_kernel(BankState b, const __grid_constant__ FirCall a, bool capture_in_slot, Nco nco)
 {
     extern __shared__ __align__(16) float2 win[];
     const uint64_t stream = blockIdx.x / a.chunks, chunk = blockIdx.x % a.chunks;
     pdl_wait(); // the decisions, and everything before them on the stream, are in memory
-    if constexpr (MODE == kBankModeRead) {
-        auto out = [&](uint64_t k, float2 v) { a.out[stream * a.nout + k] = v; };
-        if (capture_in_slot) {
-            const char *slot = b.capture_stage + stream * b.period * 8;
-            fir_tile<R>(a, threadIdx.x, stream, chunk, win, [&](const float2 *, uint64_t i) { return rx_frame(ld_stream<8>(slot + i * 8)); }, out);
-        } else {
-            const uint64_t seed = b.seed + stream, first = uint64_t(b.rx_first_frame[stream]);
-            fir_tile<R>(a, threadIdx.x, stream, chunk, win, [&](const float2 *, uint64_t i) { return rx_frame(capture_frame(seed, first + i)); }, out);
-        }
-    } else {
-        const long long off = b.tx_ring_offset[stream];
-        if (off < 0)
-            return; // dropped as late: nothing is stored (the history still advances, fir_history_kernel)
-        const long long at = b.tx_write_position[stream];
-        fir_tile<R>(a, threadIdx.x, stream, chunk, win, [](const float2 *row, uint64_t i) { return row[i]; }, [&](uint64_t k, float2 v) {
-            Pack<2> f, w;
-            f.w[0] = __float_as_uint(v.x), f.w[1] = __float_as_uint(v.y);
-            TxCf32::apply<1>(f, w, b.thr2);
-            st_stream<8>((off & 1) == 0 ? b.playback_ring + off + k * 8 : ring_frame(b, stream, uint64_t(at) + k), w);
-        });
-    }
-}
-
-// After a read's bank_fir_kernel (or straight after the plan when the call emits nothing), one CTA
-// per stream: the new history, the last hp - 1 frames of old history ++ RX(capture), read before
-// any of it is overwritten as in fir_history_kernel; and with synthetic capture the whole capture
-// slot, every frame once with the value sxgpu_bank_read stores.  (The data kernel's CTAs stage
-// overlapping windows, so none of them owns the slot's frames; here they are written in order.)
-__global__ void __launch_bounds__(kFirHistoryThreads) bank_fir_read_tail_kernel(BankState b, const __grid_constant__ FirCall a,
-                                                                                bool capture_in_slot)
-{
-    extern __shared__ __align__(16) float2 keep[]; // [hp - 1]
-    const uint32_t n = a.hp - 1;
-    const uint64_t s = blockIdx.x;
-    char *slot = b.capture_stage + s * b.period * 8;
-    const uint64_t seed = b.seed + s, first = capture_in_slot ? 0 : uint64_t(b.rx_first_frame[s]);
-    float2 *hist = a.hist + s * n;
-    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads) {
-        const uint64_t k = a.nin + i; // buffer frame
-        keep[i] = k < n ? hist[k] : rx_frame(capture_in_slot ? ld_stream<8>(slot + (k - n) * 8) : capture_frame(seed, first + k - n));
-    }
-    for (uint32_t i = threadIdx.x; i < b.period && !capture_in_slot; i += kFirHistoryThreads)
-        st_stream<8>(slot + size_t(i) * 8, capture_frame(seed, first + i));
-    __syncthreads();
-    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads)
-        hist[i] = keep[i];
-}
-
-// ---------------------------------------------------------------------------------------
-// The FIR halves with an oscillator (sxgpu_bank_read_ddc, sxgpu_bank_write_duc): the kernels above
-// with the full-rate frames mixed (sx_nco.cuh), so that the same state, results, capture, ring,
-// filter history, phases and outputs come out as from the plain half, sxgpu_nco_apply and
-// sxgpu_fir_apply one after the other.
-//   read:  input frame i of the filter is capture frame i of the period through RxCf32, mixed with
-//          phi_s + i inc_s; bank_nco_fir_read_tail_kernel mixes the history's new frames the same
-//          way, writes the capture slot as bank_fir_read_tail_kernel does, and advances phi_s.
-//   write: output k of the filter is mixed with phi_s + k inc_s before TxCf32 and the ring;
-//          bank_nco_fir_write_tail_kernel writes the filter's history as fir_history_kernel does
-//          and advances phi_s, also for a stream whose write was dropped as late.
-// Every read of phi_s is in the data kernel or before the tail kernel's barrier, and the phase
-// advances after it.
-// ---------------------------------------------------------------------------------------
-template <int R, int MODE>
-__global__ void __launch_bounds__(32) bank_nco_fir_kernel(BankState b, const __grid_constant__ FirCall a, bool capture_in_slot,
-                                                          NcoView nco)
-{
-    extern __shared__ __align__(16) float2 win[];
-    const uint64_t stream = blockIdx.x / a.chunks, chunk = blockIdx.x % a.chunks;
-    pdl_wait(); // the decisions, and everything before them on the stream, are in memory
-    const NcoStream mix = nco_stream(nco, stream);
+    const auto mix = nco_stream(nco, stream);
     if constexpr (MODE == kBankModeRead) {
         auto out = [&](uint64_t k, float2 v) { a.out[stream * a.nout + k] = v; };
         if (capture_in_slot) {
@@ -1124,8 +1066,16 @@ __global__ void __launch_bounds__(32) bank_nco_fir_kernel(BankState b, const __g
     }
 }
 
-__global__ void __launch_bounds__(kFirHistoryThreads) bank_nco_fir_read_tail_kernel(BankState b, const __grid_constant__ FirCall a,
-                                                                                    bool capture_in_slot, NcoView nco)
+// After a read's bank_fir_kernel (or straight after the plan when the call emits nothing), one CTA
+// per stream: the new history, the last hp - 1 frames of old history ++ RX(capture) (mixed as the
+// data kernel mixes them), read before any of it is overwritten as in fir_history_kernel; with
+// synthetic capture the whole capture slot, every frame once with the value sxgpu_bank_read stores;
+// and with an oscillator the phase advanced by the period, after the barrier.  (The data kernel's
+// CTAs stage overlapping windows, so none of them owns the slot's frames; here they are written in
+// order.)
+template <class Nco>
+__global__ void __launch_bounds__(kFirHistoryThreads) bank_fir_read_tail_kernel(BankState b, const __grid_constant__ FirCall a,
+                                                                                bool capture_in_slot, Nco nco)
 {
     extern __shared__ __align__(16) float2 keep[]; // [hp - 1]
     const uint32_t n = a.hp - 1;
@@ -1133,7 +1083,7 @@ __global__ void __launch_bounds__(kFirHistoryThreads) bank_nco_fir_read_tail_ker
     char *slot = b.capture_stage + s * b.period * 8;
     const uint64_t seed = b.seed + s, first = capture_in_slot ? 0 : uint64_t(b.rx_first_frame[s]);
     float2 *hist = a.hist + s * n;
-    const NcoStream mix = nco_stream(nco, s);
+    const auto mix = nco_stream(nco, s);
     for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads) {
         const uint64_t k = a.nin + i; // buffer frame
         keep[i] = k < n ? hist[k] : mix(k - n, rx_frame(capture_in_slot ? ld_stream<8>(slot + (k - n) * 8) : capture_frame(seed, first + k - n)));
@@ -1147,49 +1097,29 @@ __global__ void __launch_bounds__(kFirHistoryThreads) bank_nco_fir_read_tail_ker
         nco_advance(nco, s, b.period);
 }
 
-__global__ void __launch_bounds__(kFirHistoryThreads) bank_nco_fir_write_tail_kernel(const __grid_constant__ FirCall a, NcoView nco,
-                                                                                     uint32_t period)
-{
-    extern __shared__ __align__(16) float2 keep[]; // [hp - 1]
-    const uint32_t n = a.hp - 1;
-    const uint64_t s = blockIdx.x;
-    float2 *hist = a.hist + s * n;
-    const float2 *in = a.in + s * a.nin;
-    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads) {
-        const uint64_t k = a.nin + i; // buffer frame
-        keep[i] = k < n ? hist[k] : in[k - n];
-    }
-    __syncthreads();
-    for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads)
-        hist[i] = keep[i];
-    if (threadIdx.x == 0)
-        nco_advance(nco, s, period);
-}
-
 // The data kernel of a FIR half in its R, as a programmatic dependent of the plan kernel.
-template <int MODE>
+template <int MODE, class Nco>
 inline cudaError_t launch_bank_fir(const BankState &b, const FirCall &a, int block, size_t smem, bool capture_in_slot,
-                                   cudaStream_t st)
+                                   const Nco &nco, cudaStream_t st)
 {
     const unsigned grid = unsigned(uint64_t(b.nstreams) * a.chunks);
     if (block == 4)
-        return launch_dependent(bank_fir_kernel<4, MODE>, grid, 32, smem, st, b, a, capture_in_slot);
+        return launch_dependent(bank_fir_kernel<4, MODE, Nco>, grid, 32, smem, st, b, a, capture_in_slot, nco);
     if (block == 2)
-        return launch_dependent(bank_fir_kernel<2, MODE>, grid, 32, smem, st, b, a, capture_in_slot);
-    return launch_dependent(bank_fir_kernel<1, MODE>, grid, 32, smem, st, b, a, capture_in_slot);
+        return launch_dependent(bank_fir_kernel<2, MODE, Nco>, grid, 32, smem, st, b, a, capture_in_slot, nco);
+    return launch_dependent(bank_fir_kernel<1, MODE, Nco>, grid, 32, smem, st, b, a, capture_in_slot, nco);
 }
 
-// The same with the oscillator.
-template <int MODE>
-inline cudaError_t launch_bank_nco_fir(const BankState &b, const FirCall &a, int block, size_t smem, bool capture_in_slot,
-                                       const NcoView &nco, cudaStream_t st)
+// Lets every bank_fir_kernel with this oscillator stage a window of up to `smem` bytes.
+template <class Nco>
+inline cudaError_t bank_fir_allow_smem(size_t smem)
 {
-    const unsigned grid = unsigned(uint64_t(b.nstreams) * a.chunks);
-    if (block == 4)
-        return launch_dependent(bank_nco_fir_kernel<4, MODE>, grid, 32, smem, st, b, a, capture_in_slot, nco);
-    if (block == 2)
-        return launch_dependent(bank_nco_fir_kernel<2, MODE>, grid, 32, smem, st, b, a, capture_in_slot, nco);
-    return launch_dependent(bank_nco_fir_kernel<1, MODE>, grid, 32, smem, st, b, a, capture_in_slot, nco);
+    for (auto kernel : {bank_fir_kernel<1, kBankModeRead, Nco>, bank_fir_kernel<2, kBankModeRead, Nco>,
+                        bank_fir_kernel<4, kBankModeRead, Nco>, bank_fir_kernel<1, kBankModeWrite, Nco>,
+                        bank_fir_kernel<2, kBankModeWrite, Nco>, bank_fir_kernel<4, kBankModeWrite, Nco>})
+        if (const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)))
+            return e;
+    return cudaSuccess;
 }
 
 __global__ void bank_advance_kernel(BankState b, long long frames)

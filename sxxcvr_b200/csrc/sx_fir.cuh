@@ -23,6 +23,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "sx_nco.cuh"
+
 namespace sx {
 
 constexpr int kFirMaxTaps = 4096;  // SXGPU_FIR_MAX_TAPS
@@ -154,10 +156,13 @@ __global__ void __launch_bounds__(32) fir_apply_kernel(const __grid_constant__ F
 // The new history, hist = buf[nin .. nin + hp - 2], after fir_apply_kernel has read the old one
 // (a separate launch, so that no CTA of the apply can see a half-written history).  One CTA per
 // stream: the frames that still come from the old history (nin < hp - 1) are read into shared
-// memory before any is overwritten.
+// memory before any is overwritten.  With an oscillator (sxgpu_bank_write_duc), thread 0 then
+// advances the stream's phase by `frames`, after the barrier, as every read of it has ended.
 constexpr int kFirHistoryThreads = 128;
 
-__global__ void __launch_bounds__(kFirHistoryThreads) fir_history_kernel(const __grid_constant__ FirCall a)
+template <class Nco = NoNco>
+__global__ void __launch_bounds__(kFirHistoryThreads) fir_history_kernel(const __grid_constant__ FirCall a, Nco nco = {},
+                                                                         uint32_t frames = 0)
 {
     extern __shared__ __align__(16) float2 keep[]; // [hp - 1]
     const uint32_t n = a.hp - 1;
@@ -171,6 +176,8 @@ __global__ void __launch_bounds__(kFirHistoryThreads) fir_history_kernel(const _
     __syncthreads();
     for (uint32_t i = threadIdx.x; i < n; i += kFirHistoryThreads)
         hist[i] = keep[i];
+    if (threadIdx.x == 0)
+        nco_advance(nco, stream, frames);
 }
 
 } // namespace sx

@@ -69,6 +69,21 @@ __device__ __forceinline__ void nco_advance(const NcoView &v, uint64_t s, uint32
     v.phase[s] += frames * v.inc[s];
 }
 
+// No oscillator.  The FIR kernels that can mix (fir_history_kernel, bank_fir_kernel,
+// bank_fir_read_tail_kernel) take the oscillator as a template parameter: with NoNco the two
+// overloads below compile to nothing, so those instantiations are the plain kernels, and with
+// NcoView they are the mixing ones, from the same source.
+struct NoNco {
+};
+
+struct NoMix {
+    __device__ __forceinline__ float2 operator()(uint64_t, float2 x) const { return x; }
+};
+
+__device__ __forceinline__ NoMix nco_stream(NoNco, uint64_t) { return {}; }
+
+__device__ __forceinline__ void nco_advance(NoNco, uint64_t, uint32_t) {}
+
 // sxgpu_nco_apply: x[nstreams][nframes] mixed in place, one tile of kNcoTile frames of the flat
 // block per CTA, kNcoFramesPerThread frames per thread, kNcoThreads apart so that each warp access
 // is 256 contiguous bytes.  A frame's stream is g div nframes, found with a double reciprocal

@@ -128,10 +128,7 @@ struct sxgpu_ctx {
 
     std::atomic<uint64_t> resident_launches{0}, resident_calls{0}, flagged_calls{0};
     std::atomic<int> live_banks{0}; // banks keep a pointer to their context
-    std::atomic<int> live_iirs{0};  // so do filters
-    std::atomic<int> live_firs{0};
-    std::atomic<int> live_ncos{0};
-    std::atomic<int> live_chans{0};
+    std::atomic<int> live_dsp{0};   // so do filters, oscillators and channelizers
     bool l2_carveout_set = false;   // sxgpu_bank_repeat_begin sets the persisting-L2 limit once
 
     // host pipeline: lane 0 serves the RX conversions, lane 1 the TX conversions
@@ -174,6 +171,12 @@ struct sxgpu_ctx {
 };
 
 namespace {
+
+// The CUDA stream of a call on ctx or on one of its objects: the caller's, or the context's.
+cudaStream_t call_stream(const sxgpu_ctx *ctx, sxgpu_stream stream)
+{
+    return stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+}
 
 // Which CPUs sit next to this GPU?  Linux publishes it per PCI function; a VM without NUMA
 // topology lists every CPU and node -1, and then there is nothing to choose.
@@ -562,7 +565,7 @@ int convert_entry(sxgpu_ctx *ctx, const void *d_src, size_t src_offset, void *d_
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const char *src = static_cast<const char *>(d_src) + src_offset * (Op::kSrcWords * 4);
     char *dst = static_cast<char *>(d_dest) + dest_offset * (Op::kDstWords * 4);
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st = call_stream(ctx, stream);
     return launch_convert<Op>(ctx, src, dst, length, thr2, variant, st);
 }
 
@@ -652,6 +655,76 @@ void resident_stop(sxgpu_ctx *, HostLane &lane)
     std::atomic_thread_fence(std::memory_order_seq_cst);
     cudaStreamSynchronize(lane.s_resident);
     box->quit = 0;
+}
+
+// Before device memory that kernels may still use is freed: stop the resident converters (each
+// would hold the device-wide synchronisation up), then wait for the device.
+void quiesce(sxgpu_ctx *ctx)
+{
+    cudaSetDevice(ctx->device);
+    for (HostLane &lane : ctx->lanes) {
+        std::lock_guard<std::mutex> lock(lane.mutex);
+        resident_stop(ctx, lane);
+    }
+    cudaDeviceSynchronize();
+}
+
+// ---- the lifetime of the DSP objects (filters, oscillators, channelizers) ----------------------
+// Their device memory frees itself, so that a create that fails half-way leaves nothing behind and
+// a destroy is the object's destructor.
+struct CudaFree {
+    void operator()(void *p) const { cudaFree(p); }
+};
+template <class T> using DevPtr = std::unique_ptr<T, CudaFree>;
+
+// `bytes` of device memory holding a copy of the host's src, or zeros when src is NULL, enqueued on
+// the context's stream; the create waits for it in dsp_created.
+template <class T> cudaError_t dev_upload(sxgpu_ctx *ctx, DevPtr<T> &d, const void *src, size_t bytes)
+{
+    void *p = nullptr;
+    const cudaError_t e = cudaMalloc(&p, bytes);
+    if (e != cudaSuccess)
+        return e;
+    d.reset(static_cast<T *>(p));
+    return src ? cudaMemcpyAsync(p, src, bytes, cudaMemcpyHostToDevice, ctx->stream) : cudaMemsetAsync(p, 0, bytes, ctx->stream);
+}
+
+// The end of every DSP object's create: e is the first error of its uploads.  Waits for them, then
+// hands the object out and counts it; on an error the object and its memory go.
+template <class T> int dsp_created(sxgpu_ctx *ctx, std::unique_ptr<T> &obj, cudaError_t e, const char *what, T **out)
+{
+    if (e == cudaSuccess)
+        e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess)
+        return ctx->fail(e, what);
+    ctx->live_dsp++;
+    *out = obj.release();
+    return SXGPU_OK;
+}
+
+template <class T> int dsp_destroy(T *obj)
+{
+    if (!obj)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = obj->ctx;
+    quiesce(ctx);
+    delete obj;
+    ctx->live_dsp--;
+    return SXGPU_OK;
+}
+
+// What get_state / set_state do with a DSP object's device state: `bytes` from src to dst in the
+// direction `kind` (dst zeroed when src is NULL) on the call's stream, waited for.
+int state_copy(sxgpu_ctx *ctx, void *dst, const void *src, size_t bytes, cudaMemcpyKind kind, sxgpu_stream stream)
+{
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const cudaStream_t st = call_stream(ctx, stream);
+    if (src)
+        SX_CUDA(ctx, cudaMemcpyAsync(dst, src, bytes, kind, st));
+    else
+        SX_CUDA(ctx, cudaMemsetAsync(dst, 0, bytes, st));
+    SX_CUDA(ctx, cudaStreamSynchronize(st));
+    return SXGPU_OK;
 }
 
 int ensure_ring(sxgpu_ctx *ctx, HostLane &lane, size_t frames, bool bounce_in, bool bounce_out)
@@ -1165,7 +1238,7 @@ int convert_batch(sxgpu_ctx *ctx, const sxgpu_block *blocks, uint32_t nblocks, i
     if (!blocks)
         return ctx->invalid("null block list");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st = call_stream(ctx, stream);
 
     const BlockDesc *d_blocks = reinterpret_cast<const BlockDesc *>(blocks);
     void *staged = nullptr;
@@ -1468,18 +1541,9 @@ int sxgpu_destroy(sxgpu_ctx *ctx)
         return SXGPU_ERR_INVALID;
     if (ctx->live_banks.load() != 0)
         return ctx->invalid("destroy the context's stream banks first");
-    if (ctx->live_iirs.load() != 0 || ctx->live_firs.load() != 0)
-        return ctx->invalid("destroy the context's filters first");
-    if (ctx->live_ncos.load() != 0)
-        return ctx->invalid("destroy the context's oscillators first");
-    if (ctx->live_chans.load() != 0)
-        return ctx->invalid("destroy the context's channelizers first");
-    cudaSetDevice(ctx->device);
-    for (HostLane &lane : ctx->lanes) {
-        std::lock_guard<std::mutex> lock(lane.mutex);
-        resident_stop(ctx, lane);
-    }
-    cudaDeviceSynchronize();
+    if (ctx->live_dsp.load() != 0)
+        return ctx->invalid("destroy the context's filters, oscillators and channelizers first");
+    quiesce(ctx);
     for (HostLane &lane : ctx->lanes) {
         HostRing &r = lane.ring;
         for (int i = 0; i < kRingSlots; i++) {
@@ -1615,7 +1679,7 @@ int sxgpu_convert_loopback(sxgpu_ctx *ctx, const void *d_i2s_in, void *d_cf32, v
     if (misaligned(d_i2s_in) || misaligned(d_i2s_out) || (d_cf32 && misaligned(d_cf32)))
         return ctx->invalid("loopback buffers must be 16-byte aligned");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st = call_stream(ctx, stream);
     if (ctx->loopback_variant == 0 || ctx->loopback_variant == 2) {
         // One tile per CTA, handed out in index order by the hardware (see launch_convert): two
         // 16-byte vectors per thread in flight, 6.8 TB/s of 24 B/frame at 2^27 frames.
@@ -1694,11 +1758,6 @@ template <class T> T *carve(char *&cursor, size_t count)
 // separate thread-per-stream plan kernels are 20 % faster.
 constexpr uint32_t kBankFusedPlanStreams = 8192;
 
-
-cudaStream_t bank_stream(sxgpu_bank *bank, sxgpu_stream stream)
-{
-    return stream ? static_cast<cudaStream_t>(stream) : bank->ctx->stream;
-}
 
 int per_stream_grid(uint32_t nstreams, int block)
 {
@@ -1802,12 +1861,7 @@ int sxgpu_bank_destroy(sxgpu_bank *bank)
 {
     if (!bank)
         return SXGPU_ERR_INVALID;
-    cudaSetDevice(bank->ctx->device);
-    for (HostLane &lane : bank->ctx->lanes) { // a resident converter would hold the device-wide sync up
-        std::lock_guard<std::mutex> lock(lane.mutex);
-        resident_stop(bank->ctx, lane);
-    }
-    cudaDeviceSynchronize();
+    quiesce(bank->ctx);
     cudaFree(bank->arena);
     bank->ctx->live_banks--;
     delete bank;
@@ -1830,7 +1884,7 @@ int sxgpu_bank_advance(sxgpu_bank *bank, int64_t frames, sxgpu_stream stream)
     if (frames < 0)
         return ctx->invalid("the sample clock only runs forward");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    bank_advance_kernel<<<per_stream_grid(bank->st.nstreams, 256), 256, 0, bank_stream(bank, stream)>>>(
+    bank_advance_kernel<<<per_stream_grid(bank->st.nstreams, 256), 256, 0, call_stream(bank->ctx, stream)>>>(
         bank->st, frames);
     SX_CUDA(ctx, cudaGetLastError());
     ctx->launches++;
@@ -1845,7 +1899,7 @@ int sxgpu_bank_read(sxgpu_bank *bank, void *d_cf32, sxgpu_stream stream)
     if (!d_cf32 || reinterpret_cast<uintptr_t>(d_cf32) % 8)
         return ctx->invalid("CF32 buffer must be 8-byte aligned device memory");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(bank->ctx, stream);
     const BankState &b = bank->st;
     if (bank_split_direct(ctx, b, d_cf32)) {
         // large banks: decisions by a thread per stream, then capture and RX conversion by CTAs that
@@ -1877,7 +1931,7 @@ int sxgpu_bank_write(sxgpu_bank *bank, const void *d_cf32, int flags, const long
     if (!d_cf32 || reinterpret_cast<uintptr_t>(d_cf32) % 8)
         return ctx->invalid("CF32 buffer must be 8-byte aligned device memory");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(bank->ctx, stream);
     const BankState &b = bank->st;
     if (bank_split_direct(ctx, b, d_cf32)) {
         SX_CUDA(ctx, (launch_bank_planned<kBankModeWrite, 4>(b, const_cast<char *>(static_cast<const char *>(d_cf32)), false, flags,
@@ -1906,7 +1960,7 @@ int sxgpu_bank_repeat(sxgpu_bank *bank, void *d_cf32, long long rx_time_offset_n
     if (!d_cf32 || reinterpret_cast<uintptr_t>(d_cf32) % 8)
         return ctx->invalid("CF32 buffer must be 8-byte aligned device memory");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(bank->ctx, stream);
     const BankState &b = bank->st;
     char *cf = static_cast<char *>(d_cf32);
     const bool ext = bank->external_capture;
@@ -1976,7 +2030,7 @@ int sxgpu_bank_repeat_begin(sxgpu_bank *bank, void *d_cf32, sxgpu_stream stream)
     if (!d_cf32)
         return ctx->invalid("null CF32 buffer");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(bank->ctx, stream);
     const size_t bytes = size_t(bank->st.nstreams) * bank->st.period * 8;
     const size_t window = std::min<size_t>(bytes, size_t(ctx->prop.accessPolicyMaxWindowSize));
     if (window > 0 && ctx->prop.persistingL2CacheMaxSize > 0) {
@@ -2005,7 +2059,7 @@ int sxgpu_bank_repeat_end(sxgpu_bank *bank, const void *d_cf32, long long rx_tim
     int rc = sxgpu_bank_write(bank, d_cf32, SX_HAS_TIME, nullptr, rx_time_offset_ns, stream);
     cudaStreamAttrValue attr = {};
     attr.accessPolicyWindow.num_bytes = 0; // lift the window for whatever the stream does next
-    if (cudaStreamSetAttribute(bank_stream(bank, stream), cudaStreamAttributeAccessPolicyWindow, &attr) != cudaSuccess)
+    if (cudaStreamSetAttribute(call_stream(bank->ctx, stream), cudaStreamAttributeAccessPolicyWindow, &attr) != cudaSuccess)
         cudaGetLastError();
     return rc;
 }
@@ -2027,7 +2081,7 @@ int sxgpu_bank_ingest(sxgpu_bank *bank, uint32_t first_stream, uint32_t nstreams
     // The capture slots of consecutive streams are contiguous: one copy, from wherever the frames
     // are (pinned or pageable host memory, or device memory).
     SX_CUDA(ctx, cudaMemcpyAsync(b.capture_stage + size_t(first_stream) * b.period * 8, i2s,
-                                 size_t(nstreams) * b.period * 8, cudaMemcpyDefault, bank_stream(bank, stream)));
+                                 size_t(nstreams) * b.period * 8, cudaMemcpyDefault, call_stream(bank->ctx, stream)));
     if (!classify_pointer(ctx, i2s).on_device)
         ctx->h2d_bytes += uint64_t(nstreams) * b.period * 8;
     bank->external_capture = true;
@@ -2049,7 +2103,7 @@ int sxgpu_bank_drain(sxgpu_bank *bank, uint32_t first_stream, uint32_t nstreams,
     HostPtrInfo di = classify_pointer(ctx, i2s);
     if (!di.device_alias || di.foreign_device || reinterpret_cast<uintptr_t>(di.device_alias) % 8)
         return ctx->invalid("drain destination must be device memory or pinned host memory, 8-byte aligned");
-    bank_drain_kernel<<<per_warp_grid(ctx, nstreams, 256), 256, 0, bank_stream(bank, stream)>>>(
+    bank_drain_kernel<<<per_warp_grid(ctx, nstreams, 256), 256, 0, call_stream(bank->ctx, stream)>>>(
         b, first_stream, nstreams, uint32_t(nframes), static_cast<char *>(di.device_alias));
     SX_CUDA(ctx, cudaGetLastError());
     ctx->launches++;
@@ -2077,7 +2131,7 @@ int sxgpu_bank_last_read(sxgpu_bank *bank, int32_t *h_ret, int32_t *h_flags, int
         return SXGPU_ERR_INVALID;
     sxgpu_ctx *ctx = bank->ctx;
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(bank->ctx, stream);
     SX_TRY(copy_out(bank, h_ret, bank->st.rx_ret, st));
     SX_TRY(copy_out(bank, h_flags, bank->st.rx_flags, st));
     SX_TRY(copy_out(bank, reinterpret_cast<long long *>(h_time_ns), bank->st.rx_time_ns, st));
@@ -2091,7 +2145,7 @@ int sxgpu_bank_last_write(sxgpu_bank *bank, int32_t *h_ret, sxgpu_stream stream)
         return SXGPU_ERR_INVALID;
     sxgpu_ctx *ctx = bank->ctx;
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(bank->ctx, stream);
     SX_TRY(copy_out(bank, h_ret, bank->st.tx_ret, st));
     SX_CUDA(ctx, cudaStreamSynchronize(st));
     return SXGPU_OK;
@@ -2104,7 +2158,7 @@ int sxgpu_bank_positions(sxgpu_bank *bank, int64_t *h_clock, int64_t *h_rx_posit
         return SXGPU_ERR_INVALID;
     sxgpu_ctx *ctx = bank->ctx;
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(bank->ctx, stream);
     SX_TRY(copy_out(bank, reinterpret_cast<long long *>(h_clock), bank->st.clock, st));
     SX_TRY(copy_out(bank, reinterpret_cast<long long *>(h_rx_position), bank->st.rx_position, st));
     SX_TRY(copy_out(bank, reinterpret_cast<long long *>(h_tx_position), bank->st.tx_position, st));
@@ -2122,7 +2176,7 @@ int sxgpu_bank_playback(sxgpu_bank *bank, uint32_t index, int64_t position, size
     if (index >= b.nstreams || position < 0 || nframes > b.ring)
         return ctx->invalid("playback window outside the stream's ring");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(bank->ctx, stream);
     if (nframes == 0)
         return SXGPU_OK;
     // The rings are stored time-major (sx_bank.cuh, ring_frame): gather the window on the device,
@@ -2147,8 +2201,9 @@ int sxgpu_bank_playback(sxgpu_bank *bank, uint32_t index, int64_t position, size
 
 struct sxgpu_iir {
     sxgpu_ctx *ctx = nullptr;
-    IirView view = {};        // the state in device memory and the float32 coefficients
-    double *powers = nullptr; // sxgpu_iir_apply_long's P_j = A^(2^j) (sx_iir.cuh), in device memory
+    IirView view = {};      // the state in device memory and the float32 coefficients
+    DevPtr<float> state;    // view.state
+    DevPtr<double> powers;  // sxgpu_iir_apply_long's P_j = A^(2^j) (sx_iir.cuh), in device memory
 };
 
 namespace {
@@ -2210,11 +2265,6 @@ size_t iir_state_bytes(const IirView &v)
     return size_t(v.k.nsections) * v.nstreams * 16; // two complex64 values per section and stream
 }
 
-cudaStream_t iir_stream(sxgpu_iir *f, sxgpu_stream stream)
-{
-    return stream ? static_cast<cudaStream_t>(stream) : f->ctx->stream;
-}
-
 // A stage of the filtered iteration: the filter's view, or no sections for a stage left out.
 IirView iir_stage(const sxgpu_iir *f)
 {
@@ -2254,81 +2304,34 @@ int sxgpu_iir_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t nsections, cons
         v.k.a2[q] = float(row[5]);
     }
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t bytes = iir_state_bytes(v);
-    void *state = nullptr;
-    cudaError_t e = cudaMalloc(&state, bytes);
-    if (e != cudaSuccess)
-        return ctx->fail(e, "cudaMalloc(filter state)");
-    e = cudaMemsetAsync(state, 0, bytes, ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-        cudaFree(state);
-        return ctx->fail(e, "cudaMemset(filter state)");
-    }
-    v.state = static_cast<float *>(state);
     const std::vector<double> chain = iir_power_chain(v.k);
-    void *powers = nullptr;
-    e = cudaMalloc(&powers, chain.size() * sizeof(double));
-    if (e == cudaSuccess)
-        e = cudaMemcpy(powers, chain.data(), chain.size() * sizeof(double), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-        cudaFree(powers);
-        cudaFree(state);
-        return ctx->fail(e, "filter tables");
-    }
-    sxgpu_iir *f = new sxgpu_iir();
+    std::unique_ptr<sxgpu_iir> f(new sxgpu_iir());
     f->ctx = ctx;
+    cudaError_t e = dev_upload(ctx, f->state, nullptr, iir_state_bytes(v));
+    if (e == cudaSuccess)
+        e = dev_upload(ctx, f->powers, chain.data(), chain.size() * sizeof(double));
+    v.state = f->state.get();
     f->view = v;
-    f->powers = static_cast<double *>(powers);
-    ctx->live_iirs++;
-    *out = f;
-    return SXGPU_OK;
+    return dsp_created(ctx, f, e, "cudaMalloc(filter)", out);
 }
 
 int sxgpu_iir_destroy(sxgpu_iir *f)
 {
-    if (!f)
-        return SXGPU_ERR_INVALID;
-    cudaSetDevice(f->ctx->device);
-    for (HostLane &lane : f->ctx->lanes) { // a resident converter would hold the device-wide sync up
-        std::lock_guard<std::mutex> lock(lane.mutex);
-        resident_stop(f->ctx, lane);
-    }
-    cudaDeviceSynchronize();
-    cudaFree(f->view.state);
-    cudaFree(f->powers);
-    f->ctx->live_iirs--;
-    delete f;
-    return SXGPU_OK;
+    return dsp_destroy(f);
 }
 
 int sxgpu_iir_set_state(sxgpu_iir *f, const void *h_zi, sxgpu_stream stream)
 {
     if (!f)
         return SXGPU_ERR_INVALID;
-    sxgpu_ctx *ctx = f->ctx;
-    SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = iir_stream(f, stream);
-    const size_t bytes = iir_state_bytes(f->view);
-    if (h_zi)
-        SX_CUDA(ctx, cudaMemcpyAsync(f->view.state, h_zi, bytes, cudaMemcpyHostToDevice, st));
-    else
-        SX_CUDA(ctx, cudaMemsetAsync(f->view.state, 0, bytes, st));
-    SX_CUDA(ctx, cudaStreamSynchronize(st));
-    return SXGPU_OK;
+    return state_copy(f->ctx, f->view.state, h_zi, iir_state_bytes(f->view), cudaMemcpyHostToDevice, stream);
 }
 
 int sxgpu_iir_get_state(sxgpu_iir *f, void *h_zf, sxgpu_stream stream)
 {
     if (!f || !h_zf)
         return SXGPU_ERR_INVALID;
-    sxgpu_ctx *ctx = f->ctx;
-    SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = iir_stream(f, stream);
-    SX_CUDA(ctx, cudaMemcpyAsync(h_zf, f->view.state, iir_state_bytes(f->view), cudaMemcpyDeviceToHost, st));
-    SX_CUDA(ctx, cudaStreamSynchronize(st));
-    return SXGPU_OK;
+    return state_copy(f->ctx, h_zf, f->view.state, iir_state_bytes(f->view), cudaMemcpyDeviceToHost, stream);
 }
 
 int sxgpu_iir_apply(sxgpu_iir *f, void *d_cf32, uint32_t period, sxgpu_stream stream)
@@ -2342,7 +2345,7 @@ int sxgpu_iir_apply(sxgpu_iir *f, void *d_cf32, uint32_t period, sxgpu_stream st
         return ctx->invalid("the period is 1 to 65536 frames");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const unsigned grid = unsigned((uint64_t(f->view.nstreams) + kIirStreamsPerCta - 1) / kIirStreamsPerCta);
-    iir_apply_kernel<<<grid, kIirThreads, 0, iir_stream(f, stream)>>>(f->view, static_cast<char *>(d_cf32), period, IirChunks{});
+    iir_apply_kernel<<<grid, kIirThreads, 0, call_stream(f->ctx, stream)>>>(f->view, static_cast<char *>(d_cf32), period, IirChunks{});
     SX_CUDA(ctx, cudaGetLastError());
     ctx->launches++;
     return SXGPU_OK;
@@ -2366,7 +2369,7 @@ int sxgpu_iir_apply_long(sxgpu_iir *f, void *d_cf32, uint64_t nframes, sxgpu_str
     if (ctas > uint64_t(INT32_MAX))
         return ctx->invalid("sxgpu_iir_apply_long: the block needs more CTAs than a grid holds");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = iir_stream(f, stream);
+    cudaStream_t st = call_stream(f->ctx, stream);
     char *cf32 = static_cast<char *>(d_cf32);
     if (chunks == 1) { // the whole block is chunk 0: exactly sxgpu_iir_apply
         const unsigned grid = unsigned((nstreams + kIirStreamsPerCta - 1) / kIirStreamsPerCta);
@@ -2383,7 +2386,7 @@ int sxgpu_iir_apply_long(sxgpu_iir *f, void *d_cf32, uint64_t nframes, sxgpu_str
     double *totals[2] = {reinterpret_cast<double *>(static_cast<char *>(scratch) + edge_bytes),
                          reinterpret_cast<double *>(static_cast<char *>(scratch) + edge_bytes + total_bytes)};
     IirChunks ch = {nframes, chunks, nstreams * (chunks - 1), len, static_cast<float *>(scratch)};
-    IirCarry a = {f->powers, ch, nullptr, totals[0], groups, sequences, 0};
+    IirCarry a = {f->powers.get(), ch, nullptr, totals[0], groups, sequences, 0};
     while ((1u << a.log2_len) < len)
         a.log2_len++;
     const unsigned carry_grid = unsigned((sequences * 16 + 127) / 128);
@@ -2436,7 +2439,7 @@ int sxgpu_bank_repeat_filtered(sxgpu_bank *bank, sxgpu_iir *pre, sxgpu_iir *post
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const BankState &b = bank->st;
     SX_CUDA(ctx, launch_bank_iir<kBankModeRepeat>(b, static_cast<char *>(d_cf32), bank->external_capture, SX_HAS_TIME, nullptr,
-                                                  rx_time_offset_ns, vpre, vpost, bank_stream(bank, stream), IdentityHook()));
+                                                  rx_time_offset_ns, vpre, vpost, call_stream(bank->ctx, stream), IdentityHook()));
     ctx->launches += 2;
     ctx->frames_rx += uint64_t(b.nstreams) * b.period;
     ctx->frames_tx += uint64_t(b.nstreams) * b.period;
@@ -2458,7 +2461,7 @@ int sxgpu_bank_read_filtered(sxgpu_bank *bank, sxgpu_iir *f, void *d_cf32, sxgpu
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const BankState &b = bank->st;
     SX_CUDA(ctx, launch_bank_iir<kBankModeRead>(b, static_cast<char *>(d_cf32), bank->external_capture, 0, nullptr, 0, v,
-                                                IirView{}, bank_stream(bank, stream), IdentityHook()));
+                                                IirView{}, call_stream(bank->ctx, stream), IdentityHook()));
     ctx->launches += 2;
     ctx->frames_rx += uint64_t(b.nstreams) * b.period;
     return SXGPU_OK;
@@ -2481,7 +2484,7 @@ int sxgpu_bank_write_filtered(sxgpu_bank *bank, sxgpu_iir *f, const void *d_cf32
     const BankState &b = bank->st;
     // the kernel only loads from the block in this mode
     SX_CUDA(ctx, launch_bank_iir<kBankModeWrite>(b, const_cast<char *>(static_cast<const char *>(d_cf32)), false, flags,
-                                                 d_time_ns, rx_time_offset_ns, v, IirView{}, bank_stream(bank, stream),
+                                                 d_time_ns, rx_time_offset_ns, v, IirView{}, call_stream(bank->ctx, stream),
                                                  IdentityHook()));
     ctx->launches += 2;
     ctx->frames_tx += uint64_t(b.nstreams) * b.period;
@@ -2505,8 +2508,8 @@ struct sxgpu_fir {
     sxgpu_ctx *ctx = nullptr;
     uint32_t nstreams = 0, up = 1, down = 1, g = 1, up1 = 1, down1 = 1, hp = 1, rows = 1;
     uint32_t phase = 0;       // frames fed so far mod down: the only state kept on the host
-    float4 *taps = nullptr;   // [up][rows] tap tables (FirCall::taps), device memory
-    float2 *hist = nullptr;   // [nstreams][hp - 1], device memory; NULL when hp == 1
+    DevPtr<float4> taps;      // [up][rows] tap tables (FirCall::taps), device memory
+    DevPtr<float2> hist;      // [nstreams][hp - 1], device memory; NULL when hp == 1
 };
 
 namespace {
@@ -2528,8 +2531,8 @@ uint64_t fir_outputs(const sxgpu_fir *f, uint32_t r, uint64_t nin)
 // False when the data kernel's grid would not fit.
 bool fir_call(const sxgpu_fir *f, uint64_t nin, uint64_t n, FirCall &a, int &block, size_t &smem)
 {
-    a.hist = f->hist;
-    a.taps = f->taps;
+    a.hist = f->hist.get();
+    a.taps = f->taps.get();
     a.nin = nin;
     a.nout = n;
     a.c0 = (uint64_t(f->phase) * f->up + f->down - 1) / f->down;
@@ -2563,11 +2566,6 @@ bool fir_call(const sxgpu_fir *f, uint64_t nin, uint64_t n, FirCall &a, int &blo
 size_t fir_hist_bytes(const sxgpu_fir *f)
 {
     return size_t(f->nstreams) * (f->hp - 1) * sizeof(float2);
-}
-
-cudaStream_t fir_stream(sxgpu_fir *f, sxgpu_stream stream)
-{
-    return stream ? static_cast<cudaStream_t>(stream) : f->ctx->stream;
 }
 
 } // namespace
@@ -2618,53 +2616,18 @@ int sxgpu_fir_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t ntaps, const do
             }
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t smem = std::min<size_t>(kFirWindowBytes, ctx->prop.sharedMemPerBlockOptin);
-    SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(fir_apply_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<1, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<2, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<4, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<1, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<2, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_fir_kernel<4, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    void *d_taps = nullptr, *d_hist = nullptr;
-    cudaError_t e = cudaMalloc(&d_taps, taps.size() * sizeof(float));
-    if (e == cudaSuccess)
-        e = cudaMemcpy(d_taps, taps.data(), taps.size() * sizeof(float), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && f->hp > 1) {
-        e = cudaMalloc(&d_hist, fir_hist_bytes(f.get()));
-        if (e == cudaSuccess)
-            e = cudaMemsetAsync(d_hist, 0, fir_hist_bytes(f.get()), ctx->stream);
-        if (e == cudaSuccess)
-            e = cudaStreamSynchronize(ctx->stream);
-    }
-    if (e != cudaSuccess) {
-        cudaFree(d_hist);
-        cudaFree(d_taps);
-        return ctx->fail(e, "cudaMalloc(FIR filter)");
-    }
-    f->taps = static_cast<float4 *>(d_taps);
-    f->hist = static_cast<float2 *>(d_hist);
-    ctx->live_firs++;
-    *out = f.release();
-    return SXGPU_OK;
+    for (auto kernel : {fir_apply_kernel<1>, fir_apply_kernel<2>, fir_apply_kernel<4>})
+        SX_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, bank_fir_allow_smem<NoNco>(smem));
+    cudaError_t e = dev_upload(ctx, f->taps, taps.data(), taps.size() * sizeof(float));
+    if (e == cudaSuccess && f->hp > 1)
+        e = dev_upload(ctx, f->hist, nullptr, fir_hist_bytes(f.get()));
+    return dsp_created(ctx, f, e, "cudaMalloc(FIR filter)", out);
 }
 
 int sxgpu_fir_destroy(sxgpu_fir *f)
 {
-    if (!f)
-        return SXGPU_ERR_INVALID;
-    cudaSetDevice(f->ctx->device);
-    for (HostLane &lane : f->ctx->lanes) { // a resident converter would hold the device-wide sync up
-        std::lock_guard<std::mutex> lock(lane.mutex);
-        resident_stop(f->ctx, lane);
-    }
-    cudaDeviceSynchronize();
-    cudaFree(f->hist);
-    cudaFree(f->taps);
-    f->ctx->live_firs--;
-    delete f;
-    return SXGPU_OK;
+    return dsp_destroy(f);
 }
 
 int sxgpu_fir_output_frames(sxgpu_fir *f, uint64_t nin, uint64_t *nout)
@@ -2706,7 +2669,7 @@ int sxgpu_fir_apply(sxgpu_fir *f, const void *d_in, uint64_t nin, void *d_out, u
     a.in = static_cast<const float2 *>(d_in);
     a.out = static_cast<float2 *>(d_out);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = fir_stream(f, stream);
+    cudaStream_t st = call_stream(f->ctx, stream);
     int launches = 0;
     if (n) {
         const unsigned grid = unsigned(nstreams * a.chunks);
@@ -2731,105 +2694,13 @@ int sxgpu_fir_apply(sxgpu_fir *f, const void *d_in, uint64_t nin, void *d_out, u
     return SXGPU_OK;
 }
 
-// Why a FIR half's filter is refused (nullptr: it is not).
-static const char *bank_fir_invalid(const sxgpu_bank *bank, const sxgpu_fir *f)
-{
-    if (!f || f->ctx != bank->ctx)
-        return "the FIR filter is NULL or belongs to another context";
-    if (f->nstreams != bank->st.nstreams)
-        return "a filter must have as many streams as the bank";
-    return nullptr;
-}
-
-int sxgpu_bank_read_fir(sxgpu_bank *bank, sxgpu_fir *f, void *d_out, uint64_t *nout, sxgpu_stream stream)
-{
-    if (!bank)
-        return SXGPU_ERR_INVALID;
-    sxgpu_ctx *ctx = bank->ctx;
-    if (const char *why = bank_fir_invalid(bank, f))
-        return ctx->invalid(why);
-    if (!d_out || reinterpret_cast<uintptr_t>(d_out) % 8)
-        return ctx->invalid("sxgpu_bank_read_fir: the output must be 8-byte aligned device memory");
-    const BankState &b = bank->st;
-    const uint64_t n = fir_outputs(f, f->phase, b.period);
-    if (n > UINT64_MAX / 8 / b.nstreams)
-        return ctx->invalid("sxgpu_bank_read_fir: nstreams * nout * 8 bytes overflows 64 bits");
-    FirCall a = {};
-    int block = 0;
-    size_t smem = 0;
-    if (!fir_call(f, b.period, n, a, block, smem))
-        return ctx->invalid("sxgpu_bank_read_fir: the period needs more CTAs than a grid holds");
-    a.out = static_cast<float2 *>(d_out);
-    SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
-    const bool ext = bank->external_capture;
-    SX_CUDA(ctx, launch_bank_plan<kBankModeRead>(b, nullptr, 0, nullptr, 0, st));
-    int launches = 1;
-    if (n) {
-        SX_CUDA(ctx, launch_bank_fir<kBankModeRead>(b, a, block, smem, ext, st));
-        launches++;
-    }
-    if (f->hp > 1 || !ext) {
-        bank_fir_read_tail_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(b, a, ext);
-        SX_CUDA(ctx, cudaGetLastError());
-        launches++;
-    }
-    ctx->launches += launches;
-    ctx->frames_rx += uint64_t(b.nstreams) * b.period;
-    f->phase = uint32_t((f->phase + b.period % f->down) % f->down);
-    if (nout)
-        *nout = n;
-    return SXGPU_OK;
-}
-
-int sxgpu_bank_write_fir(sxgpu_bank *bank, sxgpu_fir *f, const void *d_in, uint64_t nin, int flags,
-                         const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream)
-{
-    if (!bank)
-        return SXGPU_ERR_INVALID;
-    sxgpu_ctx *ctx = bank->ctx;
-    if (const char *why = bank_fir_invalid(bank, f))
-        return ctx->invalid(why);
-    if (!d_in || reinterpret_cast<uintptr_t>(d_in) % 8)
-        return ctx->invalid("sxgpu_bank_write_fir: the input must be 8-byte aligned device memory");
-    const BankState &b = bank->st;
-    if (nin > UINT64_MAX / 8 / b.nstreams)
-        return ctx->invalid("sxgpu_bank_write_fir: nstreams * nin * 8 bytes overflows 64 bits");
-    if (fir_outputs(f, f->phase, nin) != b.period)
-        return ctx->invalid("sxgpu_bank_write_fir: the filter must emit exactly one period from nin frames");
-    FirCall a = {};
-    int block = 0;
-    size_t smem = 0;
-    if (!fir_call(f, nin, b.period, a, block, smem))
-        return ctx->invalid("sxgpu_bank_write_fir: the block needs more CTAs than a grid holds");
-    a.in = static_cast<const float2 *>(d_in);
-    SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
-    SX_CUDA(ctx, launch_bank_plan<kBankModeWrite>(b, nullptr, flags, d_time_ns, rx_time_offset_ns, st));
-    SX_CUDA(ctx, launch_bank_fir<kBankModeWrite>(b, a, block, smem, false, st));
-    int launches = 2;
-    if (f->hp > 1) {
-        fir_history_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(a);
-        SX_CUDA(ctx, cudaGetLastError());
-        launches++;
-    }
-    ctx->launches += launches;
-    ctx->frames_tx += uint64_t(b.nstreams) * b.period;
-    f->phase = uint32_t((f->phase + nin % f->down) % f->down);
-    return SXGPU_OK;
-}
-
 int sxgpu_fir_get_state(sxgpu_fir *f, void *h_hist, uint32_t *phase, sxgpu_stream stream)
 {
     if (!f)
         return SXGPU_ERR_INVALID;
     sxgpu_ctx *ctx = f->ctx;
-    if (h_hist && f->hp > 1) {
-        SX_CUDA(ctx, cudaSetDevice(ctx->device));
-        cudaStream_t st = fir_stream(f, stream);
-        SX_CUDA(ctx, cudaMemcpyAsync(h_hist, f->hist, fir_hist_bytes(f), cudaMemcpyDeviceToHost, st));
-        SX_CUDA(ctx, cudaStreamSynchronize(st));
-    }
+    if (h_hist && f->hp > 1)
+        SX_TRY(state_copy(ctx, h_hist, f->hist.get(), fir_hist_bytes(f), cudaMemcpyDeviceToHost, stream));
     if (phase)
         *phase = f->phase;
     return SXGPU_OK;
@@ -2842,15 +2713,8 @@ int sxgpu_fir_set_state(sxgpu_fir *f, const void *h_hist, uint32_t phase, sxgpu_
     sxgpu_ctx *ctx = f->ctx;
     if (phase >= f->down)
         return ctx->invalid("sxgpu_fir_set_state: the phase is below down");
-    if (f->hp > 1) {
-        SX_CUDA(ctx, cudaSetDevice(ctx->device));
-        cudaStream_t st = fir_stream(f, stream);
-        if (h_hist)
-            SX_CUDA(ctx, cudaMemcpyAsync(f->hist, h_hist, fir_hist_bytes(f), cudaMemcpyHostToDevice, st));
-        else
-            SX_CUDA(ctx, cudaMemsetAsync(f->hist, 0, fir_hist_bytes(f), st));
-        SX_CUDA(ctx, cudaStreamSynchronize(st));
-    }
+    if (f->hp > 1)
+        SX_TRY(state_copy(ctx, f->hist.get(), h_hist, fir_hist_bytes(f), cudaMemcpyHostToDevice, stream));
     f->phase = phase;
     return SXGPU_OK;
 }
@@ -2861,7 +2725,7 @@ int sxgpu_fir_set_state(sxgpu_fir *f, const void *h_hist, uint32_t phase, sxgpu_
 struct sxgpu_nco {
     sxgpu_ctx *ctx = nullptr;
     uint32_t nstreams = 0;
-    void *mem = nullptr; // one allocation: the tables, then the phases, then the increments
+    DevPtr<char> mem; // one allocation: the tables, then the phases, then the increments
     NcoView view = {};
 };
 
@@ -2892,11 +2756,6 @@ std::vector<float2> nco_tables()
     return tab;
 }
 
-cudaStream_t nco_stream(sxgpu_nco *n, sxgpu_stream stream)
-{
-    return stream ? static_cast<cudaStream_t>(stream) : n->ctx->stream;
-}
-
 } // namespace
 
 extern "C" {
@@ -2914,53 +2773,23 @@ int sxgpu_nco_create(sxgpu_ctx *ctx, uint32_t nstreams, const double *freq, sxgp
     const std::vector<float2> tab = nco_tables();
     const size_t tab_bytes = tab.size() * sizeof(float2), state_bytes = size_t(nstreams) * sizeof(uint32_t);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t smem = std::min<size_t>(kFirWindowBytes, ctx->prop.sharedMemPerBlockOptin);
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<1, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<2, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<4, kBankModeRead>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<1, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<2, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    SX_CUDA(ctx, cudaFuncSetAttribute(bank_nco_fir_kernel<4, kBankModeWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+    SX_CUDA(ctx, bank_fir_allow_smem<NcoView>(std::min<size_t>(kFirWindowBytes, ctx->prop.sharedMemPerBlockOptin)));
     std::unique_ptr<sxgpu_nco> n(new sxgpu_nco());
     n->ctx = ctx;
     n->nstreams = nstreams;
-    cudaError_t e = cudaMalloc(&n->mem, tab_bytes + 2 * state_bytes);
-    if (e != cudaSuccess)
-        return ctx->fail(e, "cudaMalloc(oscillator)");
-    char *mem = static_cast<char *>(n->mem);
-    n->view.tab = reinterpret_cast<const float2 *>(mem);
-    n->view.phase = reinterpret_cast<uint32_t *>(mem + tab_bytes);
-    n->view.inc = reinterpret_cast<uint32_t *>(mem + tab_bytes + state_bytes);
-    e = cudaMemcpy(mem, tab.data(), tab_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess)
-        e = cudaMemcpy(n->view.inc, inc.data(), state_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess)
-        e = cudaMemsetAsync(n->view.phase, 0, state_bytes, ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-        cudaFree(n->mem);
-        return ctx->fail(e, "cudaMemcpy(oscillator)");
-    }
-    ctx->live_ncos++;
-    *out = n.release();
-    return SXGPU_OK;
+    std::vector<char> img(tab_bytes + 2 * state_bytes, 0); // the phases start at 0
+    std::memcpy(img.data(), tab.data(), tab_bytes);
+    std::memcpy(img.data() + tab_bytes + state_bytes, inc.data(), state_bytes);
+    const cudaError_t e = dev_upload(ctx, n->mem, img.data(), img.size());
+    char *mem = n->mem.get();
+    n->view = NcoView{reinterpret_cast<const float2 *>(mem), reinterpret_cast<uint32_t *>(mem + tab_bytes),
+                      reinterpret_cast<uint32_t *>(mem + tab_bytes + state_bytes)};
+    return dsp_created(ctx, n, e, "cudaMalloc(oscillator)", out);
 }
 
 int sxgpu_nco_destroy(sxgpu_nco *n)
 {
-    if (!n)
-        return SXGPU_ERR_INVALID;
-    cudaSetDevice(n->ctx->device);
-    for (HostLane &lane : n->ctx->lanes) { // a resident converter would hold the device-wide sync up
-        std::lock_guard<std::mutex> lock(lane.mutex);
-        resident_stop(n->ctx, lane);
-    }
-    cudaDeviceSynchronize();
-    cudaFree(n->mem);
-    n->ctx->live_ncos--;
-    delete n;
-    return SXGPU_OK;
+    return dsp_destroy(n);
 }
 
 int sxgpu_nco_apply(sxgpu_nco *n, void *d_cf32, uint64_t nframes, sxgpu_stream stream)
@@ -2978,7 +2807,7 @@ int sxgpu_nco_apply(sxgpu_nco *n, void *d_cf32, uint64_t nframes, sxgpu_stream s
     if (ctas > uint64_t(INT32_MAX))
         return ctx->invalid("sxgpu_nco_apply: the block needs more CTAs than a grid holds");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = nco_stream(n, stream);
+    cudaStream_t st = call_stream(n->ctx, stream);
     nco_apply_kernel<<<unsigned(ctas), kNcoThreads, 0, st>>>(n->view, static_cast<float2 *>(d_cf32), nframes, total,
                                                              1.0 / double(nframes));
     SX_CUDA(ctx, cudaGetLastError());
@@ -2997,7 +2826,7 @@ int sxgpu_nco_set_frequencies(sxgpu_nco *n, const double *h_freq, sxgpu_stream s
     if (const char *why = nco_increments(n->nstreams, h_freq, inc))
         return ctx->invalid(why);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = nco_stream(n, stream);
+    cudaStream_t st = call_stream(n->ctx, stream);
     SX_CUDA(ctx, cudaMemcpyAsync(n->view.inc, inc.data(), inc.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     SX_CUDA(ctx, cudaStreamSynchronize(st));
     return SXGPU_OK;
@@ -3009,7 +2838,7 @@ int sxgpu_nco_get_state(sxgpu_nco *n, uint32_t *h_phase, uint32_t *h_inc, sxgpu_
         return SXGPU_ERR_INVALID;
     sxgpu_ctx *ctx = n->ctx;
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = nco_stream(n, stream);
+    cudaStream_t st = call_stream(n->ctx, stream);
     const size_t bytes = size_t(n->nstreams) * sizeof(uint32_t);
     if (h_phase)
         SX_CUDA(ctx, cudaMemcpyAsync(h_phase, n->view.phase, bytes, cudaMemcpyDeviceToHost, st));
@@ -3025,7 +2854,7 @@ int sxgpu_nco_set_state(sxgpu_nco *n, const uint32_t *h_phase, const uint32_t *h
         return SXGPU_ERR_INVALID;
     sxgpu_ctx *ctx = n->ctx;
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = nco_stream(n, stream);
+    cudaStream_t st = call_stream(n->ctx, stream);
     const size_t bytes = size_t(n->nstreams) * sizeof(uint32_t);
     if (h_phase)
         SX_CUDA(ctx, cudaMemcpyAsync(n->view.phase, h_phase, bytes, cudaMemcpyHostToDevice, st));
@@ -3035,8 +2864,23 @@ int sxgpu_nco_set_state(sxgpu_nco *n, const uint32_t *h_phase, const uint32_t *h
     return SXGPU_OK;
 }
 
+// ---- the stream bank's FIR halves, with or without an oscillator (sx_bank.cuh) -------------------
+} // extern "C"
+
+namespace {
+
+// Why a FIR half's filter is refused (nullptr: it is not).
+const char *bank_fir_invalid(const sxgpu_bank *bank, const sxgpu_fir *f)
+{
+    if (!f || f->ctx != bank->ctx)
+        return "the FIR filter is NULL or belongs to another context";
+    if (f->nstreams != bank->st.nstreams)
+        return "a filter must have as many streams as the bank";
+    return nullptr;
+}
+
 // Why a half's oscillator is refused (nullptr: it is not).
-static const char *bank_nco_invalid(const sxgpu_bank *bank, const sxgpu_nco *n)
+const char *bank_nco_invalid(const sxgpu_bank *bank, const sxgpu_nco *n)
 {
     if (!n || n->ctx != bank->ctx)
         return "the oscillator is NULL or belongs to another context";
@@ -3045,39 +2889,40 @@ static const char *bank_nco_invalid(const sxgpu_bank *bank, const sxgpu_nco *n)
     return nullptr;
 }
 
-int sxgpu_bank_read_ddc(sxgpu_bank *bank, sxgpu_nco *nco, sxgpu_fir *f, void *d_out, uint64_t *nout, sxgpu_stream stream)
+// sxgpu_bank_read_fir (nco: NoNco) and sxgpu_bank_read_ddc (nco: the oscillator's NcoView), after
+// the entry point `name` has checked the filter and the oscillator.
+template <class Nco>
+int bank_read_fir(sxgpu_bank *bank, sxgpu_fir *f, const Nco &nco, void *d_out, uint64_t *nout, sxgpu_stream stream,
+                  const char *name)
 {
-    if (!bank)
-        return SXGPU_ERR_INVALID;
     sxgpu_ctx *ctx = bank->ctx;
-    if (const char *why = bank_nco_invalid(bank, nco))
-        return ctx->invalid(why);
-    if (const char *why = bank_fir_invalid(bank, f))
-        return ctx->invalid(why);
+    auto refuse = [&](const char *why) { return ctx->invalid((std::string(name) + ": " + why).c_str()); };
     if (!d_out || reinterpret_cast<uintptr_t>(d_out) % 8)
-        return ctx->invalid("sxgpu_bank_read_ddc: the output must be 8-byte aligned device memory");
+        return refuse("the output must be 8-byte aligned device memory");
     const BankState &b = bank->st;
     const uint64_t n = fir_outputs(f, f->phase, b.period);
     if (n > UINT64_MAX / 8 / b.nstreams)
-        return ctx->invalid("sxgpu_bank_read_ddc: nstreams * nout * 8 bytes overflows 64 bits");
+        return refuse("nstreams * nout * 8 bytes overflows 64 bits");
     FirCall a = {};
     int block = 0;
     size_t smem = 0;
     if (!fir_call(f, b.period, n, a, block, smem))
-        return ctx->invalid("sxgpu_bank_read_ddc: the period needs more CTAs than a grid holds");
+        return refuse("the period needs more CTAs than a grid holds");
     a.out = static_cast<float2 *>(d_out);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
+    cudaStream_t st = call_stream(ctx, stream);
     const bool ext = bank->external_capture;
     SX_CUDA(ctx, launch_bank_plan<kBankModeRead>(b, nullptr, 0, nullptr, 0, st));
     int launches = 1;
     if (n) {
-        SX_CUDA(ctx, launch_bank_nco_fir<kBankModeRead>(b, a, block, smem, ext, nco->view, st));
+        SX_CUDA(ctx, launch_bank_fir<kBankModeRead>(b, a, block, smem, ext, nco, st));
         launches++;
     }
-    bank_nco_fir_read_tail_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(b, a, ext, nco->view);
-    SX_CUDA(ctx, cudaGetLastError());
-    launches++;
+    if (f->hp > 1 || !ext || !std::is_same<Nco, NoNco>::value) { // with an oscillator the tail advances the phases
+        bank_fir_read_tail_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(b, a, ext, nco);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
     ctx->launches += launches;
     ctx->frames_rx += uint64_t(b.nstreams) * b.period;
     f->phase = uint32_t((f->phase + b.period % f->down) % f->down);
@@ -3086,39 +2931,87 @@ int sxgpu_bank_read_ddc(sxgpu_bank *bank, sxgpu_nco *nco, sxgpu_fir *f, void *d_
     return SXGPU_OK;
 }
 
+// sxgpu_bank_write_fir (nco: NoNco) and sxgpu_bank_write_duc (nco: the oscillator's NcoView), after
+// the entry point `name` has checked the filter and the oscillator.
+template <class Nco>
+int bank_write_fir(sxgpu_bank *bank, sxgpu_fir *f, const Nco &nco, const void *d_in, uint64_t nin, int flags,
+                   const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream, const char *name)
+{
+    sxgpu_ctx *ctx = bank->ctx;
+    auto refuse = [&](const char *why) { return ctx->invalid((std::string(name) + ": " + why).c_str()); };
+    if (!d_in || reinterpret_cast<uintptr_t>(d_in) % 8)
+        return refuse("the input must be 8-byte aligned device memory");
+    const BankState &b = bank->st;
+    if (nin > UINT64_MAX / 8 / b.nstreams)
+        return refuse("nstreams * nin * 8 bytes overflows 64 bits");
+    if (fir_outputs(f, f->phase, nin) != b.period)
+        return refuse("the filter must emit exactly one period from nin frames");
+    FirCall a = {};
+    int block = 0;
+    size_t smem = 0;
+    if (!fir_call(f, nin, b.period, a, block, smem))
+        return refuse("the block needs more CTAs than a grid holds");
+    a.in = static_cast<const float2 *>(d_in);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = call_stream(ctx, stream);
+    SX_CUDA(ctx, launch_bank_plan<kBankModeWrite>(b, nullptr, flags, d_time_ns, rx_time_offset_ns, st));
+    SX_CUDA(ctx, launch_bank_fir<kBankModeWrite>(b, a, block, smem, false, nco, st));
+    int launches = 2;
+    if (f->hp > 1 || !std::is_same<Nco, NoNco>::value) { // with an oscillator the tail advances the phases
+        fir_history_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(a, nco, b.period);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
+    ctx->launches += launches;
+    ctx->frames_tx += uint64_t(b.nstreams) * b.period;
+    f->phase = uint32_t((f->phase + nin % f->down) % f->down);
+    return SXGPU_OK;
+}
+
+} // namespace
+
+extern "C" {
+
+int sxgpu_bank_read_fir(sxgpu_bank *bank, sxgpu_fir *f, void *d_out, uint64_t *nout, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    if (const char *why = bank_fir_invalid(bank, f))
+        return bank->ctx->invalid(why);
+    return bank_read_fir(bank, f, NoNco{}, d_out, nout, stream, "sxgpu_bank_read_fir");
+}
+
+int sxgpu_bank_read_ddc(sxgpu_bank *bank, sxgpu_nco *nco, sxgpu_fir *f, void *d_out, uint64_t *nout, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    if (const char *why = bank_nco_invalid(bank, nco))
+        return bank->ctx->invalid(why);
+    if (const char *why = bank_fir_invalid(bank, f))
+        return bank->ctx->invalid(why);
+    return bank_read_fir(bank, f, nco->view, d_out, nout, stream, "sxgpu_bank_read_ddc");
+}
+
+int sxgpu_bank_write_fir(sxgpu_bank *bank, sxgpu_fir *f, const void *d_in, uint64_t nin, int flags,
+                         const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream)
+{
+    if (!bank)
+        return SXGPU_ERR_INVALID;
+    if (const char *why = bank_fir_invalid(bank, f))
+        return bank->ctx->invalid(why);
+    return bank_write_fir(bank, f, NoNco{}, d_in, nin, flags, d_time_ns, rx_time_offset_ns, stream, "sxgpu_bank_write_fir");
+}
+
 int sxgpu_bank_write_duc(sxgpu_bank *bank, sxgpu_fir *f, sxgpu_nco *nco, const void *d_in, uint64_t nin, int flags,
                          const long long *d_time_ns, long long rx_time_offset_ns, sxgpu_stream stream)
 {
     if (!bank)
         return SXGPU_ERR_INVALID;
-    sxgpu_ctx *ctx = bank->ctx;
     if (const char *why = bank_fir_invalid(bank, f))
-        return ctx->invalid(why);
+        return bank->ctx->invalid(why);
     if (const char *why = bank_nco_invalid(bank, nco))
-        return ctx->invalid(why);
-    if (!d_in || reinterpret_cast<uintptr_t>(d_in) % 8)
-        return ctx->invalid("sxgpu_bank_write_duc: the input must be 8-byte aligned device memory");
-    const BankState &b = bank->st;
-    if (nin > UINT64_MAX / 8 / b.nstreams)
-        return ctx->invalid("sxgpu_bank_write_duc: nstreams * nin * 8 bytes overflows 64 bits");
-    if (fir_outputs(f, f->phase, nin) != b.period)
-        return ctx->invalid("sxgpu_bank_write_duc: the filter must emit exactly one period from nin frames");
-    FirCall a = {};
-    int block = 0;
-    size_t smem = 0;
-    if (!fir_call(f, nin, b.period, a, block, smem))
-        return ctx->invalid("sxgpu_bank_write_duc: the block needs more CTAs than a grid holds");
-    a.in = static_cast<const float2 *>(d_in);
-    SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = bank_stream(bank, stream);
-    SX_CUDA(ctx, launch_bank_plan<kBankModeWrite>(b, nullptr, flags, d_time_ns, rx_time_offset_ns, st));
-    SX_CUDA(ctx, launch_bank_nco_fir<kBankModeWrite>(b, a, block, smem, false, nco->view, st));
-    bank_nco_fir_write_tail_kernel<<<b.nstreams, kFirHistoryThreads, (f->hp - 1) * sizeof(float2), st>>>(a, nco->view, b.period);
-    SX_CUDA(ctx, cudaGetLastError());
-    ctx->launches += 3;
-    ctx->frames_tx += uint64_t(b.nstreams) * b.period;
-    f->phase = uint32_t((f->phase + nin % f->down) % f->down);
-    return SXGPU_OK;
+        return bank->ctx->invalid(why);
+    return bank_write_fir(bank, f, nco->view, d_in, nin, flags, d_time_ns, rx_time_offset_ns, stream, "sxgpu_bank_write_duc");
 }
 
 // ---- polyphase DFT channelizers (sx_chan.cuh) -------------------------------------------------
@@ -3128,8 +3021,8 @@ struct sxgpu_chan {
     sxgpu_ctx *ctx = nullptr;
     uint32_t nstreams = 0, m = 2, log2m = 1, down = 1, ntaps = 1;
     uint32_t phase = 0;     // frames fed so far mod M: the only state kept on the host
-    void *mem = nullptr;    // one allocation: the twiddles [1024], then the taps [ntaps]
-    float2 *hist = nullptr; // [nstreams][ntaps - 1], device memory; NULL when ntaps == 1
+    DevPtr<float2> mem;     // one allocation: the twiddles [1024], then the taps [ntaps]
+    DevPtr<float2> hist;    // [nstreams][ntaps - 1], device memory; NULL when ntaps == 1
 };
 
 namespace {
@@ -3149,9 +3042,9 @@ uint64_t chan_outputs(const sxgpu_chan *c, uint32_t r, uint64_t nin)
 bool chan_call(const sxgpu_chan *c, uint64_t nin, uint64_t n, ChanCall &a, uint32_t &threads, size_t &smem)
 {
     const uint32_t M = c->m, D = c->down;
-    a.hist = c->hist;
-    a.tw = static_cast<const float2 *>(c->mem);
-    a.taps = reinterpret_cast<const float *>(static_cast<const float2 *>(c->mem) + kNcoTableSize);
+    a.hist = c->hist.get();
+    a.tw = c->mem.get();
+    a.taps = reinterpret_cast<const float *>(c->mem.get() + kNcoTableSize);
     a.nin = nin;
     a.nout = n;
     a.m = M;
@@ -3186,11 +3079,6 @@ bool chan_call(const sxgpu_chan *c, uint64_t nin, uint64_t n, ChanCall &a, uint3
 size_t chan_hist_bytes(const sxgpu_chan *c)
 {
     return size_t(c->nstreams) * (c->ntaps - 1) * sizeof(float2);
-}
-
-cudaStream_t chan_stream(sxgpu_chan *c, sxgpu_stream stream)
-{
-    return stream ? static_cast<cudaStream_t>(stream) : c->ctx->stream;
 }
 
 } // namespace
@@ -3231,50 +3119,23 @@ int sxgpu_chan_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t channels, uint
     for (uint32_t i = 0; i < ntaps; i++)
         taps[i] = float(h[i]);
     const size_t tw_bytes = tw.size() * sizeof(float2), taps_bytes = taps.size() * sizeof(float);
+    std::vector<char> img(tw_bytes + taps_bytes);
+    std::memcpy(img.data(), tw.data(), tw_bytes);
+    std::memcpy(img.data() + tw_bytes, taps.data(), taps_bytes);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
     SX_CUDA(ctx, cudaFuncSetAttribute(chan_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       int(std::min<size_t>(kChanSmemBytes, ctx->prop.sharedMemPerBlockOptin))));
-    SX_CUDA(ctx, cudaFuncSetAttribute(fir_history_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    SX_CUDA(ctx, cudaFuncSetAttribute(fir_history_kernel<NoNco>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       int((kChanMaxTaps - 1) * sizeof(float2))));
-    cudaError_t e = cudaMalloc(&c->mem, tw_bytes + taps_bytes);
-    if (e == cudaSuccess)
-        e = cudaMemcpy(c->mem, tw.data(), tw_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess)
-        e = cudaMemcpy(static_cast<char *>(c->mem) + tw_bytes, taps.data(), taps_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && ntaps > 1) {
-        void *d_hist = nullptr;
-        e = cudaMalloc(&d_hist, chan_hist_bytes(c.get()));
-        c->hist = static_cast<float2 *>(d_hist);
-        if (e == cudaSuccess)
-            e = cudaMemsetAsync(d_hist, 0, chan_hist_bytes(c.get()), ctx->stream);
-        if (e == cudaSuccess)
-            e = cudaStreamSynchronize(ctx->stream);
-    }
-    if (e != cudaSuccess) {
-        cudaFree(c->hist);
-        cudaFree(c->mem);
-        return ctx->fail(e, "cudaMalloc(channelizer)");
-    }
-    ctx->live_chans++;
-    *out = c.release();
-    return SXGPU_OK;
+    cudaError_t e = dev_upload(ctx, c->mem, img.data(), img.size());
+    if (e == cudaSuccess && ntaps > 1)
+        e = dev_upload(ctx, c->hist, nullptr, chan_hist_bytes(c.get()));
+    return dsp_created(ctx, c, e, "cudaMalloc(channelizer)", out);
 }
 
 int sxgpu_chan_destroy(sxgpu_chan *c)
 {
-    if (!c)
-        return SXGPU_ERR_INVALID;
-    cudaSetDevice(c->ctx->device);
-    for (HostLane &lane : c->ctx->lanes) { // a resident converter would hold the device-wide sync up
-        std::lock_guard<std::mutex> lock(lane.mutex);
-        resident_stop(c->ctx, lane);
-    }
-    cudaDeviceSynchronize();
-    cudaFree(c->hist);
-    cudaFree(c->mem);
-    c->ctx->live_chans--;
-    delete c;
-    return SXGPU_OK;
+    return dsp_destroy(c);
 }
 
 int sxgpu_chan_output_frames(sxgpu_chan *c, uint64_t nin, uint64_t *nout)
@@ -3313,7 +3174,7 @@ int sxgpu_chan_apply(sxgpu_chan *c, const void *d_in, uint64_t nin, void *d_out,
     a.in = static_cast<const float2 *>(d_in);
     a.out = static_cast<float2 *>(d_out);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = chan_stream(c, stream);
+    cudaStream_t st = call_stream(c->ctx, stream);
     int launches = 0;
     if (n) {
         chan_apply_kernel<<<unsigned(nstreams * a.tiles), threads, smem, st>>>(a);
@@ -3324,7 +3185,7 @@ int sxgpu_chan_apply(sxgpu_chan *c, const void *d_in, uint64_t nin, void *d_out,
         // fir_history_kernel keeps the last hp - 1 frames of buf = hist ++ in: the same history.
         FirCall hc = {};
         hc.in = a.in;
-        hc.hist = c->hist;
+        hc.hist = c->hist.get();
         hc.nin = nin;
         hc.hp = c->ntaps;
         fir_history_kernel<<<unsigned(nstreams), kFirHistoryThreads, (c->ntaps - 1) * sizeof(float2), st>>>(hc);
@@ -3343,12 +3204,8 @@ int sxgpu_chan_get_state(sxgpu_chan *c, void *h_hist, uint32_t *phase, sxgpu_str
     if (!c)
         return SXGPU_ERR_INVALID;
     sxgpu_ctx *ctx = c->ctx;
-    if (h_hist && c->ntaps > 1) {
-        SX_CUDA(ctx, cudaSetDevice(ctx->device));
-        cudaStream_t st = chan_stream(c, stream);
-        SX_CUDA(ctx, cudaMemcpyAsync(h_hist, c->hist, chan_hist_bytes(c), cudaMemcpyDeviceToHost, st));
-        SX_CUDA(ctx, cudaStreamSynchronize(st));
-    }
+    if (h_hist && c->ntaps > 1)
+        SX_TRY(state_copy(ctx, h_hist, c->hist.get(), chan_hist_bytes(c), cudaMemcpyDeviceToHost, stream));
     if (phase)
         *phase = c->phase;
     return SXGPU_OK;
@@ -3361,15 +3218,8 @@ int sxgpu_chan_set_state(sxgpu_chan *c, const void *h_hist, uint32_t phase, sxgp
     sxgpu_ctx *ctx = c->ctx;
     if (phase >= c->m)
         return ctx->invalid("sxgpu_chan_set_state: the phase is below the channel count");
-    if (c->ntaps > 1) {
-        SX_CUDA(ctx, cudaSetDevice(ctx->device));
-        cudaStream_t st = chan_stream(c, stream);
-        if (h_hist)
-            SX_CUDA(ctx, cudaMemcpyAsync(c->hist, h_hist, chan_hist_bytes(c), cudaMemcpyHostToDevice, st));
-        else
-            SX_CUDA(ctx, cudaMemsetAsync(c->hist, 0, chan_hist_bytes(c), st));
-        SX_CUDA(ctx, cudaStreamSynchronize(st));
-    }
+    if (c->ntaps > 1)
+        SX_TRY(state_copy(ctx, c->hist.get(), h_hist, chan_hist_bytes(c), cudaMemcpyHostToDevice, stream));
     c->phase = phase;
     return SXGPU_OK;
 }
@@ -3386,7 +3236,7 @@ int sxgpu_fill_silence(sxgpu_ctx *ctx, void *d_i2s, size_t offset, size_t length
     if (frames_overflow(offset, length))
         return ctx->invalid("offset + length overflows");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st = call_stream(ctx, stream);
     int block = 256;
     uint64_t ctas = (length + block - 1) / block;
     int grid = int(std::min<uint64_t>(ctas, uint64_t(ctx->prop.multiProcessorCount) * 8));
@@ -3486,7 +3336,7 @@ int sxgpu_stats_words(sxgpu_ctx *ctx, const void *d_words, size_t nwords, uint64
         return ctx->invalid("word buffer must be 4-byte aligned");
     std::lock_guard<std::mutex> lock(ctx->stats_mutex);
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st = call_stream(ctx, stream);
     SX_CUDA(ctx, cudaMemsetAsync(ctx->d_stats, 0, sizeof(StatsAcc), st));
     int block = 256;
     uint64_t ctas = (nwords + block - 1) / block;
@@ -3517,7 +3367,7 @@ int sxgpu_synth_frames(sxgpu_ctx *ctx, void *d_i2s, uint64_t first_frame, size_t
     if (!d_i2s || reinterpret_cast<uintptr_t>(d_i2s) % 8)
         return ctx->invalid("I2S buffer must be 8-byte aligned");
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st = call_stream(ctx, stream);
     int block = 256;
     uint64_t ctas = (nframes + block - 1) / block;
     int grid = int(std::min<uint64_t>(ctas, uint64_t(ctx->prop.multiProcessorCount) * 8));
@@ -3581,7 +3431,7 @@ int sxgpu_memcpy_h2d(sxgpu_ctx *ctx, void *d_dst, const void *h_src, size_t byte
     if (!ctx)
         return SXGPU_ERR_INVALID;
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st = call_stream(ctx, stream);
     SX_CUDA(ctx, cudaMemcpyAsync(d_dst, h_src, bytes, cudaMemcpyHostToDevice, st));
     ctx->h2d_bytes += bytes;
     return SXGPU_OK;
@@ -3592,7 +3442,7 @@ int sxgpu_memcpy_d2h(sxgpu_ctx *ctx, void *h_dst, const void *d_src, size_t byte
     if (!ctx)
         return SXGPU_ERR_INVALID;
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
+    cudaStream_t st = call_stream(ctx, stream);
     SX_CUDA(ctx, cudaMemcpyAsync(h_dst, d_src, bytes, cudaMemcpyDeviceToHost, st));
     ctx->d2h_bytes += bytes;
     return SXGPU_OK;
@@ -3619,7 +3469,7 @@ int sxgpu_stream_sync(sxgpu_ctx *ctx, sxgpu_stream stream)
     if (!ctx)
         return SXGPU_ERR_INVALID;
     SX_CUDA(ctx, cudaSetDevice(ctx->device));
-    SX_CUDA(ctx, cudaStreamSynchronize(stream ? static_cast<cudaStream_t>(stream) : ctx->stream));
+    SX_CUDA(ctx, cudaStreamSynchronize(call_stream(ctx, stream)));
     return SXGPU_OK;
 }
 

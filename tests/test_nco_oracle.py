@@ -161,15 +161,18 @@ def nco_kernels_sass():
             kernels[name] = []
         elif name:
             kernels[name].append(line)
-    return {k: "\n".join(v) for k, v in kernels.items() if "nco" in k}
+    # the mixing instantiations of the FIR kernels have NcoView among their template arguments
+    return {k: "\n".join(v) for k, v in kernels.items() if "nco" in k or "NcoView" in k}
 
 
-def test_nco_kernels_have_no_fused_multiply_add():
+def test_nco_and_mixing_fir_kernels_have_no_fused_multiply_add():
     kernels = nco_kernels_sass()
-    for must in ("nco_apply_kernel", "nco_advance_kernel", "bank_nco_fir_kernel", "bank_nco_fir_read_tail_kernel",
-                 "bank_nco_fir_write_tail_kernel"):
-        assert any(must in k for k in kernels), (must, sorted(kernels))
+    assert any("nco_apply_kernel" in k for k in kernels), sorted(kernels)
+    assert any("nco_advance_kernel" in k for k in kernels), sorted(kernels)
+    for must in ("bank_fir_kernel", "bank_fir_read_tail_kernel", "fir_history_kernel"):
+        assert any(must in k and "NcoView" in k for k in kernels), (must, sorted(kernels))
+    assert sum("bank_fir_kernel" in k for k in kernels) == 6, sorted(kernels)  # R = 1, 2, 4, read and write
     for name, sass in kernels.items():
         assert not re.search(r"\bFFMA2?\b", sass), name
-        if "apply" in name or "nco_fir_kernel" in name or "read_tail" in name:
+        if "apply" in name or "bank_fir_kernel" in name or "read_tail" in name:
             assert re.search(r"\bFMUL2?\b", sass) and re.search(r"\bFADD2?\b", sass), name
