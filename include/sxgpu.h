@@ -470,6 +470,54 @@ int sxgpu_chan_apply(sxgpu_chan *c, const void *d_in, uint64_t nin, void *d_out,
 int sxgpu_chan_get_state(sxgpu_chan *c, void *h_hist, uint32_t *phase, sxgpu_stream stream);
 int sxgpu_chan_set_state(sxgpu_chan *c, const void *h_hist, uint32_t phase, sxgpu_stream stream);
 
+/* A transmitter that places many channels in one band: M channel-rate streams of each stream
+ * interpolated by D, each moved to its channel and summed, in one pass: the synthesis channelizer,
+ * the adjoint of sxgpu_chan_*.  Its input, [nstreams][M][nin], is what sxgpu_chan_apply emits, so
+ * channelize -> per-channel DSP -> synthesize needs no transposes.  M = channels, a power of two from
+ * 2 to SXGPU_CHAN_MAX_CHANNELS; D = up divides M (D = M critically sampled, D = M/2 oversampled by
+ * 2); h is one real prototype of ntaps taps, with the limits of sxgpu_chan_create, so one design
+ * serves both directions.  X counts the input frames per channel fed since creation or set_state;
+ * channel frames before the first are 0.  Output frame n of a stream, counted from output frame 0
+ * (X D + o for output o of a call), is
+ *     x[n] = sum_{k < M} sum_m h[n - m D] y_k[m] e^{+j 2 pi k n / M},
+ * i.e. sxgpu_fir_apply(h, up D, down 1) of each channel, then sxgpu_nco_apply at +k / M counted from
+ * output frame 0 (k >= M/2: (k - M) / M), summed over the channels, up to rounding.  Bit for bit
+ * (tests/sxchansynth.py restates it), with h rounded to float32 once, I and Q separately and every
+ * product and sum one float32 rounding (no FMA):
+ *   1. for every input frame m, an unnormalised M-point inverse DFT: a[i] = y_{rev(i)}[m], rev
+ *      reversing the log2 M bits of i; radix-2 decimation-in-time stages h = 1, 2, .. M/2: for every
+ *      i with (i mod 2h) < h,
+ *        w = T+[(i mod 2h) M / (2h)], p = a[i], q = a[i+h],
+ *        t.re = q.re w.re - q.im w.im, t.im = q.re w.im + q.im w.re, a[i] = p + t, a[i+h] = p - t,
+ *      every butterfly multiplied by its twiddle, T+[0] included; T+[j] = A[j 1024 / M], the
+ *      oscillators' coarse table entry, not conjugated; Y_m[i] = a[i] (no 1 / M);
+ *   2. output n = m D + t (t < D), P_t = ceil((ntaps - t) / D) (0 when t >= ntaps):
+ *        acc = +0;  for p = P_t - 1 down to 0:  acc = acc + Y_{m-p}[n mod M] * h[t + p D],
+ *      the oldest input frame first and only taps that exist multiplied.  For finite inputs this is
+ *      sxgpu_fir_apply(h, up D, down 1) of the sequence m -> Y_m[n mod M], bit for bit: a +-0
+ *      product added to an accumulator that starts at +0 changes no bit. */
+typedef struct sxgpu_chan_synth sxgpu_chan_synth;
+/* Refused: what sxgpu_chan_create refuses, with up in place of down.  The history starts at zero
+ * and the phase at 0.  sxgpu_destroy of the context refuses while a synthesizer is alive. */
+int sxgpu_chan_synth_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t channels, uint32_t up, uint32_t ntaps,
+                            const double *h, sxgpu_chan_synth **out);
+int sxgpu_chan_synth_destroy(sxgpu_chan_synth *s);
+/* d_in[nstreams][channels][nin] -> d_out[nstreams][nin * up], CF32: always nin * up output frames.
+ * The history and the phase are carried.  The phase, X mod (channels / up), lives on the host and is
+ * all the call depends on besides the buffers, so a call with nin a multiple of channels / up (which
+ * leaves the phase as it was; with up = channels, every call) may be captured in a CUDA graph and
+ * replayed; other calls must not be.  Only kernels are enqueued: chan_synth_kernel, then
+ * fir_history_kernel over the nstreams * channels rows when ceil(ntaps / up) > 1, so 2 launches per
+ * call at most, counted in "launches".  Refused: nin 0, a NULL or not 8-byte aligned buffer, byte
+ * sizes that overflow 64 bits, d_in and d_out overlapping, a grid of more than 2^31 - 1 CTAs. */
+int sxgpu_chan_synth_apply(sxgpu_chan_synth *s, const void *d_in, uint64_t nin, void *d_out, sxgpu_stream stream);
+/* The history, [nstreams][channels][hp - 1] complex64 on the host, hp = ceil(ntaps / up): each
+ * channel's last hp - 1 raw inputs, oldest first (nothing when hp = 1), and the phase
+ * X mod (channels / up).  get: either pointer may be NULL.  set: NULL h_hist = zeros; a phase of
+ * channels / up or more is refused.  Both synchronise with `stream`. */
+int sxgpu_chan_synth_get_state(sxgpu_chan_synth *s, void *h_hist, uint32_t *phase, sxgpu_stream stream);
+int sxgpu_chan_synth_set_state(sxgpu_chan_synth *s, const void *h_hist, uint32_t phase, sxgpu_stream stream);
+
 /* ---- the hot path, host buffers ---------------------------------------------------------- */
 
 /* Same contracts as the two converters above, but src and dest are HOST memory, as they

@@ -4,6 +4,6 @@ The product is native: CUDA kernels behind the C ABI of include/sxgpu.h (lib/lib
 and a C++ driver=sx SoapySDR device above it (lib/libsxsoapy.so).  This package only holds
 the build recipes and ctypes views that tests/ and bench.py use.
 """
-from .capi import Bank, Chan, Context, Fir, Iir, Multi, Nco, SxGpuError, load_library, library_path  # noqa: F401
+from .capi import Bank, Chan, ChanSynth, Context, Fir, Iir, Multi, Nco, SxGpuError, load_library, library_path  # noqa: F401
 
-__all__ = ["Bank", "Chan", "Context", "Fir", "Iir", "Multi", "Nco", "SxGpuError", "load_library", "library_path"]
+__all__ = ["Bank", "Chan", "ChanSynth", "Context", "Fir", "Iir", "Multi", "Nco", "SxGpuError", "load_library", "library_path"]

@@ -111,6 +111,11 @@ SIGNATURES = {
     "sxgpu_chan_apply": (C.c_int, [_P, _P, C.c_uint64, _P, C.POINTER(C.c_uint64), _P]),
     "sxgpu_chan_get_state": (C.c_int, [_P, _P, C.POINTER(C.c_uint32), _P]),
     "sxgpu_chan_set_state": (C.c_int, [_P, _P, C.c_uint32, _P]),
+    "sxgpu_chan_synth_create": (C.c_int, [_P, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, _P, C.POINTER(_P)]),
+    "sxgpu_chan_synth_destroy": (C.c_int, [_P]),
+    "sxgpu_chan_synth_apply": (C.c_int, [_P, _P, C.c_uint64, _P, _P]),
+    "sxgpu_chan_synth_get_state": (C.c_int, [_P, _P, C.POINTER(C.c_uint32), _P]),
+    "sxgpu_chan_synth_set_state": (C.c_int, [_P, _P, C.c_uint32, _P]),
     "sxgpu_convert_rx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S]),
     "sxgpu_convert_rx_buffer_host_gated": (C.c_int, [_P, _P, _S, _P, _S, _S, _P, _P]),
     "sxgpu_convert_tx_buffer_host": (C.c_int, [_P, _P, _S, _P, _S, _S, _F]),
@@ -650,6 +655,55 @@ class Chan(_Owned):
                 raise ValueError(f"hist must have shape {(self.nstreams, self.ntaps - 1)}, got {hist.shape}")
             ptr = hist.ctypes.data
         self.ctx.check(self.lib.sxgpu_chan_set_state(self.handle, ptr, phase, stream), "sxgpu_chan_set_state")
+
+
+class ChanSynth(_Owned):
+    """A polyphase synthesis channelizer per stream (sxgpu_chan_synth_* in include/sxgpu.h): the
+    `channels` channel-rate streams of each stream, in Chan.apply's layout, interpolated by `up`
+    (default: channels, critically sampled) with the real prototype `taps`, channel k moved to
+    k / channels cycles per output sample (numpy's fft order) and summed into one stream, the last
+    inputs carried from call to call."""
+
+    _destroy = "sxgpu_chan_synth_destroy"
+
+    def __init__(self, ctx: Context, nstreams: int, taps, channels: int, up: int | None = None):
+        import numpy as np
+        self.np = np
+        self.ctx, self.lib = ctx, ctx.lib
+        up = channels if up is None else up
+        taps = np.ascontiguousarray(np.asarray(taps, dtype=np.float64))
+        if taps.ndim != 1:
+            raise ValueError(f"taps must be one-dimensional, got shape {taps.shape}")
+        h = _P()
+        ctx.check(self.lib.sxgpu_chan_synth_create(ctx.handle, nstreams, channels, up, taps.size,
+                                                   taps.ctypes.data if taps.size else None, C.byref(h)),
+                  "sxgpu_chan_synth_create")
+        self.handle, self.nstreams, self.ntaps, self.channels, self.up = h, nstreams, taps.size, channels, up
+        self.hp = -(-taps.size // up)
+
+    def apply(self, d_in, nin, d_out, stream=None):
+        """d_in[nstreams][channels][nin] -> d_out[nstreams][nin * up] (complex64 on the device)."""
+        self.ctx.check(self.lib.sxgpu_chan_synth_apply(self.handle, d_in, nin, d_out, stream), "sxgpu_chan_synth_apply")
+
+    def state(self, stream=None):
+        """(history, phase): each channel's last hp - 1 inputs, (nstreams, channels, hp - 1) complex64
+        oldest first, and the input frames fed so far mod channels / up."""
+        hist = self.np.empty((self.nstreams, self.channels, self.hp - 1), self.np.complex64)
+        phase = C.c_uint32()
+        self.ctx.check(self.lib.sxgpu_chan_synth_get_state(self.handle, hist.ctypes.data, C.byref(phase), stream),
+                       "sxgpu_chan_synth_get_state")
+        return hist, phase.value
+
+    def set_state(self, hist=None, phase=0, stream=None):
+        """Set the history, (nstreams, channels, hp - 1) complex64 (None = zeros), and the phase."""
+        ptr = None
+        if hist is not None:
+            hist = self.np.ascontiguousarray(hist, dtype=self.np.complex64)
+            shape = (self.nstreams, self.channels, self.hp - 1)
+            if hist.shape != shape:
+                raise ValueError(f"hist must have shape {shape}, got {hist.shape}")
+            ptr = hist.ctypes.data
+        self.ctx.check(self.lib.sxgpu_chan_synth_set_state(self.handle, ptr, phase, stream), "sxgpu_chan_synth_set_state")
 
 
 class Multi:

@@ -3224,6 +3224,185 @@ int sxgpu_chan_set_state(sxgpu_chan *c, const void *h_hist, uint32_t phase, sxgp
     return SXGPU_OK;
 }
 
+// ---- polyphase synthesis channelizers (sx_chan.cuh) -------------------------------------------
+} // extern "C"
+
+struct sxgpu_chan_synth {
+    sxgpu_ctx *ctx = nullptr;
+    uint32_t nstreams = 0, m = 2, log2m = 1, up = 1, log2up = 0, ntaps = 1, hp = 1;
+    uint32_t phase = 0;     // input frames fed so far mod M / D: the only state kept on the host
+    DevPtr<float2> mem;     // one allocation: the twiddles [1024], then the taps [ntaps]
+    DevPtr<float2> hist;    // [nstreams][M][hp - 1], device memory; NULL when hp == 1
+};
+
+namespace {
+
+constexpr size_t kChanSynthSmemBytes = 96 * 1024; // two CTAs of chan_synth_kernel fit an SM's 227 KB
+constexpr uint32_t kChanSynthMaxThreads = 1024;
+
+// The geometry of a call of nin frames per channel, without its buffers, and the kernel's threads
+// and shared memory.  False when the grid would not fit.
+bool chan_synth_call(const sxgpu_chan_synth *c, uint64_t nin, ChanSynthCall &a, uint32_t &threads, size_t &smem)
+{
+    const uint32_t M = c->m, D = c->up;
+    a.hist = c->hist.get();
+    a.tw = c->mem.get();
+    a.taps = reinterpret_cast<const float *>(c->mem.get() + kNcoTableSize);
+    a.nin = nin;
+    a.m = M;
+    a.log2m = c->log2m;
+    a.log2up = c->log2up;
+    a.ntaps = c->ntaps;
+    a.hp = c->hp;
+    a.rot0 = (c->phase * D) % M;
+    // As many input frames per tile as the threads can keep the outputs of (fewer for a short call),
+    // so that the hp - 1 frames each tile transforms again are few against its own.
+    uint32_t b = kChanSynthBlock * kChanSynthMaxThreads / D;
+    while (b > 1 && b / 2 >= nin)
+        b /= 2;
+    a.frames = b;
+    threads = std::max<uint32_t>(32, b * D / kChanSynthBlock);
+    const size_t row = size_t(M + 1) * sizeof(float2);
+    a.chunk = uint32_t(std::max<size_t>(1, std::min<size_t>(b + c->hp - 1, kChanSynthSmemBytes / row)));
+    smem = a.chunk * row;
+    a.tiles = (nin + b - 1) / b;
+    return a.tiles <= uint64_t(INT32_MAX) / c->nstreams;
+}
+
+size_t chan_synth_hist_bytes(const sxgpu_chan_synth *c)
+{
+    return size_t(c->nstreams) * c->m * (c->hp - 1) * sizeof(float2);
+}
+
+} // namespace
+
+extern "C" {
+
+int sxgpu_chan_synth_create(sxgpu_ctx *ctx, uint32_t nstreams, uint32_t channels, uint32_t up, uint32_t ntaps,
+                            const double *h, sxgpu_chan_synth **out)
+{
+    if (!ctx || !out)
+        return SXGPU_ERR_INVALID;
+    *out = nullptr;
+    if (channels < 2 || channels > SXGPU_CHAN_MAX_CHANNELS || (channels & (channels - 1)))
+        return ctx->invalid("a synthesizer has a power of two of 2 to SXGPU_CHAN_MAX_CHANNELS channels");
+    if (nstreams == 0 || uint64_t(nstreams) * channels > uint64_t(INT32_MAX))
+        return ctx->invalid("a synthesizer has 1 to (2^31 - 1) / channels streams");
+    if (up == 0 || channels % up)
+        return ctx->invalid("a synthesizer's interpolation divides its channel count");
+    if (ntaps < 1 || ntaps > SXGPU_CHAN_MAX_TAPS || ntaps > 32 * channels || !h)
+        return ctx->invalid("a synthesizer has 1 to min(SXGPU_CHAN_MAX_TAPS, 32 channels) taps");
+    for (uint32_t i = 0; i < ntaps; i++)
+        if (!std::isfinite(h[i]))
+            return ctx->invalid("every synthesizer tap must be finite");
+    std::unique_ptr<sxgpu_chan_synth> c(new sxgpu_chan_synth());
+    c->ctx = ctx;
+    c->nstreams = nstreams;
+    c->m = channels;
+    while ((1u << c->log2m) < channels)
+        c->log2m++;
+    c->up = up;
+    while ((1u << c->log2up) < up)
+        c->log2up++;
+    c->ntaps = ntaps;
+    c->hp = (ntaps + up - 1) / up;
+    // The twiddles: the oscillator's coarse table as it is, then the taps rounded once.
+    std::vector<float2> tw = nco_tables();
+    tw.resize(kNcoTableSize);
+    std::vector<float> taps(ntaps);
+    for (uint32_t i = 0; i < ntaps; i++)
+        taps[i] = float(h[i]);
+    const size_t tw_bytes = tw.size() * sizeof(float2), taps_bytes = taps.size() * sizeof(float);
+    std::vector<char> img(tw_bytes + taps_bytes);
+    std::memcpy(img.data(), tw.data(), tw_bytes);
+    std::memcpy(img.data() + tw_bytes, taps.data(), taps_bytes);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    SX_CUDA(ctx, cudaFuncSetAttribute(chan_synth_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      int(std::min<size_t>(kChanSynthSmemBytes, ctx->prop.sharedMemPerBlockOptin))));
+    SX_CUDA(ctx, cudaFuncSetAttribute(fir_history_kernel<NoNco>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      int((kChanMaxTaps - 1) * sizeof(float2))));
+    cudaError_t e = dev_upload(ctx, c->mem, img.data(), img.size());
+    if (e == cudaSuccess && c->hp > 1)
+        e = dev_upload(ctx, c->hist, nullptr, chan_synth_hist_bytes(c.get()));
+    return dsp_created(ctx, c, e, "cudaMalloc(synthesizer)", out);
+}
+
+int sxgpu_chan_synth_destroy(sxgpu_chan_synth *s)
+{
+    return dsp_destroy(s);
+}
+
+int sxgpu_chan_synth_apply(sxgpu_chan_synth *s, const void *d_in, uint64_t nin, void *d_out, sxgpu_stream stream)
+{
+    if (!s)
+        return SXGPU_ERR_INVALID;
+    sxgpu_ctx *ctx = s->ctx;
+    if (!d_in || !d_out || reinterpret_cast<uintptr_t>(d_in) % 8 || reinterpret_cast<uintptr_t>(d_out) % 8)
+        return ctx->invalid("sxgpu_chan_synth_apply: input and output must be 8-byte aligned device memory");
+    if (nin == 0)
+        return ctx->invalid("sxgpu_chan_synth_apply: a block has at least one frame");
+    const uint64_t nstreams = s->nstreams, rows = nstreams * s->m;
+    if (nin > UINT64_MAX / 8 / rows)
+        return ctx->invalid("sxgpu_chan_synth_apply: nstreams * channels * nin * 8 bytes overflows 64 bits");
+    if (nin > UINT64_MAX / 8 / nstreams / s->up)
+        return ctx->invalid("sxgpu_chan_synth_apply: nstreams * nin * up * 8 bytes overflows 64 bits");
+    const uintptr_t in0 = reinterpret_cast<uintptr_t>(d_in), out0 = reinterpret_cast<uintptr_t>(d_out);
+    const uint64_t in_bytes = rows * nin * 8, out_bytes = nstreams * nin * s->up * 8;
+    if (in0 >= out0 ? in0 - out0 < out_bytes : out0 - in0 < in_bytes)
+        return ctx->invalid("sxgpu_chan_synth_apply: input and output overlap");
+
+    ChanSynthCall a = {};
+    uint32_t threads = 0;
+    size_t smem = 0;
+    if (!chan_synth_call(s, nin, a, threads, smem))
+        return ctx->invalid("sxgpu_chan_synth_apply: the block needs more CTAs than a grid holds");
+    a.in = static_cast<const float2 *>(d_in);
+    a.out = static_cast<float2 *>(d_out);
+    SX_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = call_stream(ctx, stream);
+    chan_synth_kernel<<<unsigned(nstreams * a.tiles), threads, smem, st>>>(a);
+    SX_CUDA(ctx, cudaGetLastError());
+    int launches = 1;
+    if (s->hp > 1) {
+        // Each of the nstreams * M channel rows keeps its last hp - 1 raw inputs, as a FIR filter's.
+        FirCall hc = {};
+        hc.in = a.in;
+        hc.hist = s->hist.get();
+        hc.nin = nin;
+        hc.hp = s->hp;
+        fir_history_kernel<<<unsigned(rows), kFirHistoryThreads, (s->hp - 1) * sizeof(float2), st>>>(hc);
+        SX_CUDA(ctx, cudaGetLastError());
+        launches++;
+    }
+    ctx->launches += launches;
+    const uint32_t period = s->m / s->up;
+    s->phase = uint32_t((s->phase + nin % period) % period);
+    return SXGPU_OK;
+}
+
+int sxgpu_chan_synth_get_state(sxgpu_chan_synth *s, void *h_hist, uint32_t *phase, sxgpu_stream stream)
+{
+    if (!s)
+        return SXGPU_ERR_INVALID;
+    if (h_hist && s->hp > 1)
+        SX_TRY(state_copy(s->ctx, h_hist, s->hist.get(), chan_synth_hist_bytes(s), cudaMemcpyDeviceToHost, stream));
+    if (phase)
+        *phase = s->phase;
+    return SXGPU_OK;
+}
+
+int sxgpu_chan_synth_set_state(sxgpu_chan_synth *s, const void *h_hist, uint32_t phase, sxgpu_stream stream)
+{
+    if (!s)
+        return SXGPU_ERR_INVALID;
+    if (phase >= s->m / s->up)
+        return s->ctx->invalid("sxgpu_chan_synth_set_state: the phase is below channels / up");
+    if (s->hp > 1)
+        SX_TRY(state_copy(s->ctx, s->hist.get(), h_hist, chan_synth_hist_bytes(s), cudaMemcpyHostToDevice, stream));
+    s->phase = phase;
+    return SXGPU_OK;
+}
+
 int sxgpu_fill_silence(sxgpu_ctx *ctx, void *d_i2s, size_t offset, size_t length,
                        sxgpu_stream stream)
 {
